@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the phi-FEM hot path: cut-cell tags + CSR assembly, cells/s.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--n 204] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--n 204] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the synthetic 3D P1 configuration of BASELINE.json
 (config E, SURVEY.md section 8d): classify all cells and facets of a 6 n^3 Kuhn-tetrahedra unit cube
@@ -418,9 +418,10 @@ class Workload:
                 "interior": int(c[0]), "cut": int(c[1]), "exterior": int(c[2])}
 
 
-def timed_steps(w, steps, world, sampler=None, presteps=15):
+def timed_steps(w, steps, world, sampler=None, presteps=15, after=None):
     """EXACTLY `steps` steps bracketed by barrier + synchronize, device-timed, max over ranks; per-phase means from the
-    events recorded inside the timed region (eager runs) and the assembly split from a short untimed loop."""
+    events recorded inside the timed region (eager runs) and the assembly split from a short untimed loop.  `after()`
+    runs once the timed steps and the sampler have stopped, while the outputs are still those of the last timed step."""
     import torch
     import torch.distributed as dist
     dev = w.mesh.device
@@ -448,6 +449,8 @@ def timed_steps(w, steps, world, sampler=None, presteps=15):
     if world > 1:
         dist.barrier()
     clocks = sampler.stop() if sampler is not None else None
+    if after is not None:
+        after()
     total_ms = start.elapsed_time(stop)
     if world > 1:
         t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
@@ -475,6 +478,28 @@ def timed_steps(w, steps, world, sampler=None, presteps=15):
         per["assemble_surface"] = per.pop("assemble_ghost")      # ghost penalty + one-sided term, one pass
         per.pop("assemble_boundary")
     return total_ms / steps, per, clocks
+
+
+DUMP_SAMPLE = 1 << 20    # entries kept of a longer output array (--dump-outputs)
+DUMP_SEED = 0
+
+
+def dump_outputs(w, outdir):
+    """What a caller of compute_tags_measures + assemble_strong_dirichlet receives from the step just run -- cell and
+    facet tags, CSR pattern and values, load vector -- as outdir/<name>.npy (tags float32, the rest float64; every value
+    exact).  An array longer than DUMP_SAMPLE entries keeps DUMP_SAMPLE of them, at sorted positions drawn with DUMP_SEED
+    from its length alone: two builds that compute the same arrays write the same files, 40 MB at most."""
+    import torch
+    os.makedirs(outdir, exist_ok=True)
+    arrays = {"cell_tags": (w.ws.cell_tags8, np.float32), "facet_tags": (w.ws.facet_tags8, np.float32),
+              "A_indptr": (w.plan.indptr, np.float64), "A_indices": (w.plan.indices, np.float64),
+              "A_data": (w.data, np.float64), "b": (w.b, np.float64)}
+    for name, (t, dtype) in arrays.items():
+        t = t.reshape(-1)
+        if t.numel() > DUMP_SAMPLE:
+            pos = np.sort(np.random.default_rng(DUMP_SEED).choice(t.numel(), DUMP_SAMPLE, replace=False))
+            t = t[torch.from_numpy(pos).to(t.device)]
+        np.save(os.path.join(outdir, name + ".npy"), t.cpu().numpy().astype(dtype))
 
 
 def roofline_of(w, per, ms_per_step, clocks):
@@ -1041,7 +1066,8 @@ def run_ours(args):
     for _ in range(args.warmup):
         w.step()
     torch.cuda.synchronize()
-    ms_per_step, per, clocks = timed_steps(w, args.steps, world, sampler=ClockSampler(local_rank))
+    dump = (lambda: dump_outputs(w, args.dump_outputs)) if args.dump_outputs else None
+    ms_per_step, per, clocks = timed_steps(w, args.steps, world, sampler=ClockSampler(local_rank), after=dump)
 
     n_cells_local = problem.n_owned_cells if problem is not None else mesh.num_cells
     n_cells_total = n_cells_local
@@ -1271,16 +1297,26 @@ def parser():
                     help="multi-GPU: exchange the exterior-cell counts with an NCCL all-reduce instead of peer memory")
     ap.add_argument("--no-graph", action="store_true", help="strong scaling: eager launches instead of one CUDA graph")
     ap.add_argument("--no-e2e", action="store_true", help="skip the end-to-end leg (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the tags, CSR arrays and load vector of the last one as DIR/<name>.npy "
+                         "(one GPU, --impl ours; arrays over %d entries as a fixed seeded sample)" % DUMP_SAMPLE)
     return ap
 
 
 def main():
+    # the benchmark reads the tree and never writes to it (the tree may be read-only): no bytecode caches there either
+    sys.dont_write_bytecode = True
     ap = parser()
     args = ap.parse_args()
     if args.n is None:
         args.n = CONFIGS[args.config][0]
-    if args.config != "3d-p1" and (args.gpus > 1 or int(os.environ.get("WORLD_SIZE", "1")) > 1):
+    multi_gpu = args.gpus > 1 or int(os.environ.get("WORLD_SIZE", "1")) > 1
+    if args.config != "3d-p1" and multi_gpu:
         raise SystemExit("bench.py: the multi-GPU path runs the 3d-p1 configuration")
+    if args.steps < 1:
+        raise SystemExit("bench.py: --steps must be at least 1")
+    if args.dump_outputs and (multi_gpu or args.impl != "ours"):
+        raise SystemExit("bench.py: --dump-outputs writes the outputs of the single-GPU path (--impl ours)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     _quiet_stdout()
     if args.impl == "reference":

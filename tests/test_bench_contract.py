@@ -25,8 +25,50 @@ def test_defaults_of_the_command_line():
     a = bench.parser().parse_args([])
     assert a.gpus == 1 and a.impl == "ours" and a.config == "3d-p1" and a.warmup >= 3 and a.steps >= 10
     assert a.cell_pass == "rows" and not a.no_e2e and not a.no_e2e_pipeline and not a.no_others
+    assert a.dump_outputs is None
     assert bench.CONFIGS["3d-p1"][0] == 204          # 6 * 204^3 = 50 937 984 tetrahedra: BASELINE.json configs[4]
     assert 6 * 204 ** 3 == 50937984
+
+
+def test_dump_outputs_writes_exact_values_and_a_seeded_sample(tmp_path):
+    """--dump-outputs on a stand-in workload of host tensors: one .npy per output, values exact in float32 / float64,
+    short arrays whole, long ones sampled at the same positions on every call, under 64 MB in all."""
+    import types
+
+    import numpy as np
+    import torch
+    n_long = bench.DUMP_SAMPLE + 12345
+    rng = np.random.default_rng(5)
+    plan = types.SimpleNamespace(indptr=torch.arange(0, 3 * 1001, 3, dtype=torch.int32),
+                                 indices=torch.from_numpy(rng.integers(0, 2 ** 31 - 1, n_long).astype(np.int32)))
+    ws = types.SimpleNamespace(cell_tags8=torch.from_numpy(rng.integers(1, 4, n_long).astype(np.int8)),
+                               facet_tags8=torch.from_numpy(rng.integers(0, 5, 777).astype(np.int8)))
+    w = types.SimpleNamespace(ws=ws, plan=plan, data=torch.from_numpy(rng.standard_normal(n_long)),
+                              b=torch.from_numpy(rng.standard_normal(1000)))
+    bench.dump_outputs(w, str(tmp_path / "a"))
+    bench.dump_outputs(w, str(tmp_path / "b"))
+    names = {"cell_tags", "facet_tags", "A_indptr", "A_indices", "A_data", "b"}
+    assert {p.stem for p in (tmp_path / "a").iterdir()} == names
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= 64 * 2 ** 20
+    got = {nm: np.load(tmp_path / "a" / (nm + ".npy")) for nm in names}
+    for nm in names:
+        assert np.array_equal(got[nm], np.load(tmp_path / "b" / (nm + ".npy")))
+    assert got["cell_tags"].dtype == got["facet_tags"].dtype == np.float32
+    assert got["A_data"].dtype == got["A_indices"].dtype == got["A_indptr"].dtype == got["b"].dtype == np.float64
+    assert np.array_equal(got["facet_tags"], ws.facet_tags8.numpy()) and np.array_equal(got["b"], w.b.numpy())
+    assert np.array_equal(got["A_indptr"], plan.indptr.numpy())
+    pos = np.sort(np.random.default_rng(bench.DUMP_SEED).choice(n_long, bench.DUMP_SAMPLE, replace=False))
+    assert np.array_equal(got["A_data"], w.data.numpy()[pos])
+    assert np.array_equal(got["A_indices"], plan.indices.numpy()[pos])
+    assert np.array_equal(got["cell_tags"], ws.cell_tags8.numpy()[pos])
+
+
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--dump-outputs", "out", "--impl", "reference"],
+                                  ["--dump-outputs", "out", "--gpus", "2"]])
+def test_bench_refuses_arguments_it_cannot_honour(argv, monkeypatch):
+    monkeypatch.setattr("sys.argv", ["bench.py"] + argv)
+    with pytest.raises(SystemExit, match="bench.py: "):
+        bench.main()
 
 
 def test_algorithmic_bytes_is_the_yardstick_of_the_survey():
