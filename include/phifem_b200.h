@@ -462,7 +462,18 @@ int phifem_bicgstab_iterate(int64_t n_act, int64_t nnz, const int32_t* rows, con
  * `f` and `u_n` are P1 (vertex values).  robin_coef != 0 turns the penalty combination into
  * y.grad phi - |grad phi| robin_coef u + h^-1 p phi: the Robin operator of demo/robin/square/main.py:118-174 (u_n = the
  * Robin data; its ghost penalty runs over dS(2): pass those facets to phifem_assemble_neumann_ghost).  Slot maps: cells entry-major [nm*nm, n_active], one-sided entities
- * [n, nm*nm], interior facets tagged 3 [n, (2 nm)^2] (macro order [mixed dofs of cell +, of cell -]).  ADD semantics. */
+ * [n, nm*nm], interior facets tagged 3 [n, (2 nm)^2] (macro order [mixed dofs of cell +, of cell -]).  ADD semantics.
+ *
+ * Quadrilaterals (mesh->cell_type == PHIFEM_QUADRILATERAL, vertices in tensor order, the demo's own mesh): the mixed
+ * space is Q1 x Q1^2 x DG0 (nm = 13: [u x4, y node-major x8, p]) and the bilinear cell map is evaluated at every
+ * quadrature point (csrc/assemble_quad.cu).  There
+ *   - phifem_quadrature.cell_points holds REFERENCE coordinates (xi, eta) [n_cell_points, 2] on [0,1]^2, weights summing
+ *     to 1 (phifem_b200/quadrature.py rules_for_neumann_quad); the facet table stays the segment rule
+ *     [n_facet_points, 2] = (1 - t, t), t running from the edge's lower-global-id vertex to the higher one;
+ *   - space_phi->n_dofs_per_cell must be 4 (Q1, degree 1, dofmap may be NULL) or 9 (Q2, degree 2, dolfinx-local order:
+ *     vertices, the edges (0,1),(0,2),(1,3),(2,3), interior); any other value returns PHIFEM_ERR_ARGUMENT;
+ *   - every interior cell is integrated by the cell rule too (no closed form on a non-affine cell);
+ *   - cells must be convex (either orientation); a non-convex quadrilateral is outside the method and not checked. */
 /* `cut_positions` [n_cut]: positions in `active` of the cells tagged 2 (every term of the form, by quadrature); the
  * other active cells carry the P1 stiffness + mass block of u only (closed form, a separate light kernel). */
 int phifem_assemble_neumann_cells(const phifem_mesh* mesh, const phifem_pk_space* space_phi,

@@ -375,9 +375,12 @@ def assemble_weak_dirichlet(plan, phi_h, f_h, u_D=None, pen_coef=1.0, stab_coef=
 def build_plan_neumann(mesh, cells_tags, facets_tags, ds=None, V_phi=None, ghost_tag=3):
     """Symbolic phase for `a` and `L` of the Neumann demo (reference demo/neumann/square/main.py:103-158): mixed space
     (u, y, p) in P1 x P1^d x DG0 (`mixed_space`, main.py:71-79) on triangles / tetrahedra, level-set space `V_phi`
-    (P1 or P2; default P1).  Mixed vector layout: u at vertex s -> (d+1) s, y_c -> (d+1) s + 1 + c, p of cell k ->
-    (d+1) Nv + k (`plan.split(x)` returns the three fields).  ghost_tag: facets of the gradient-jump term, dS(3) in the
-    Neumann demo (main.py:136-139), dS(2) in the Robin demo (demo/robin/square/main.py:143-150)."""
+    (P1 or P2; default P1).  On quadrilaterals (the demo's own mesh) the space is Q1 x Q1^2 x DG0 and `V_phi` is Q1 or
+    Q2, integrated by the Gauss product rule of `quadrature.rules_for_neumann_quad` (convex cells of either
+    orientation; a non-convex quadrilateral is outside the method).  Mixed vector layout: u at vertex s -> (d+1) s,
+    y_c -> (d+1) s + 1 + c, p of cell k -> (d+1) Nv + k (`plan.split(x)` returns the three fields).  ghost_tag: facets
+    of the gradient-jump term, dS(3) in the Neumann demo (main.py:136-139), dS(2) in the Robin demo
+    (demo/robin/square/main.py:143-150)."""
     from . import fem
     from .assemble_pk import PkAssemblyPlan
     V = fem.functionspace(mesh, 1)
@@ -391,7 +394,8 @@ def build_plan_neumann(mesh, cells_tags, facets_tags, ds=None, V_phi=None, ghost
 
 
 def assemble_neumann(plan, phi_h, f_h, u_N, pen_coef=1.0, stab_coef=1.0, robin_coef=0.0):
-    """A (CSR over the mixed dofs) and b of reference demo/neumann/square/main.py:117-161; `f_h`, `u_N` are P1.
+    """A (CSR over the mixed dofs) and b of reference demo/neumann/square/main.py:117-161; `f_h`, `u_N` are P1 (Q1 on
+    quadrilaterals: vertex values).
     robin_coef != 0 (with a plan built with ghost_tag=2): the Robin operator of demo/robin/square/main.py:118-174,
     `u_N` being the Robin data u_R."""
     from .assemble_pk import assemble_neumann_into

@@ -33,7 +33,12 @@ class PkAssemblyPlan:
         if form == "neumann" and V.degree != 1:
             raise NotImplementedError("the Neumann operator is implemented for P1 u and y (main.py:37-39)")
         self.form = form
-        if mesh.cell_type not in ("triangle", "tetrahedron"):
+        if mesh.cell_type == "quadrilateral":
+            # bilinear cell map: the Neumann kernels of csrc/assemble_quad.cu; the strong / weak forms need second
+            # derivatives of the map (their Hessian terms) and are not implemented there
+            if form != "neumann":
+                raise NotImplementedError("P_k assembly on quadrilaterals implements the Neumann operator only")
+        elif mesh.cell_type not in ("triangle", "tetrahedron"):
             raise NotImplementedError("P_k assembly supports triangles and tetrahedra")
         for sp in (V, V_phi):
             if sp.mesh is not mesh:
@@ -50,8 +55,8 @@ class PkAssemblyPlan:
             self.pattern_dofmap = torch.cat([2 * self.dofmap, 2 * self.dofmap + 1], dim=1).contiguous()
             self.n_rows = n = 2 * int(V.num_dofs)
         elif form == "neumann":
-            # mixed space (u, y, p) in P1 x P1^d x DG0: u at vertex s -> (d+1) s, y_c -> (d+1) s + 1 + c,
-            # p of cell k -> (d+1) Nv + k; cell-local order [u, y node-major, p]
+            # mixed space (u, y, p) in P1 x P1^d x DG0 (Q1 x Q1^2 x DG0 on quadrilaterals): u at vertex s -> (d+1) s,
+            # y_c -> (d+1) s + 1 + c, p of cell k -> (d+1) Nv + k; cell-local order [u, y node-major, p]
             d_, nvx = mesh.gdim, mesh.num_vertices
             c = mesh.cells.long()
             y = ((d_ + 1) * c[:, :, None] + 1 + torch.arange(d_, device=dev)[None, None, :]).reshape(c.shape[0], -1)
@@ -106,7 +111,9 @@ class PkAssemblyPlan:
 
         # quadrature tables and C structs (kept alive with the plan)
         d = mesh.gdim
-        if form == "neumann":
+        if form == "neumann" and mesh.cell_type == "quadrilateral":
+            (cl, cw), (fl, fw) = quadrature.rules_for_neumann_quad(V_phi.degree)   # cell points: (xi, eta)
+        elif form == "neumann":
             (cl, cw), (fl, fw) = quadrature.rules_for_neumann(d, V_phi.degree)
         else:
             rules = quadrature.rules_for_weak if form == "weak" else quadrature.rules_for

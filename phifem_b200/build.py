@@ -12,7 +12,7 @@ LIB = os.path.join(HERE, "libphifem_b200.so")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"] + ARCH
 # tags.cu restates the reference's exact ==1.0 comparisons: no FMA contraction there
-SOURCES = [("capi.cu", []), ("tags.cu", ["-fmad=false"]), ("assemble.cu", []), ("assemble_rows.cu", []), ("assemble_tiles.cu", []), ("assemble_pk.cu", []), ("assemble_elasticity.cu", []), ("symbolic.cu", []), ("rows_plan.cu", []), ("solve.cu", []), ("peer.cu", [])]
+SOURCES = [("capi.cu", []), ("tags.cu", ["-fmad=false"]), ("assemble.cu", []), ("assemble_rows.cu", []), ("assemble_tiles.cu", []), ("assemble_pk.cu", []), ("assemble_quad.cu", []), ("assemble_elasticity.cu", []), ("symbolic.cu", []), ("rows_plan.cu", []), ("solve.cu", []), ("peer.cu", [])]
 
 
 def _nvcc():

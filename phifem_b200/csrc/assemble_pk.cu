@@ -1028,6 +1028,17 @@ void dispatch(int cell_type, int kw, int kp, F&& f) {
 }
 
 }  // namespace
+
+// the Neumann operator on quadrilaterals (bilinear cell map): csrc/assemble_quad.cu
+int quad_neumann_cells(const phifem_mesh* mesh, const phifem_pk_space* space_phi, const phifem_quadrature* quad_rule,
+                       const double* phi, const double* f, const double* u_n, const int8_t* cell_tags8,
+                       const int32_t* active, int64_t n_active, const int32_t* cut_positions, int64_t n_cut,
+                       const int32_t* slots, const int32_t* mixed_dofmap, double gamma, double robin_coef,
+                       double* data, double* b, cudaStream_t st);
+int quad_neumann_boundary(const phifem_mesh* mesh, const int32_t* entities, int64_t n_entities, const int32_t* slots,
+                          double* data, cudaStream_t st);
+int quad_neumann_ghost(const phifem_mesh* mesh, const phifem_quadrature* quad_rule, const int32_t* facets,
+                       int64_t n_facets, const int32_t* slots, double sigma, double* data, cudaStream_t st);
 }  // namespace phifem
 
 using namespace phifem;
@@ -1193,6 +1204,21 @@ extern "C" int phifem_assemble_neumann_cells(const phifem_mesh* mesh, const phif
                                              const int32_t* slots, const int32_t* mixed_dofmap, double gamma,
                                              double robin_coef, double* data, double* b, void* stream) {
   PHIFEM_CHECK_ARG(quad != nullptr && space_phi != nullptr, "quadrature / level-set space is null");
+  if (mesh != nullptr && mesh->cell_type == PHIFEM_QUADRILATERAL) {
+    PHIFEM_CHECK_ARG(mesh->x && mesh->cells && mesh->gdim == 2, "quadrilateral mesh needs x, cells and gdim 2");
+    PHIFEM_CHECK_ARG(space_phi->n_dofs_per_cell == 4 || space_phi->n_dofs_per_cell == 9,
+                     "space_phi->n_dofs_per_cell must be 4 (Q1) or 9 (Q2) on quadrilaterals");
+    PHIFEM_CHECK_ARG(space_phi->degree == (space_phi->n_dofs_per_cell == 4 ? 1 : 2),
+                     "space_phi->degree does not match n_dofs_per_cell");
+    PHIFEM_CHECK_ARG(space_phi->dofmap || space_phi->degree == 1, "a Q2 level set needs its dofmap");
+    PHIFEM_CHECK_ARG(quad->cell_points && quad->cell_weights && quad->n_cell_points > 0 &&
+                         quad->n_cell_points <= kMaxQuadPoints, "quadrature rule (1..128 points)");
+    if (n_active == 0) return PHIFEM_OK;
+    PHIFEM_CHECK_ARG(phi && f && u_n && cell_tags8 && data && b && mixed_dofmap && active && slots, "null pointer");
+    PHIFEM_CHECK_ARG(n_cut >= 0 && n_cut <= n_active && (n_cut == 0 || cut_positions), "cut-cell positions");
+    return quad_neumann_cells(mesh, space_phi, quad, phi, f, u_n, cell_tags8, active, n_active, cut_positions, n_cut,
+                              slots, mixed_dofmap, gamma, robin_coef, data, b, (cudaStream_t)stream);
+  }
   phifem_pk_space p1{1, mesh && mesh->cell_type == PHIFEM_TRIANGLE ? 3 : 4, 0, nullptr};
   if (int rc = check_pk(mesh, &p1, space_phi, quad->cell_points, quad->cell_weights, quad->n_cell_points)) return rc;
   if (n_active == 0) return PHIFEM_OK;
@@ -1218,13 +1244,19 @@ extern "C" int phifem_assemble_neumann_boundary(const phifem_mesh* mesh, const i
                                                 int64_t n_entities, const int32_t* slots, double* data,
                                                 void* stream) {
   PHIFEM_CHECK_ARG(mesh != nullptr && mesh->x && mesh->cells, "mesh is null");
-  if (mesh->cell_type != PHIFEM_TRIANGLE && mesh->cell_type != PHIFEM_TETRAHEDRON) {
-    set_error("the Neumann operator supports triangles and tetrahedra, got cell type %d", mesh->cell_type);
+  if (mesh->cell_type != PHIFEM_TRIANGLE && mesh->cell_type != PHIFEM_TETRAHEDRON &&
+      mesh->cell_type != PHIFEM_QUADRILATERAL) {
+    set_error("the Neumann operator supports triangles, quadrilaterals and tetrahedra, got cell type %d",
+              mesh->cell_type);
     return PHIFEM_ERR_UNSUPPORTED;
   }
   if (n_entities == 0) return PHIFEM_OK;
   PHIFEM_CHECK_ARG(entities && slots && data, "null pointer");
   cudaStream_t st = (cudaStream_t)stream;
+  if (mesh->cell_type == PHIFEM_QUADRILATERAL) {
+    PHIFEM_CHECK_ARG(mesh->gdim == 2, "gdim mismatch");
+    return quad_neumann_boundary(mesh, entities, n_entities, slots, data, st);
+  }
   if (mesh->cell_type == PHIFEM_TRIANGLE)
     k_assemble_boundary_neumann<2><<<(unsigned)((n_entities * 3 + kBlockPk - 1) / kBlockPk), kBlockPk, 0, st>>>(
         *mesh, entities, n_entities, slots, data);
@@ -1239,6 +1271,14 @@ extern "C" int phifem_assemble_neumann_ghost(const phifem_mesh* mesh, const phif
                                              const int32_t* facets, int64_t n_facets, const int32_t* slots,
                                              double sigma, double* data, void* stream) {
   PHIFEM_CHECK_ARG(quad != nullptr, "quadrature is null");
+  if (mesh != nullptr && mesh->cell_type == PHIFEM_QUADRILATERAL) {
+    PHIFEM_CHECK_ARG(mesh->x && mesh->cells && mesh->gdim == 2, "quadrilateral mesh needs x, cells and gdim 2");
+    PHIFEM_CHECK_ARG(quad->facet_points && quad->facet_weights && quad->n_facet_points > 0 &&
+                         quad->n_facet_points <= kMaxQuadPoints, "quadrature rule (1..128 points)");
+    if (n_facets == 0) return PHIFEM_OK;
+    PHIFEM_CHECK_ARG(data && mesh->c2f && mesh->f2c && facets && slots, "null pointer");
+    return quad_neumann_ghost(mesh, quad, facets, n_facets, slots, sigma, data, (cudaStream_t)stream);
+  }
   phifem_pk_space p1{1, mesh && mesh->cell_type == PHIFEM_TRIANGLE ? 3 : 4, 0, nullptr};
   if (int rc = check_pk(mesh, &p1, &p1, quad->facet_points, quad->facet_weights, quad->n_facet_points)) return rc;
   if (n_facets == 0) return PHIFEM_OK;

@@ -215,3 +215,21 @@ def rules_for_neumann(d, kphi):
     level set: the penalty block (y.grad phi + p phi / h)^2 has degree 2 (kphi + 1) at most (|grad phi_h| in the
     load term is not polynomial for kphi = 2: integrated by the same rule); the facet terms are constant / linear."""
     return simplex_rule(d, 2 * (kphi + 1)), simplex_rule(d - 1, 2)
+
+
+def square_rule(m):
+    """m x m Gauss-Legendre product rule on the reference square [0, 1]^2: (points [m^2, 2] in reference coordinates
+    (xi, eta), xi fastest; weights [m^2] summing to 1), exact for xi^a eta^b with a, b <= 2m - 1."""
+    t, w = gauss_jacobi(int(m), 0)
+    X, Y = np.meshgrid(t, t, indexing="xy")
+    W = w[None, :] * w[:, None]
+    return np.ascontiguousarray(np.stack([X.ravel(), Y.ravel()], axis=1)), np.ascontiguousarray(W.ravel())
+
+
+def rules_for_neumann_quad(kphi):
+    """Cell and facet rules of the Neumann forms on quadrilaterals for Q1 u / y and a Q_kphi level set: on a
+    parallelogram the worst polynomial term, (y.grad phi)^2, has degree 2 (kphi + 1) in each reference direction, so
+    kphi + 2 Gauss points per direction integrate every polynomial term exactly.  |grad phi_h| is not polynomial even
+    for kphi = 1, and on a non-affine cell no integrand is: the operator is defined at this rule.  Facets: the 2-point
+    segment rule (Q1 restricted to a straight edge is linear; on a parallelogram the gradient jumps are too)."""
+    return square_rule(kphi + 2), simplex_rule(1, 2)

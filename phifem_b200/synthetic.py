@@ -2,7 +2,8 @@
 
 S-2D(n): n x n squares split by the "right" diagonal -> 2 n^2 triangles (what
 `dolfinx.mesh.create_rectangle` gives the reference demos,
-demo/strong-dirichlet/flower/main.py:48-49).  S-3D(n): n^3 cubes x 6 Kuhn tetrahedra.
+demo/strong-dirichlet/flower/main.py:48-49).  Q-2D(n): the same n x n squares as quadrilaterals (the cell type of
+demo/neumann/square).  S-3D(n): n^3 cubes x 6 Kuhn tetrahedra.
 Vertices are numbered lexicographically; generated directly on the target device.
 """
 import itertools
@@ -33,6 +34,18 @@ def rectangle_mesh(n, lo=(-1.0, -1.0), hi=(1.0, 1.0), device=None):
     t1 = torch.stack([v00, v01, v11], dim=1)
     cells = torch.stack([t0, t1], dim=1).reshape(-1, 3).to(torch.int32)
     return Mesh(x, cells, "triangle", device)
+
+
+def quadrilateral_mesh(n, lo=(-1.0, -1.0), hi=(1.0, 1.0), device=None):
+    """n^2 quadrilaterals in dolfinx tensor order (v0 = (x_i, y_j), v1 = (x_i+1, y_j), v2 = (x_i, y_j+1),
+    v3 = (x_i+1, y_j+1)); vertex id = i*(n+1)+j for the point (x_i, y_j), as in `rectangle_mesh`."""
+    device = torch.device(device) if device is not None else default_device()
+    x = _grid_vertices(lo, hi, n, device)
+    i = torch.arange(n, device=device, dtype=torch.int64)
+    I, J = torch.meshgrid(i, i, indexing="ij")
+    v00 = (I * (n + 1) + J).reshape(-1)
+    cells = torch.stack([v00, v00 + (n + 1), v00 + 1, v00 + (n + 1) + 1], dim=1).to(torch.int32).contiguous()
+    return Mesh(x, cells, "quadrilateral", device)
 
 
 def box_mesh(n, lo=(0.0, 0.0, 0.0), hi=(1.0, 1.0, 1.0), device=None):

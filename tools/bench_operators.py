@@ -1,9 +1,11 @@
 #!/usr/bin/env python
 """Timing of the mixed-space operators beside the headline path (not the bench.py contract: one JSON line per operator).
 
-    python tools/bench_operators.py [--ops neumann,elasticity-2d,elasticity-3d] [--steps 10] [--warmup 3]
+    python tools/bench_operators.py [--ops neumann,neumann-quad,elasticity-2d,elasticity-3d] [--steps 10] [--warmup 3]
 
   neumann        BASELINE.json configs[1]: demo/neumann forms on a synthetic 4 M-cell triangle mesh (n = 1414), disc
+  neumann-quad   the same forms on the demo's cell type: 2 M quadrilaterals on the same 2 M vertices (n = 1414), same
+                 disc, Q2 level set (as the demo, levelset_degree = 2)
   elasticity-2d  BASELINE.json configs[3] forms on 2 M triangles of the demo's box [-1.5, 1.5]^2 (n = 1000), unit disc
   elasticity-3d  BASELINE.json configs[3] as stated ("3D tetra mesh"): 384 000 Kuhn tetrahedra (n = 40), sphere
 
@@ -27,7 +29,9 @@ SYMMETRIC_BC = True   # --full-bc: the pass over the whole matrix instead of the
 
 
 def _tags(mesh, phi):
-    dls = mesh_scripts._DeviceLevelset(mesh, fem.Function(fem.functionspace_p1_device(mesh), phi), 1)
+    # quadrilaterals: the tag kernels gather the level set through a dofmap, which only the full space carries
+    V = fem.functionspace(mesh, 1) if mesh.cell_type == "quadrilateral" else fem.functionspace_p1_device(mesh)
+    dls = mesh_scripts._DeviceLevelset(mesh, fem.Function(V, phi), 1)
     ws = mesh_scripts.TagWorkspace(mesh)
     mesh_scripts.classify(mesh, dls, ws=ws)
     tdim = mesh.topology.dim
@@ -55,9 +59,9 @@ def _time(step, steps, warmup):
 def run(op, steps, warmup):
     dev = torch.device("cuda", 0)
     t0 = time.perf_counter()
-    if op == "neumann":
+    if op in ("neumann", "neumann-quad"):
         n = 1414
-        mesh = synthetic.rectangle_mesh(n, device=dev)
+        mesh = (synthetic.quadrilateral_mesh if op == "neumann-quad" else synthetic.rectangle_mesh)(n, device=dev)
         phi = synthetic.sphere_levelset(mesh.x, center=(0.0031, 0.0027), radius=0.6)
     elif op == "elasticity-2d":
         n = 1000
@@ -68,17 +72,21 @@ def run(op, steps, warmup):
         mesh = synthetic.box_mesh(n, device=dev)
         phi = synthetic.sphere_levelset(mesh.x)
     mesh.c2f
-    mesh.detj_bounds()
+    if mesh.cell_type != "quadrilateral":
+        mesh.detj_bounds()
     dls, ws, ctags, ftags, ds = _tags(mesh, phi)
     torch.cuda.synchronize()
     t1 = time.perf_counter()
     g = torch.Generator(device="cpu").manual_seed(1234)
-    if op == "neumann":
-        plan = assemble.build_plan_neumann(mesh, ctags, ftags, ds(100))
+    if op in ("neumann", "neumann-quad"):
+        V_phi = fem.functionspace(mesh, 2) if op == "neumann-quad" else None
+        plan = assemble.build_plan_neumann(mesh, ctags, ftags, ds(100), V_phi=V_phi)
+        phi_a = phi if V_phi is None else synthetic.sphere_levelset(V_phi.dof_coordinates_dev(),
+                                                                    center=(0.0031, 0.0027), radius=0.6)
         f = (2 * torch.rand(mesh.num_vertices, generator=g, dtype=torch.float64) - 1).to(dev)
         un = (2 * torch.rand(mesh.num_vertices, generator=g, dtype=torch.float64) - 1).to(dev)
         data, b = plan.new_outputs()
-        asm = lambda: assemble_pk.assemble_neumann_into(plan, phi, f, un, 1.0, 1.0, data, b)   # noqa: E731
+        asm = lambda: assemble_pk.assemble_neumann_into(plan, phi_a, f, un, 1.0, 1.0, data, b)   # noqa: E731
     else:
         plan = elasticity.build_plan_interface_elasticity(mesh, ctags, ftags, ds)
         f = (2 * torch.rand(mesh.num_vertices, mesh.gdim, generator=g, dtype=torch.float64) - 1).to(dev)
