@@ -1,12 +1,14 @@
 #!/usr/bin/env python
 """The reference's strong-Dirichlet demo on the GPU (background-mesh mode):
 
-    python demo/strong_dirichlet_flower.py [--n 200] [--degree 1]
+    python demo/strong_dirichlet_flower.py [--n 200] [--degree 1] [--cell-type triangle|quadrilateral]
 
 mirrors reference demo/strong-dirichlet/flower/main.py (`python main.py bg`) step by step -- background mesh of
 [-4.5, 4.5]^2 (main.py:47-49), tags from the non-smooth detection level set (:52-64), phi-FEM forms with the
 smooth level set (:85-131), solve (:138-157), u_h = phi_h w_h (:159-165) -- with the dolfinx / PETSc calls
-replaced by phifem_b200 (INTEGRATION.md).  Prints the timings of each stage and a summary of the solution."""
+replaced by phifem_b200 (INTEGRATION.md).  Prints the timings of each stage and a summary of the solution.
+--cell-type quadrilateral runs the same steps on n^2 quadrilaterals of the same box (Q1 fields and level set; a Q2 trial
+space is not implemented on quadrilaterals)."""
 import argparse
 import os
 import sys
@@ -20,7 +22,11 @@ from phifem_b200 import assemble, fem, solve, synthetic  # noqa: E402
 from phifem.mesh_scripts import compute_tags_measures  # noqa: E402  (the reference's import line)
 
 
-def main(n=200, degree=1, quiet=False):
+def main(n=200, degree=1, quiet=False, cell_type="triangle"):
+    if cell_type not in ("triangle", "quadrilateral"):
+        raise ValueError("cell_type must be 'triangle' or 'quadrilateral'")
+    if cell_type == "quadrilateral" and degree != 1:
+        raise ValueError("the strong-Dirichlet operator on quadrilaterals implements degree 1 (Q1) only")
     t = [time.perf_counter()]
 
     def lap(label):
@@ -29,7 +35,8 @@ def main(n=200, degree=1, quiet=False):
         if not quiet:
             print("%-28s %8.2f ms" % (label, (t[-1] - t[-2]) * 1e3))
 
-    bg_mesh = synthetic.rectangle_mesh(n, lo=(-4.5, -4.5), hi=(4.5, 4.5))
+    make_mesh = synthetic.quadrilateral_mesh if cell_type == "quadrilateral" else synthetic.rectangle_mesh
+    bg_mesh = make_mesh(n, lo=(-4.5, -4.5), hi=(4.5, 4.5))
     levelset_space = fem.functionspace(bg_mesh, ("Lagrange", 1))
     detection_levelset_h = fem.Function(levelset_space).interpolate(synthetic.flower_detection)
     lap("mesh + detection level set")
@@ -66,5 +73,8 @@ if __name__ == "__main__":
     ap = argparse.ArgumentParser()
     ap.add_argument("--n", type=int, default=200)
     ap.add_argument("--degree", type=int, default=1, choices=[1, 2])
+    ap.add_argument("--cell-type", default="triangle", choices=["triangle", "quadrilateral"])
     a = ap.parse_args()
-    main(a.n, a.degree)
+    if a.cell_type == "quadrilateral" and a.degree != 1:
+        ap.error("--degree 2 is not implemented with --cell-type quadrilateral")
+    main(a.n, a.degree, cell_type=a.cell_type)

@@ -379,6 +379,15 @@ typedef struct phifem_quadrature {
   const double* facet_weights; /* [n_facet_points] */
 } phifem_quadrature;
 
+/* Quadrilaterals (mesh->cell_type == PHIFEM_QUADRILATERAL, vertices in tensor order): the three entry points below
+ * assemble the same forms with the bilinear cell map evaluated at every quadrature point (csrc/assemble_quad.cu); the
+ * Hessian terms use the map's second derivative d^2 x / dxi deta.  There
+ *   - space_w must be Q1 (degree 1, 4 dofs per cell): degree 2 returns PHIFEM_ERR_UNSUPPORTED;
+ *   - space_phi->n_dofs_per_cell must be 4 (Q1) or 9 (Q2, with its dofmap, in the order of the Neumann entry points);
+ *     any other value, or a degree that does not match, returns PHIFEM_ERR_ARGUMENT;
+ *   - cell_points holds REFERENCE coordinates (xi, eta) [n_cell_points, 2] on [0,1]^2 (phifem_b200/quadrature.py
+ *     rules_for_strong_quad); the facet table is the segment rule [n_facet_points, 2] = (1 - t, t);
+ *   - cells must be convex (either orientation). */
 /* dx((1,2)) + dx(2) terms and the load vector (:105,107-112,126-128).  slots[nd*nd, n_active]: CSR position of
  * entry (test dof i, trial dof j) of active cell e at slots[(i*nd + j) * n_active + e] (entry-major, so that
  * consecutive threads read consecutive words).  `f` lives in the trial/test space. */

@@ -245,10 +245,26 @@ def build_plan(mesh, cells_tags, facets_tags, ds=None, method="rows", capacity=N
     `ds_bdy(100)` (main.py:64): a MeasureRestriction, a flat entity array, or None (no boundary term).
     `V` / `V_phi`: the demo's `primal_space` / `levelset_space` (main.py:74-75); omitted or both of degree 1
     => the closed-form P1 kernels, otherwise the quadrature kernels for P1 / P2 (phifem_b200/assemble_pk.py).
+    A quadrilateral mesh always takes the quadrature kernels, with V defaulting to Q1 and V_phi to V (a Q1 trial space
+    and a Q1 or Q2 level set); method "blocked" / "atomic", geometry, cell_pass != "rows" and symbolic="native" raise
+    ValueError there.
     cell_pass (row-gather plans): "rows" = one evaluation per (row, cell) record, "tiles" = the cell-once pass of
     csrc/assemble_tiles.cu.  geometry (row-gather plans): tabulate the cells' geometry factors once per plan (phifem_b200/rows.py; an
     option kept for the record, slower than the default on the B200)."""
     c8, f8, ents = _plan_inputs(mesh, cells_tags, facets_tags, ds)
+    if mesh.cell_type == "quadrilateral":
+        # the quadrature kernels of csrc/assemble_quad.cu (PkAssemblyPlan); the row-gather options have no
+        # quadrilateral implementation
+        if method not in ("rows", "pk"):
+            raise ValueError("method=%r: quadrilateral meshes are assembled by the quadrature kernels only" % method)
+        if geometry or cell_pass != "rows" or symbolic == "native":
+            raise ValueError("geometry, cell_pass and symbolic='native' are options of the row-gather plans, which "
+                             "have no quadrilateral implementation")
+        from . import fem
+        from .assemble_pk import PkAssemblyPlan
+        V = fem.functionspace(mesh, 1) if V is None else V
+        V_phi = V if V_phi is None else V_phi
+        return PkAssemblyPlan(mesh, c8, f8, ents, V, V_phi)
     V_phi = V if V_phi is None else V_phi
     V = V_phi if V is None else V
     if V is not None and (V.degree != 1 or V_phi.degree != 1 or method == "pk"):

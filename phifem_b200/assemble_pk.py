@@ -1,6 +1,7 @@
 """Strong-Dirichlet phi-FEM operator for Lagrange P1 / P2 trial-test spaces and P1 / P2 level sets
 (`fe_degree`, `levelset_degree` of reference demo/strong-dirichlet/flower/main.py:37-41), assembled into CSR
-by the quadrature kernels of csrc/assemble_pk.cu.
+by the quadrature kernels of csrc/assemble_pk.cu; on quadrilaterals Q1 trial-test spaces with a Q1 / Q2 level set
+(csrc/assemble_quad.cu, the same C entry points).
 
     V, Vphi = fem.functionspace(mesh, 2), fem.functionspace(mesh, 2)
     plan = assemble.build_plan(mesh, cells_tags, facets_tags, ds_bdy(100), V=V, V_phi=Vphi)
@@ -34,10 +35,13 @@ class PkAssemblyPlan:
             raise NotImplementedError("the Neumann operator is implemented for P1 u and y (main.py:37-39)")
         self.form = form
         if mesh.cell_type == "quadrilateral":
-            # bilinear cell map: the Neumann kernels of csrc/assemble_quad.cu; the strong / weak forms need second
-            # derivatives of the map (their Hessian terms) and are not implemented there
-            if form != "neumann":
-                raise NotImplementedError("P_k assembly on quadrilaterals implements the Neumann operator only")
+            # bilinear cell map: the Neumann and strong-Dirichlet kernels of csrc/assemble_quad.cu (the latter for a Q1
+            # trial / test space); the weak form is not implemented there
+            if form == "weak":
+                raise NotImplementedError("the weak-Dirichlet operator is not implemented on quadrilaterals")
+            if form == "strong" and V.degree != 1:
+                raise NotImplementedError("the strong-Dirichlet operator on quadrilaterals implements a Q1 trial "
+                                          "space only")
         elif mesh.cell_type not in ("triangle", "tetrahedron"):
             raise NotImplementedError("P_k assembly supports triangles and tetrahedra")
         for sp in (V, V_phi):
@@ -113,6 +117,8 @@ class PkAssemblyPlan:
         d = mesh.gdim
         if form == "neumann" and mesh.cell_type == "quadrilateral":
             (cl, cw), (fl, fw) = quadrature.rules_for_neumann_quad(V_phi.degree)   # cell points: (xi, eta)
+        elif mesh.cell_type == "quadrilateral":
+            (cl, cw), (fl, fw) = quadrature.rules_for_strong_quad(V_phi.degree)
         elif form == "neumann":
             (cl, cw), (fl, fw) = quadrature.rules_for_neumann(d, V_phi.degree)
         else:

@@ -1012,6 +1012,25 @@ int check_pk(const phifem_mesh* m, const phifem_pk_space* sw, const phifem_pk_sp
   return PHIFEM_OK;
 }
 
+// the strong-Dirichlet operator on quadrilaterals: a Q1 trial / test space, a Q1 or Q2 level set
+int check_quad_strong(const phifem_mesh* m, const phifem_pk_space* sw, const phifem_pk_space* sp,
+                      const double* points, const double* weights, int nq) {
+  PHIFEM_CHECK_ARG(m->x && m->cells && m->gdim == 2, "quadrilateral mesh needs x, cells and gdim 2");
+  PHIFEM_CHECK_ARG(sw && sp, "function spaces are null");
+  if (sw->degree != 1) {
+    set_error("the strong-Dirichlet operator on quadrilaterals implements a Q1 trial space, got degree %d", sw->degree);
+    return PHIFEM_ERR_UNSUPPORTED;
+  }
+  PHIFEM_CHECK_ARG(sw->n_dofs_per_cell == 4, "space_w->n_dofs_per_cell must be 4 (Q1) on quadrilaterals");
+  PHIFEM_CHECK_ARG(sp->n_dofs_per_cell == 4 || sp->n_dofs_per_cell == 9,
+                   "space_phi->n_dofs_per_cell must be 4 (Q1) or 9 (Q2) on quadrilaterals");
+  PHIFEM_CHECK_ARG(sp->degree == (sp->n_dofs_per_cell == 4 ? 1 : 2),
+                   "space_phi->degree does not match n_dofs_per_cell on quadrilaterals");
+  PHIFEM_CHECK_ARG(sp->dofmap || sp->degree == 1, "a Q2 level set on quadrilaterals needs its dofmap");
+  PHIFEM_CHECK_ARG(points && weights && nq > 0 && nq <= kMaxQuadPoints, "quadrature rule (1..128 points)");
+  return PHIFEM_OK;
+}
+
 // instantiate kernel<D, KW, KP> for the runtime (cell type, degrees)
 template <typename F>
 void dispatch(int cell_type, int kw, int kp, F&& f) {
@@ -1039,6 +1058,17 @@ int quad_neumann_boundary(const phifem_mesh* mesh, const int32_t* entities, int6
                           double* data, cudaStream_t st);
 int quad_neumann_ghost(const phifem_mesh* mesh, const phifem_quadrature* quad_rule, const int32_t* facets,
                        int64_t n_facets, const int32_t* slots, double sigma, double* data, cudaStream_t st);
+// the strong-Dirichlet operator on quadrilaterals (Q1 trial / test space): csrc/assemble_quad.cu
+int quad_strong_cells(const phifem_mesh* mesh, const phifem_pk_space* space_w, const phifem_pk_space* space_phi,
+                      const phifem_quadrature* quad_rule, const double* phi, const double* f, const int8_t* cell_tags8,
+                      const int32_t* active, int64_t n_active, const int32_t* slots, double sigma, double* data,
+                      double* b, cudaStream_t st);
+int quad_strong_boundary(const phifem_mesh* mesh, const phifem_pk_space* space_phi, const phifem_quadrature* quad_rule,
+                         const double* phi, const int32_t* entities, int64_t n_entities, const int32_t* slots,
+                         double* data, cudaStream_t st);
+int quad_strong_ghost(const phifem_mesh* mesh, const phifem_pk_space* space_phi, const phifem_quadrature* quad_rule,
+                      const double* phi, const int32_t* facets, int64_t n_facets, const int32_t* slots, double sigma,
+                      double* data, cudaStream_t st);
 }  // namespace phifem
 
 using namespace phifem;
@@ -1049,6 +1079,15 @@ extern "C" int phifem_assemble_cells_pk(const phifem_mesh* mesh, const phifem_pk
                                         const int32_t* active, int64_t n_active, const int32_t* slots,
                                         double sigma, double* data, double* b, void* stream) {
   PHIFEM_CHECK_ARG(quad != nullptr, "quadrature is null");
+  if (mesh != nullptr && mesh->cell_type == PHIFEM_QUADRILATERAL) {
+    if (int rc = check_quad_strong(mesh, space_w, space_phi, quad->cell_points, quad->cell_weights,
+                                   quad->n_cell_points))
+      return rc;
+    if (n_active == 0) return PHIFEM_OK;
+    PHIFEM_CHECK_ARG(phi && f && cell_tags8 && data && b && active && slots, "null pointer");
+    return quad_strong_cells(mesh, space_w, space_phi, quad, phi, f, cell_tags8, active, n_active, slots, sigma, data,
+                             b, (cudaStream_t)stream);
+  }
   if (int rc = check_pk(mesh, space_w, space_phi, quad->cell_points, quad->cell_weights, quad->n_cell_points))
     return rc;
   if (n_active == 0) return PHIFEM_OK;
@@ -1081,6 +1120,14 @@ extern "C" int phifem_assemble_boundary_pk(const phifem_mesh* mesh, const phifem
                                            const double* phi, const int32_t* entities, int64_t n_entities,
                                            const int32_t* slots, double* data, void* stream) {
   PHIFEM_CHECK_ARG(quad != nullptr, "quadrature is null");
+  if (mesh != nullptr && mesh->cell_type == PHIFEM_QUADRILATERAL) {
+    if (int rc = check_quad_strong(mesh, space_w, space_phi, quad->facet_points, quad->facet_weights,
+                                   quad->n_facet_points))
+      return rc;
+    if (n_entities == 0) return PHIFEM_OK;
+    PHIFEM_CHECK_ARG(phi && data && entities && slots, "null pointer");
+    return quad_strong_boundary(mesh, space_phi, quad, phi, entities, n_entities, slots, data, (cudaStream_t)stream);
+  }
   if (int rc = check_pk(mesh, space_w, space_phi, quad->facet_points, quad->facet_weights, quad->n_facet_points))
     return rc;
   if (n_entities == 0) return PHIFEM_OK;
@@ -1103,6 +1150,14 @@ extern "C" int phifem_assemble_ghost_pk(const phifem_mesh* mesh, const phifem_pk
                                         const double* phi, const int32_t* facets, int64_t n_facets,
                                         const int32_t* slots, double sigma, double* data, void* stream) {
   PHIFEM_CHECK_ARG(quad != nullptr, "quadrature is null");
+  if (mesh != nullptr && mesh->cell_type == PHIFEM_QUADRILATERAL) {
+    if (int rc = check_quad_strong(mesh, space_w, space_phi, quad->facet_points, quad->facet_weights,
+                                   quad->n_facet_points))
+      return rc;
+    if (n_facets == 0) return PHIFEM_OK;
+    PHIFEM_CHECK_ARG(phi && data && mesh->c2f && mesh->f2c && facets && slots, "null pointer");
+    return quad_strong_ghost(mesh, space_phi, quad, phi, facets, n_facets, slots, sigma, data, (cudaStream_t)stream);
+  }
   if (int rc = check_pk(mesh, space_w, space_phi, quad->facet_points, quad->facet_weights, quad->n_facet_points))
     return rc;
   if (n_facets == 0) return PHIFEM_OK;

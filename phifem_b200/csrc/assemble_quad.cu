@@ -10,6 +10,10 @@
 //
 // The entry points stay phifem_assemble_neumann_{cells,boundary,ghost} (assemble_pk.cu): they validate the arguments
 // and call the launchers at the end of this file when mesh->cell_type == PHIFEM_QUADRILATERAL.
+//
+// The same file holds the strong-Dirichlet operator (demo/strong-dirichlet/flower/main.py:104-128) for a Q1 trial /
+// test space and a Q1 or Q2 level set, behind phifem_assemble_{cells,boundary,ghost}_pk; its Hessian terms need the
+// second derivative of the bilinear map (see k_quad_cells_strong).
 #include "common.cuh"
 #include "pk_common.cuh"
 
@@ -404,6 +408,255 @@ __global__ void __launch_bounds__(kBlockPk) k_quad_ghost_neumann(
   }
 }
 
+// ==== strong-Dirichlet phi-FEM operator (reference demo/strong-dirichlet/flower/main.py:104-128) on Q1 =============
+//   a = int_{dx(1,2)} grad(phi w).grad(phi v) - int_{ds(100)} (grad(phi w).n) phi v
+//       + sigma int_{dS(2,3)} avg(h) [grad(phi w).n][grad(phi v).n] + sigma h^2 int_{dx(2)} lap(phi w) lap(phi v)
+//   L = int_{dx(1,2)} f phi v - sigma h^2 int_{dx(2)} f lap(phi v)
+// The physical Hessian on the bilinear cell: with K = J^-1 and c = d^2 x / dxi deta = X0 - X1 - X2 + X3 (the map's only
+// second derivative), H u = K^T (H_ref u - (c.grad u) E) K, E = [[0, 1], [1, 0]].  Only its trace is needed:
+// lap u = M00 P00 + 2 M01 P01 + M11 P11 with M = H_ref u - (c.grad u) E and P = K K^T.
+
+// 1-D Lagrange basis of lagrange_1d with second derivatives
+template <int K>
+__device__ __forceinline__ void lagrange_1d_d2(double t, double (&L)[K + 1], double (&dL)[K + 1],
+                                               double (&d2L)[K + 1]) {
+  lagrange_1d<K>(t, L, dL);
+  if constexpr (K == 1) {
+    d2L[0] = d2L[1] = 0.0;
+  } else {
+    d2L[0] = 4.0;  d2L[1] = -8.0;  d2L[2] = 4.0;
+  }
+}
+
+// eval_phi with the reference Hessian hr = (phi_xixi, phi_xieta, phi_etaeta)
+template <int K>
+__device__ __forceinline__ void eval_phi_hess(double xi, double eta, const double (&Jit)[2][2],
+                                              const double (&pc)[QSpace<K>::ND], double& ph, double (&gph)[2],
+                                              double (&hr)[3]) {
+  double Lx[K + 1], dLx[K + 1], d2Lx[K + 1], Ly[K + 1], dLy[K + 1], d2Ly[K + 1];
+  lagrange_1d_d2<K>(xi, Lx, dLx, d2Lx);
+  lagrange_1d_d2<K>(eta, Ly, dLy, d2Ly);
+  double gr0 = 0.0, gr1 = 0.0;
+  ph = hr[0] = hr[1] = hr[2] = 0.0;
+#pragma unroll
+  for (int k = 0; k < QSpace<K>::ND; ++k) {
+    const int ix = tensor_index<K>(k, 0), iy = tensor_index<K>(k, 1);
+    ph += pc[k] * Lx[ix] * Ly[iy];
+    gr0 += pc[k] * dLx[ix] * Ly[iy];
+    gr1 += pc[k] * Lx[ix] * dLy[iy];
+    hr[1] += pc[k] * dLx[ix] * dLy[iy];
+    if (K == 2) {
+      hr[0] += pc[k] * d2Lx[ix] * Ly[iy];
+      hr[2] += pc[k] * Lx[ix] * d2Ly[iy];
+    }
+  }
+  gph[0] = Jit[0][0] * gr0 + Jit[0][1] * gr1;
+  gph[1] = Jit[1][0] * gr0 + Jit[1][1] * gr1;
+}
+
+// Cells of dx(1,2): row a of the 4 x 4 element tensor and b_a, the Hessian terms on cut cells only.  One thread per
+// (active cell, test dof a); slots entry-major ([16, n_active]).
+template <int KP>
+__global__ void __launch_bounds__(kBlockPk) k_quad_cells_strong(
+    phifem_mesh m, phifem_pk_space sw, phifem_pk_space sp, const double* __restrict__ qpt_g,
+    const double* __restrict__ qw_g, int nq, const double* __restrict__ phi, const double* __restrict__ f,
+    const int8_t* __restrict__ ctags, const int32_t* __restrict__ active, int64_t n_active,
+    const int32_t* __restrict__ slots, double sigma, double* __restrict__ data, double* __restrict__ b) {
+  constexpr int NDP = QSpace<KP>::ND;
+  __shared__ double qpt[kMaxQuadPoints * 2], qw[kMaxQuadPoints];
+  for (int i = threadIdx.x; i < nq * 2; i += blockDim.x) qpt[i] = qpt_g[i];
+  for (int i = threadIdx.x; i < nq; i += blockDim.x) qw[i] = qw_g[i];
+  __syncthreads();
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_active * NV) return;
+  const int64_t e = t / NV;
+  const int a = (int)(t - e * NV);
+  const int64_t c = __ldg(active + e);
+  Cell g;
+  load_cell(m, c, g);
+  double pc[NDP], fc[NV];
+  load_phi<KP>(m, sp, phi, c, pc);
+  const int32_t* dm = sw.dofmap ? sw.dofmap + c * NV : m.cells + c * NV;
+#pragma unroll
+  for (int k = 0; k < NV; ++k) fc[k] = __ldg(f + __ldg(dm + k));
+  const bool cut = ctags[c] == 2;
+  const double sh2 = sigma * g.h2;
+  const double c0 = g.X[0][0] - g.X[1][0] - g.X[2][0] + g.X[3][0];   // c = d^2 x / dxi deta
+  const double c1 = g.X[0][1] - g.X[1][1] - g.X[2][1] + g.X[3][1];
+  const double sa = (a == 0 || a == 3) ? 1.0 : -1.0;                // H_ref psi_a = s_a E
+  double A[NV], bv = 0.0;
+#pragma unroll
+  for (int j = 0; j < NV; ++j) A[j] = 0.0;
+  for (int q = 0; q < nq; ++q) {
+    const double xi = qpt[2 * q], eta = qpt[2 * q + 1];
+    double N[NV], G[NV][2], Jit[2][2];
+    const double w = qw[q] * map_point(g, xi, eta, N, G, Jit);
+    double ph, gph[2], hr[3];
+    eval_phi_hess<KP>(xi, eta, Jit, pc, ph, gph, hr);
+    double fq = 0.0, na = N[0], ga[2] = {G[0][0], G[0][1]};
+#pragma unroll
+    for (int k = 0; k < NV; ++k) {
+      fq += fc[k] * N[k];
+      if (k == a) {
+        na = N[k];
+        ga[0] = G[k][0];
+        ga[1] = G[k][1];
+      }
+    }
+    double gu[NV][2];
+#pragma unroll
+    for (int j = 0; j < NV; ++j)
+#pragma unroll
+      for (int d = 0; d < 2; ++d) gu[j][d] = N[j] * gph[d] + ph * G[j][d];
+    double wga[2];
+#pragma unroll
+    for (int d = 0; d < 2; ++d) wga[d] = w * (na * gph[d] + ph * ga[d]);
+    bv += w * fq * ph * na;
+#pragma unroll
+    for (int j = 0; j < NV; ++j) A[j] += dotd<2>(wga, gu[j]);
+    if (cut) {
+      const double P00 = Jit[0][0] * Jit[0][0] + Jit[1][0] * Jit[1][0];   // P = K K^T, K^T = Jit
+      const double P01 = Jit[0][0] * Jit[0][1] + Jit[1][0] * Jit[1][1];
+      const double P11 = Jit[0][1] * Jit[0][1] + Jit[1][1] * Jit[1][1];
+      const double lph = hr[0] * P00 + 2.0 * (hr[1] - (c0 * gph[0] + c1 * gph[1])) * P01 + hr[2] * P11;
+      double lu[NV];
+#pragma unroll
+      for (int j = 0; j < NV; ++j) {
+        const double sj = (j == 0 || j == 3) ? 1.0 : -1.0;
+        const double lpsi = 2.0 * P01 * (sj - (c0 * G[j][0] + c1 * G[j][1]));
+        lu[j] = N[j] * lph + 2.0 * (gph[0] * G[j][0] + gph[1] * G[j][1]) + ph * lpsi;
+      }
+      const double lua = na * lph + 2.0 * dotd<2>(gph, ga) + ph * 2.0 * P01 * (sa - (c0 * ga[0] + c1 * ga[1]));
+      const double ws = w * sh2 * lua;
+      bv -= ws * fq;
+#pragma unroll
+      for (int j = 0; j < NV; ++j) A[j] += ws * lu[j];
+    }
+  }
+  atomicAdd(b + __ldg(dm + a), bv);
+#pragma unroll
+  for (int j = 0; j < NV; ++j) atomicAdd(data + __ldg(slots + (int64_t)(a * NV + j) * n_active + e), A[j]);
+}
+
+// -int_{ds(100)} (grad(phi w).n) phi v on (cell, local facet) pairs, along the straight edge with its constant normal.
+// One thread per (entity, test dof i); v_i vanishes on an edge without vertex i.  Slots entity-major ([n, 16]).
+template <int KP>
+__global__ void __launch_bounds__(kBlockPk) k_quad_boundary_strong(
+    phifem_mesh m, phifem_pk_space sp, const double* __restrict__ qfp_g, const double* __restrict__ qw_g, int nq,
+    const double* __restrict__ phi, const int32_t* __restrict__ entities, int64_t n_entities,
+    const int32_t* __restrict__ slots, double* __restrict__ data) {
+  constexpr int NDP = QSpace<KP>::ND;
+  __shared__ double qt[kMaxQuadPoints], qw[kMaxQuadPoints];
+  for (int i = threadIdx.x; i < nq; i += blockDim.x) {
+    qt[i] = qfp_g[2 * i + 1];   // segment point (1 - t, t): the parameter t
+    qw[i] = qw_g[i];
+  }
+  __syncthreads();
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_entities * NV) return;
+  const int64_t e = t / NV;
+  const int i = (int)(t - e * NV);
+  const int64_t c = __ldg(entities + 2 * e);
+  const int o = __ldg(entities + 2 * e + 1);
+  const int la = facet_vertex(o, 0), lb = facet_vertex(o, 1);
+  if (i != la && i != lb) return;
+  Cell g;
+  load_cell(m, c, g);
+  double pc[NDP];
+  load_phi<KP>(m, sp, phi, c, pc);
+  double n[2], len;
+  edge_normal(g, o, n, len);
+  const double r0[2] = {(double)(la & 1), (double)(la >> 1)}, r1[2] = {(double)(lb & 1), (double)(lb >> 1)};
+  double A[NV];
+#pragma unroll
+  for (int j = 0; j < NV; ++j) A[j] = 0.0;
+  for (int q = 0; q < nq; ++q) {
+    const double tq = qt[q];
+    const double xi = (1.0 - tq) * r0[0] + tq * r1[0], eta = (1.0 - tq) * r0[1] + tq * r1[1];
+    double N[NV], G[NV][2], Jit[2][2];
+    map_point(g, xi, eta, N, G, Jit);
+    double ph, gph[2];
+    eval_phi<KP>(xi, eta, Jit, pc, ph, gph);
+    const double gpn = dotd<2>(gph, n);
+    const double ui = -qw[q] * len * ph * pk::pick<NV>(N, i);
+#pragma unroll
+    for (int j = 0; j < NV; ++j) A[j] += ui * (N[j] * gpn + ph * dotd<2>(G[j], n));
+  }
+#pragma unroll
+  for (int j = 0; j < NV; ++j) atomicAdd(data + __ldg(slots + (e * NV + i) * NV + j), A[j]);
+}
+
+// sigma avg(h) int_F [grad(phi w).n][grad(phi v).n] over interior facets, into the 8 x 8 macro slots [dofs of cell +
+// (f2c[f][0]), of cell -].  The edge parameter runs from the lower- to the higher-global-id vertex (as in
+// k_quad_ghost_neumann), so both sides evaluate the same physical points; each side evaluates phi and grad(phi) from
+// its own cell's dofs.  One thread per (facet, macro dof a: a / 4 = side).
+template <int KP>
+__global__ void __launch_bounds__(kBlockPk) k_quad_ghost_strong(
+    phifem_mesh m, phifem_pk_space sp, const double* __restrict__ qfp_g, const double* __restrict__ qw_g, int nq,
+    const double* __restrict__ phi, const int32_t* __restrict__ facets, int64_t n_facets,
+    const int32_t* __restrict__ slots, double sigma, double* __restrict__ data) {
+  constexpr int NDP = QSpace<KP>::ND, NU = 2 * NV;
+  __shared__ double qt[kMaxQuadPoints], qw[kMaxQuadPoints];
+  for (int i = threadIdx.x; i < nq; i += blockDim.x) {
+    qt[i] = qfp_g[2 * i + 1];
+    qw[i] = qw_g[i];
+  }
+  __syncthreads();
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_facets * NU) return;
+  const int64_t e = t / NU;
+  const int a = (int)(t - e * NU);
+  const int32_t fct = __ldg(facets + e);
+  const int2 cc = __ldg(reinterpret_cast<const int2*>(m.f2c) + fct);
+  Cell g[2];
+  double pc[2][NDP], n[2][2], len = 0.0, r0[2][2], r1[2][2];
+#pragma unroll
+  for (int s = 0; s < 2; ++s) {
+    const int64_t c = s == 0 ? cc.x : cc.y;
+    load_cell(m, c, g[s]);
+    load_phi<KP>(m, sp, phi, c, pc[s]);
+    int o = 0;
+#pragma unroll
+    for (int k = 0; k < NV; ++k)
+      if (__ldg(m.c2f + c * NV + k) == fct) o = k;
+    int la = facet_vertex(o, 0), lb = facet_vertex(o, 1);
+    if (__ldg(m.cells + c * NV + la) > __ldg(m.cells + c * NV + lb)) {
+      const int tmp = la;
+      la = lb;
+      lb = tmp;
+    }
+    r0[s][0] = la & 1; r0[s][1] = la >> 1;
+    r1[s][0] = lb & 1; r1[s][1] = lb >> 1;
+    double l;
+    edge_normal(g[s], o, n[s], l);
+    if (s == 0) len = l;
+  }
+  const double coef = sigma * 0.5 * (sqrt(g[0].h2) + sqrt(g[1].h2)) * len;
+  double E[NU];
+#pragma unroll
+  for (int bb = 0; bb < NU; ++bb) E[bb] = 0.0;
+  for (int q = 0; q < nq; ++q) {
+    const double tq = qt[q];
+    double J[NU];
+#pragma unroll
+    for (int s = 0; s < 2; ++s) {
+      const double xi = (1.0 - tq) * r0[s][0] + tq * r1[s][0], eta = (1.0 - tq) * r0[s][1] + tq * r1[s][1];
+      double N[NV], G[NV][2], Jit[2][2];
+      map_point(g[s], xi, eta, N, G, Jit);
+      double ph, gph[2];
+      eval_phi<KP>(xi, eta, Jit, pc[s], ph, gph);
+      const double gpn = dotd<2>(gph, n[s]);
+#pragma unroll
+      for (int k = 0; k < NV; ++k) J[s * NV + k] = N[k] * gpn + ph * dotd<2>(G[k], n[s]);
+    }
+    const double wa = qw[q] * coef * pk::pick<NU>(J, a);
+#pragma unroll
+    for (int bb = 0; bb < NU; ++bb) E[bb] += wa * J[bb];
+  }
+#pragma unroll
+  for (int bb = 0; bb < NU; ++bb) atomicAdd(data + __ldg(slots + (e * NU + a) * NU + bb), E[bb]);
+}
+
 inline unsigned blocks(int64_t threads) { return (unsigned)((threads + kBlockPk - 1) / kBlockPk); }
 
 }  // namespace quad
@@ -447,6 +700,55 @@ int quad_neumann_ghost(const phifem_mesh* mesh, const phifem_quadrature* quad_ru
   k_quad_ghost_neumann<<<blocks(n_facets * 2 * NV), kBlockPk, 0, st>>>(
       *mesh, quad_rule->facet_points, quad_rule->facet_weights, quad_rule->n_facet_points, facets, n_facets, slots,
       sigma, data);
+  PHIFEM_CHECK_LAUNCH();
+  return PHIFEM_OK;
+}
+
+int quad_strong_cells(const phifem_mesh* mesh, const phifem_pk_space* space_w, const phifem_pk_space* space_phi,
+                      const phifem_quadrature* quad_rule, const double* phi, const double* f, const int8_t* cell_tags8,
+                      const int32_t* active, int64_t n_active, const int32_t* slots, double sigma, double* data,
+                      double* b, cudaStream_t st) {
+  using namespace quad;
+  const double *qp = quad_rule->cell_points, *qw = quad_rule->cell_weights;
+  const int nq = quad_rule->n_cell_points;
+  if (space_phi->n_dofs_per_cell == QSpace<1>::ND)
+    k_quad_cells_strong<1><<<blocks(n_active * NV), kBlockPk, 0, st>>>(
+        *mesh, *space_w, *space_phi, qp, qw, nq, phi, f, cell_tags8, active, n_active, slots, sigma, data, b);
+  else
+    k_quad_cells_strong<2><<<blocks(n_active * NV), kBlockPk, 0, st>>>(
+        *mesh, *space_w, *space_phi, qp, qw, nq, phi, f, cell_tags8, active, n_active, slots, sigma, data, b);
+  PHIFEM_CHECK_LAUNCH();
+  return PHIFEM_OK;
+}
+
+int quad_strong_boundary(const phifem_mesh* mesh, const phifem_pk_space* space_phi, const phifem_quadrature* quad_rule,
+                         const double* phi, const int32_t* entities, int64_t n_entities, const int32_t* slots,
+                         double* data, cudaStream_t st) {
+  using namespace quad;
+  const double *qp = quad_rule->facet_points, *qw = quad_rule->facet_weights;
+  const int nq = quad_rule->n_facet_points;
+  if (space_phi->n_dofs_per_cell == QSpace<1>::ND)
+    k_quad_boundary_strong<1><<<blocks(n_entities * NV), kBlockPk, 0, st>>>(*mesh, *space_phi, qp, qw, nq, phi,
+                                                                             entities, n_entities, slots, data);
+  else
+    k_quad_boundary_strong<2><<<blocks(n_entities * NV), kBlockPk, 0, st>>>(*mesh, *space_phi, qp, qw, nq, phi,
+                                                                             entities, n_entities, slots, data);
+  PHIFEM_CHECK_LAUNCH();
+  return PHIFEM_OK;
+}
+
+int quad_strong_ghost(const phifem_mesh* mesh, const phifem_pk_space* space_phi, const phifem_quadrature* quad_rule,
+                      const double* phi, const int32_t* facets, int64_t n_facets, const int32_t* slots, double sigma,
+                      double* data, cudaStream_t st) {
+  using namespace quad;
+  const double *qp = quad_rule->facet_points, *qw = quad_rule->facet_weights;
+  const int nq = quad_rule->n_facet_points;
+  if (space_phi->n_dofs_per_cell == QSpace<1>::ND)
+    k_quad_ghost_strong<1><<<blocks(n_facets * 2 * NV), kBlockPk, 0, st>>>(*mesh, *space_phi, qp, qw, nq, phi, facets,
+                                                                            n_facets, slots, sigma, data);
+  else
+    k_quad_ghost_strong<2><<<blocks(n_facets * 2 * NV), kBlockPk, 0, st>>>(*mesh, *space_phi, qp, qw, nq, phi, facets,
+                                                                            n_facets, slots, sigma, data);
   PHIFEM_CHECK_LAUNCH();
   return PHIFEM_OK;
 }

@@ -233,3 +233,12 @@ def rules_for_neumann_quad(kphi):
     for kphi = 1, and on a non-affine cell no integrand is: the operator is defined at this rule.  Facets: the 2-point
     segment rule (Q1 restricted to a straight edge is linear; on a parallelogram the gradient jumps are too)."""
     return square_rule(kphi + 2), simplex_rule(1, 2)
+
+
+def rules_for_strong_quad(kphi):
+    """Cell and facet rules of the strong-Dirichlet forms on quadrilaterals for Q1 w / v and a Q_kphi level set: on a
+    parallelogram every integrand (stiffness, Hessian products, one-sided term, gradient jumps) is a polynomial of degree
+    at most 2 (kphi + 1) per reference direction, and the load f phi v of degree kphi + 2: kphi + 2 Gauss points per
+    direction on cells and a degree 2 kphi + 2 rule on edges are exact.  On a non-affine cell no integrand is
+    polynomial: the operator is defined at these rules."""
+    return square_rule(kphi + 2), simplex_rule(1, 2 * kphi + 2)
