@@ -31,24 +31,6 @@ def needs_build():
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build_variant(tag, defines, sources=("assemble_tiles.cu", "assemble_rows.cu", "tags.cu")):
-    """libphifem_b200_<tag>.so with extra -D flags on the kernel files (tuning sweeps on the GPU box: select it with
-    PHIFEM_B200_LIB); every other object is reused from the default build."""
-    build()
-    nvcc = _nvcc()
-    objs = []
-    for name, extra in SOURCES:
-        obj = os.path.join(CSRC, name[:-3] + ".o")
-        if name in sources:
-            obj = os.path.join(CSRC, name[:-3] + "." + tag + ".o")
-            subprocess.run([nvcc, "-c", os.path.join(CSRC, name), "-o", obj] + COMMON + extra
-                           + ["-D" + d for d in defines], check=True)
-        objs.append(obj)
-    lib = os.path.join(HERE, "libphifem_b200_%s.so" % tag)
-    subprocess.run([nvcc, "-shared", "-o", lib] + objs + ARCH, check=True)
-    return lib
-
-
 def build(force=False, verbose=False):
     if not force and not needs_build():
         return LIB

@@ -17,19 +17,6 @@ namespace phifem {
 using namespace pk;
 namespace {
 
-#ifndef PHIFEM_PK_UNROLL_Q
-#define PHIFEM_PK_UNROLL_Q 1
-#endif
-#ifndef PHIFEM_PK_SINGLE_STORES
-#define PHIFEM_PK_SINGLE_STORES 1
-#endif
-// k_assemble_ghost_pk: add the facet's duplicate entries up in shared memory before the reductions (400 -> 196 per P2
-// tetrahedron facet).  MEASURED at the 3d-p2 configuration: 1.253 ms against 1.040 ms for the plain scatter (2d-p2: 0.043
-// against 0.039): three more barriers and the strided shared-memory rows cost more than 204 same-address reductions.
-// Parity green (tests/test_gpu_assembly_pk.py with -DPHIFEM_PK_GHOST_DEDUPE=1); off by default.
-#ifndef PHIFEM_PK_GHOST_DEDUPE
-#define PHIFEM_PK_GHOST_DEDUPE 0
-#endif
 // Does exactly ONE cell of a conforming simplicial mesh contribute to the CSR entry (dof i, dof j) of a cell?  True when
 // the vertices the two dofs sit on (a vertex dof: itself; a P2 edge dof: the edge's two vertices) are all D + 1 vertices
 // of the cell between them AND no facet contains them all -- in 2D: two different edge dofs, or a vertex dof and the
@@ -51,7 +38,7 @@ __host__ __device__ constexpr bool single_contributor(int i, int j) {
 // ---- cells: rows [I0, I1) of the symmetric element matrix (columns j >= i) and of the load vector ----
 //   A_ij = int grad(phi psi_i).grad(phi psi_j) + [cut] sigma h^2 int lap(phi psi_i) lap(phi psi_j)   (main.py:105-112)
 //   b_i  = int f phi psi_i - [cut] sigma h^2 int f lap(phi psi_i)                                     (:126-128)
-template <int D, int KW, int KP, int I0, int I1, bool SLOTS_SHARED = false>
+template <int D, int KW, int KP, int I0, int I1>
 __device__ __forceinline__ void cell_rows(const Geometry<D>& g, const double (&pc)[Space<D, KP>::ND],
                                           const double (&fc)[Space<D, KW>::ND], bool is_cut, double sigma,
                                           const double* __restrict__ qlam, const double* __restrict__ qw,
@@ -75,9 +62,6 @@ __device__ __forceinline__ void cell_rows(const Geometry<D>& g, const double (&p
     for (int k = 0; k < NDP; ++k) lph += pc[k] * pl[k];
   }
   const double sh2 = is_cut ? sigma * g.h2 : 0.0;
-#if PHIFEM_PK_UNROLL_Q == 2
-#pragma unroll 2
-#endif
   for (int q = 0; q < nq; ++q) {
     double lam[NV];
 #pragma unroll
@@ -125,9 +109,9 @@ __device__ __forceinline__ void cell_rows(const Geometry<D>& g, const double (&p
 #pragma unroll
     for (int j = i; j < ND; ++j) {
       const double v = A[i - I0][j];
-      const int32_t sij = SLOTS_SHARED ? slots[(i * ND + j) * stride] : __ldg(slots + (int64_t)(i * ND + j) * stride);
-      const int32_t sji = SLOTS_SHARED ? slots[(j * ND + i) * stride] : __ldg(slots + (int64_t)(j * ND + i) * stride);
-      if (PHIFEM_PK_SINGLE_STORES && single_contributor<D, KW>(i, j)) {
+      const int32_t sij = __ldg(slots + (int64_t)(i * ND + j) * stride);
+      const int32_t sji = __ldg(slots + (int64_t)(j * ND + i) * stride);
+      if (single_contributor<D, KW>(i, j)) {
         data[sij] = v;
         data[sji] = v;
       } else {
@@ -144,20 +128,14 @@ template <> struct Passes<10> { static constexpr int N = 3; };
 
 // measured on the B200 at config C (16 M P2 triangles, cell kernel): 128 threads x 3 CTAs per SM 1.252 ms, x 2 CTAs 1.252,
 // x 4 CTAs (spills) 1.268; 64 threads x 6 CTAs 1.214; + the slot lines prefetched into L1 before the quadrature loop 1.188;
-// 64 x 4 (226 registers, nothing spilled) 1.174; the quadrature loop unrolled by two: 1.172 (64 x 4), 1.274 (64 x 6)
-#ifndef PHIFEM_PK_CELLS_MINBLOCKS_2D
-#define PHIFEM_PK_CELLS_MINBLOCKS_2D 4
-#endif
-#ifndef PHIFEM_PK_CELLS_BLOCK
-#define PHIFEM_PK_CELLS_BLOCK 64
-#endif
-#ifndef PHIFEM_PK_PREFETCH_SLOTS
-#define PHIFEM_PK_PREFETCH_SLOTS 1
-#endif
-constexpr int kBlockPkCells = PHIFEM_PK_CELLS_BLOCK;
+// 64 x 4 (226 registers, nothing spilled) 1.174; the quadrature loop unrolled by two: 1.172 (64 x 4), 1.274 (64 x 6).
+// A persistent version with the next cells' loads pipelined through cp.async measured 1.331 against 1.175 ms: the kernel
+// is bound by the number of its scattered reductions, not by the latency in front of them (DESIGN.md §4, K2p).
+constexpr int kBlockPkCells = 64;
+constexpr int kPkCellsMinBlocks2D = 4;
 
 template <int D, int KW, int KP>
-__global__ void __launch_bounds__(kBlockPkCells, D == 2 ? PHIFEM_PK_CELLS_MINBLOCKS_2D : 256 / kBlockPkCells) k_assemble_cells_pk(
+__global__ void __launch_bounds__(kBlockPkCells, D == 2 ? kPkCellsMinBlocks2D : 256 / kBlockPkCells) k_assemble_cells_pk(
     phifem_mesh m, phifem_pk_space sw, phifem_pk_space sp, const double* __restrict__ qlam_g,
     const double* __restrict__ qw_g, int nq, const double* __restrict__ phi, const double* __restrict__ f,
     const int8_t* __restrict__ ctags, const int32_t* __restrict__ active, int64_t n_active,
@@ -183,14 +161,12 @@ __global__ void __launch_bounds__(kBlockPkCells, D == 2 ? PHIFEM_PK_CELLS_MINBLO
   }
   const bool is_cut = ctags[c] == 2;
   const int32_t* sl = slots + e;
-#if PHIFEM_PK_PREFETCH_SLOTS
   // the slot lines of the final scatter (entry-major: one coalesced line per entry and warp) are requested now, so that
   // the ND^2 dependent load -> reduction pairs at the end find them in L1
   if ((threadIdx.x & 31) == 0) {
 #pragma unroll
     for (int k = 0; k < ND * ND; ++k) asm volatile("prefetch.global.L1 [%0];" ::"l"(sl + (int64_t)k * n_active));
   }
-#endif
   if constexpr (ND == 10) {
     if (blockIdx.y == 0)
       cell_rows<D, KW, KP, 0, 2>(g, pc, fc, is_cut, sigma, qlam, qw, nq, sl, n_active, dofs, data, b);
@@ -202,150 +178,6 @@ __global__ void __launch_bounds__(kBlockPkCells, D == 2 ? PHIFEM_PK_CELLS_MINBLO
     cell_rows<D, KW, KP, 0, ND>(g, pc, fc, is_cut, sigma, qlam, qw, nq, sl, n_active, dofs, data, b);
   }
 }
-
-// ---- the same cells as a PERSISTENT, software-pipelined kernel (single-pass spaces: ND <= 6) --------------------------
-// The kernel above spends 30 % of its stall samples in the prologue (active[e] -> cell / dof ids -> coordinates and
-// coefficients: three dependent global loads before the first fp64 instruction) and 17 % in the final scatter (ND^2
-// slot load -> reduction pairs), with 8 warps per SM to hide them (226 registers).  Here a thread walks cells
-// e, e + T, e + 2 T, ... (T = threads of the grid) and the loads of the NEXT cells travel while the current one is
-// integrated, through per-thread shared-memory slots filled by cp.async (no registers held across the quadrature loop):
-//   top of iteration k:  wait for what iteration k-1 issued -> coordinates / coefficients of cell k into registers;
-//                        active[e_(k+3)] -> register; ids of cell k+2 (cp.async, 4 B); coordinates, coefficients and
-//                        the ND^2 slots of cell k+1 (cp.async, 8 / 4 B; addresses from the ids that landed last time);
-//   then the quadrature loop of cell k and its scatter with the slots read from shared memory.
-// MEASURED at config C (16 M P2 triangles, profiles/round2_r4d_bench_*.json): 1.331 ms against 1.175 ms for the kernel
-// above (3 CTAs per SM 1.328, 5 CTAs 1.638) -- hiding the prologue and the slot loads buys nothing, the 60 cp.async and
-// their shared-memory reads per cell cost 13 %: the kernel is bound by the NUMBER of its scattered L2 reductions (42
-// per triangle), not by the latency in front of them.  Parity green (tests/test_gpu_assembly_pk.py with
-// -DPHIFEM_PK_PIPE=1); off by default.
-#ifndef PHIFEM_PK_PIPE
-#define PHIFEM_PK_PIPE 0
-#endif
-#ifndef PHIFEM_PK_PIPE_MINBLOCKS
-#define PHIFEM_PK_PIPE_MINBLOCKS 4
-#endif
-#if PHIFEM_PK_PIPE
-__device__ __forceinline__ void pk_cp_async4(void* smem, const void* gmem) {
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((uint32_t)__cvta_generic_to_shared(smem)), "l"(gmem)
-               : "memory");
-}
-__device__ __forceinline__ void pk_cp_async8(void* smem, const void* gmem) {
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((uint32_t)__cvta_generic_to_shared(smem)), "l"(gmem)
-               : "memory");
-}
-
-template <int D, int KW, int KP>
-__global__ void __launch_bounds__(kBlockPkCells, PHIFEM_PK_PIPE_MINBLOCKS) k_assemble_cells_pk_pipe(
-    phifem_mesh m, phifem_pk_space sw, phifem_pk_space sp, const double* __restrict__ qlam_g,
-    const double* __restrict__ qw_g, int nq, const double* __restrict__ phi, const double* __restrict__ f,
-    const int8_t* __restrict__ ctags, const int32_t* __restrict__ active, int64_t n_active,
-    const int32_t* __restrict__ slots, double sigma, double* __restrict__ data, double* __restrict__ b) {
-  constexpr int NV = D + 1, ND = Space<D, KW>::ND, NDP = Space<D, KP>::ND, B = kBlockPkCells;
-  constexpr int NVAL = NV * D + NDP + ND;   // coordinates, level-set coefficients, source coefficients
-  constexpr int NID = NV + ND + NDP;        // vertex ids, dof ids of the two spaces
-  static_assert(ND <= 6, "single-pass spaces only");
-  __shared__ double qlam[kMaxQuadPoints * NV], qw[kMaxQuadPoints];
-  __shared__ double val_s[NVAL * B];
-  __shared__ int32_t slot_s[2][ND * ND * B];
-  __shared__ int32_t id_s[2][NID * B];
-  for (int i = threadIdx.x; i < nq * NV; i += blockDim.x) qlam[i] = qlam_g[i];
-  for (int i = threadIdx.x; i < nq; i += blockDim.x) qw[i] = qw_g[i];
-  __syncthreads();
-  const int tid = threadIdx.x;
-  const int64_t T = (int64_t)gridDim.x * B;
-  const int64_t e0 = (int64_t)blockIdx.x * B + tid;
-  const int32_t* __restrict__ dmw = sw.dofmap ? sw.dofmap : m.cells;
-  const int32_t* __restrict__ dmp = sp.dofmap ? sp.dofmap : m.cells;
-
-  auto issue_ids = [&](int64_t c, int buf) {   // ids of cell c -> id_s[buf]
-    int32_t* dst = id_s[buf] + tid;
-#pragma unroll
-    for (int k = 0; k < NV; ++k) pk_cp_async4(dst + k * B, m.cells + c * NV + k);
-#pragma unroll
-    for (int k = 0; k < ND; ++k) pk_cp_async4(dst + (NV + k) * B, dmw + c * ND + k);
-#pragma unroll
-    for (int k = 0; k < NDP; ++k) pk_cp_async4(dst + (NV + ND + k) * B, dmp + c * NDP + k);
-  };
-  auto issue_values = [&](int64_t e, int buf) {   // coordinates / coefficients of the cell whose ids sit in id_s[buf], slots of e
-    const int32_t* ids = id_s[buf] + tid;
-    double* dst = val_s + tid;
-#pragma unroll
-    for (int k = 0; k < NV; ++k) {
-      const int64_t v = ids[k * B];
-#pragma unroll
-      for (int d = 0; d < D; ++d) pk_cp_async8(dst + (k * D + d) * B, m.x + v * D + d);
-    }
-#pragma unroll
-    for (int k = 0; k < NDP; ++k) pk_cp_async8(dst + (NV * D + k) * B, phi + ids[(NV + ND + k) * B]);
-#pragma unroll
-    for (int k = 0; k < ND; ++k) pk_cp_async8(dst + (NV * D + NDP + k) * B, f + ids[(NV + k) * B]);
-    int32_t* sl = slot_s[buf] + tid;
-#pragma unroll
-    for (int k = 0; k < ND * ND; ++k) pk_cp_async4(sl + k * B, slots + (int64_t)k * n_active + e);
-  };
-  auto commit = [] { asm volatile("cp.async.commit_group;" ::: "memory"); };
-  auto wait_all = [] { asm volatile("cp.async.wait_all;" ::: "memory"); };
-
-  // prime the pipeline: ids of cells 0 and 1, values of cell 0, active[] of cells 2 and 3
-  int64_t c2 = -1, c3 = -1;   // active[e_(k+2)], active[e_(k+3)] at the top of iteration k
-  int cut0 = 0, cut1 = 0, cut2 = 0;   // cell tags of cells k, k + 1, k + 2 (compared where they are used)
-  if (e0 < n_active) {
-    const int64_t c = __ldg(active + e0);
-    cut0 = ctags[c];
-    issue_ids(c, 0);
-  }
-  if (e0 + T < n_active) {
-    const int64_t c = __ldg(active + e0 + T);
-    cut1 = ctags[c];
-    issue_ids(c, 1);
-  }
-  if (e0 + 2 * T < n_active) c2 = __ldg(active + e0 + 2 * T);
-  if (e0 + 3 * T < n_active) c3 = __ldg(active + e0 + 3 * T);
-  commit();
-  wait_all();
-  if (e0 < n_active) issue_values(e0, 0);
-  commit();
-
-  int k = 0;
-  for (int64_t e = e0; e < n_active; e += T, ++k) {
-    const int buf = k & 1;
-    wait_all();   // values / slots of cell k, ids of cell k + 1
-    Geometry<D> g;
-    double pc[NDP], fc[ND];
-    int32_t dofs[ND];
-    {
-      const double* src = val_s + tid;
-#pragma unroll
-      for (int a = 0; a < NV; ++a)
-#pragma unroll
-        for (int d = 0; d < D; ++d) g.X[a][d] = src[(a * D + d) * B];
-#pragma unroll
-      for (int a = 0; a < NDP; ++a) pc[a] = src[(NV * D + a) * B];
-#pragma unroll
-      for (int a = 0; a < ND; ++a) fc[a] = src[(NV * D + NDP + a) * B];
-      const int32_t* ids = id_s[buf] + tid;
-#pragma unroll
-      for (int a = 0; a < ND; ++a) dofs[a] = ids[(NV + a) * B];
-    }
-    const bool is_cut = cut0 == 2;
-    // the loads of the next cells
-    if (c2 >= 0) {
-      cut2 = ctags[c2];
-      issue_ids(c2, buf);                         // ids of cell k + 2 (the ids of cell k are in registers now)
-    }
-    if (e + T < n_active) issue_values(e + T, buf ^ 1);
-    commit();
-    c2 = c3;
-    c3 = e + 4 * T < n_active ? (int64_t)__ldg(active + e + 4 * T) : -1;
-    cut0 = cut1;
-    cut1 = cut2;
-    geometry_from_vertices<D>(g);
-    cell_rows<D, KW, KP, 0, ND, true>(g, pc, fc, is_cut, sigma, qlam, qw, nq, slot_s[buf] + tid, B, dofs, data, b);
-  }
-  wait_all();
-}
-
-#endif  // PHIFEM_PK_PIPE
 
 // ---- one-sided boundary term: one thread per (entity, test dof i) ------------------------------------------
 //   A_ij = -int_F (grad(phi psi_j).n) phi psi_i    (main.py:106), n = outward normal of the entity's cell
@@ -551,58 +383,11 @@ __global__ void __launch_bounds__(kBlockPk) k_assemble_ghost_pk(
       for (int bb = 0; bb < NM; ++bb) E[bb] += wa * jq[bb];
     }
   }
-#if PHIFEM_PK_GHOST_DEDUPE
-  // The dofs on the facet appear on both sides of the macro element: of the NM^2 entries of E only (NM - NF)^2 land on
-  // distinct CSR entries (196 of 400 for the P2 tetrahedron), the others are 2 or 4 contributions of THIS facet to one
-  // entry -- same-address reductions issued by neighbouring threads at the same moment.  They are added up in shared
-  // memory first: twin rows / columns are recognised by their slots (row a and row a' are the same dof iff their
-  // entries in column 0 share a slot), every thread folds the twin columns of its own row, the first of two twin rows
-  // takes the other one in, and only the distinct entries go to memory.
-  constexpr int LD = NM + 1;                                            // padded row of Es
-  double* Es = Pq + (size_t)FPB * 2 * nq * NP;                           // [FPB][NM][LD]
-  int* twin = reinterpret_cast<int*>(Es + (size_t)FPB * NM * LD);        // [FPB][4][NM]: row sig, col sig, row twin, col twin
-  int* sig_r = twin + (size_t)(fl < FPB ? fl : 0) * 4 * NM;
-  int* sig_c = sig_r + NM, *tw_r = sig_c + NM, *tw_c = tw_r + NM;
-  double* row = Es + ((size_t)(fl < FPB ? fl : 0) * NM + a) * LD;
-  const int32_t* sl = slots + e * NM * NM;
-  if (live) {
-    sig_r[a] = __ldg(sl + a * NM);      // slot of (a, column 0)
-    sig_c[a] = __ldg(sl + a);           // slot of (row 0, a)
-#pragma unroll
-    for (int bb = 0; bb < NM; ++bb) row[bb] = E[bb];
-  }
-  __syncthreads();
-  if (live) {
-    int tr = a, tc = a;
-    for (int k = a - 1; k >= 0; --k) {
-      if (sig_r[k] == sig_r[a]) tr = k;
-      if (sig_c[k] == sig_c[a]) tc = k;
-    }
-    tw_r[a] = tr;
-    tw_c[a] = tc;
-  }
-  __syncthreads();
-  if (live) {
-    for (int bb = 0; bb < NM; ++bb) {   // fold the twin columns of this row (ascending: a twin points to a smaller index)
-      const int t = tw_c[bb];
-      if (t != bb) row[t] += row[bb];
-    }
-  }
-  __syncthreads();
-  if (live && tw_r[a] == a) {
-    for (int k = a + 1; k < NM; ++k)
-      if (tw_r[k] == a) {               // the other side's copy of this dof
-        const double* other = Es + ((size_t)fl * NM + k) * LD;
-        for (int bb = 0; bb < NM; ++bb) row[bb] += other[bb];
-      }
-    for (int bb = 0; bb < NM; ++bb)
-      if (tw_c[bb] == bb) atomicAdd(data + __ldg(sl + a * NM + bb), row[bb]);
-  }
-#else
+  // Adding the facet's duplicate entries up in shared memory first (400 -> 196 reductions per P2 tetrahedron facet)
+  // measured 1.253 against 1.040 ms at 3d-p2: the pass is not bound by its reductions (DESIGN.md §4, K2p).
   if (!live) return;
 #pragma unroll
   for (int bb = 0; bb < NM; ++bb) atomicAdd(data + __ldg(slots + (e * NM + a) * NM + bb), E[bb]);
-#endif
 }
 
 // ==== weak-Dirichlet (dual) phi-FEM operator on the mixed space (u, p) in P_KW x P_KW ========================
@@ -1096,16 +881,6 @@ extern "C" int phifem_assemble_cells_pk(const phifem_mesh* mesh, const phifem_pk
   cudaStream_t st = (cudaStream_t)stream;
   dispatch(mesh->cell_type, space_w->degree, space_phi->degree, [&](auto d, auto kw, auto kp) {
     constexpr int D = decltype(d)::value, KW = decltype(kw)::value, KP = decltype(kp)::value;
-#if PHIFEM_PK_PIPE
-    if constexpr (Space<D, KW>::ND <= 6) {
-      auto kernel = k_assemble_cells_pk_pipe<D, KW, KP>;
-      const int grid = persistent_grid(kernel, kBlockPkCells, (n_active + kBlockPkCells - 1) / kBlockPkCells);
-      kernel<<<grid, kBlockPkCells, 0, st>>>(*mesh, *space_w, *space_phi, quad->cell_points, quad->cell_weights,
-                                            quad->n_cell_points, phi, f, cell_tags8, active, n_active, slots, sigma,
-                                            data, b);
-      return;
-    }
-#endif
     const dim3 grid((unsigned)((n_active + kBlockPkCells - 1) / kBlockPkCells), Passes<Space<D, KW>::ND>::N);
     k_assemble_cells_pk<D, KW, KP><<<grid, kBlockPkCells, 0, st>>>(
         *mesh, *space_w, *space_phi, quad->cell_points, quad->cell_weights, quad->n_cell_points, phi, f,
@@ -1169,10 +944,7 @@ extern "C" int phifem_assemble_ghost_pk(const phifem_mesh* mesh, const phifem_pk
     constexpr int D = decltype(d)::value, KW = decltype(kw)::value, KP = decltype(kp)::value;
     constexpr int FPB = GhostLayout<D, KW>::FPB, NM = GhostLayout<D, KW>::NM;
     const int nq = quad->n_facet_points;
-    size_t smem = sizeof(double) * ((size_t)nq * (D + 1) + (size_t)FPB * nq * (NM + 2 * (D + 3)));
-#if PHIFEM_PK_GHOST_DEDUPE
-    smem += sizeof(double) * (size_t)FPB * NM * (NM + 1) + sizeof(int) * (size_t)FPB * 4 * NM;
-#endif
+    const size_t smem = sizeof(double) * ((size_t)nq * (D + 1) + (size_t)FPB * nq * (NM + 2 * (D + 3)));
     if (smem > 48 * 1024)
       cudaFuncSetAttribute(k_assemble_ghost_pk<D, KW, KP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     k_assemble_ghost_pk<D, KW, KP><<<(unsigned)((n_facets + FPB - 1) / FPB), kBlockPk, smem, st>>>(

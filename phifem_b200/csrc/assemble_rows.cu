@@ -25,22 +25,8 @@ namespace {
 
 // 64 threads x 8 CTAs per SM (the same 16 warps and 128 registers as 128 x 4): cell pass 1.200 -> 1.174 ms at config E
 // (profiles/round2_i_rows_variants.md, tools/r3_run_h.sh) -- half the accumulator slab per CTA, finer-grained tail
-#ifndef PHIFEM_ROWS_BLOCK
-#define PHIFEM_ROWS_BLOCK 64
-#endif
-constexpr int kRowsBlock = PHIFEM_ROWS_BLOCK;
-#ifndef PHIFEM_ROWS_MINBLOCKS
-#define PHIFEM_ROWS_MINBLOCKS (512 / PHIFEM_ROWS_BLOCK)
-#endif
-#ifndef PHIFEM_SURF_MINBLOCKS
-#define PHIFEM_SURF_MINBLOCKS PHIFEM_ROWS_MINBLOCKS
-#endif
-#ifndef PHIFEM_SURF_DEPTH
-#define PHIFEM_SURF_DEPTH 2
-#endif
-#ifndef PHIFEM_ONCE_MINBLOCKS
-#define PHIFEM_ONCE_MINBLOCKS 1
-#endif
+constexpr int kRowsBlock = 64;
+constexpr int kRowsMinBlocks = 512 / kRowsBlock;
 constexpr uint32_t kPad = 0xffffffffu;
 
 // Row 0 of the cell tensor of simplex X (local vertex 0 = the row's vertex): dx((1,2)) stiffness,
@@ -273,7 +259,7 @@ __device__ __forceinline__ void ldg256(const double* p, double& a, double& b, do
 }
 
 template <int D>
-__global__ void __launch_bounds__(kRowsBlock, PHIFEM_ONCE_MINBLOCKS) k_surface_once_p1(
+__global__ void __launch_bounds__(kRowsBlock, 1) k_surface_once_p1(
     const double* __restrict__ x, const double* __restrict__ phi, double sigma,
     const int32_t* __restrict__ macro, int64_t n_facets, const int32_t* __restrict__ entity_macro,
     int64_t n_entities, double* __restrict__ work) {
@@ -521,7 +507,7 @@ struct OthersGeom {
 
 // One pass over one row list.  KIND == kCells writes data / b of its rows, the surface passes add to them.
 template <int D, int KIND>
-__global__ void __launch_bounds__(kRowsBlock, KIND == 1 ? PHIFEM_SURF_MINBLOCKS : PHIFEM_ROWS_MINBLOCKS) k_assemble_rows_p1(
+__global__ void __launch_bounds__(kRowsBlock, kRowsMinBlocks) k_assemble_rows_p1(
     const double* __restrict__ x, const double* __restrict__ phi, const double* __restrict__ f,
     double sigma, const int32_t* __restrict__ indptr, const int32_t* __restrict__ indices,
     phifem_row_list rl, const double* __restrict__ surface_work, double* __restrict__ data,
@@ -706,33 +692,8 @@ __global__ void __launch_bounds__(kRowsBlock, KIND == 1 ? PHIFEM_SURF_MINBLOCKS 
       for (int j = 0; j < NG - 1; ++j)  // j-th other macro vertex = macro index j (j < a) or j + 1
         acc[((rec.x >> (8 * j)) & 0xff) * kRowsBlock] += j < a ? K[j] : K[j + 1];
     };
-#if PHIFEM_SURF_DEPTH == 3
-    // three work buffers: the records of facets k + 1 and k + 2 are in flight while record k is evaluated (the pass is
-    // bound by the latency of these L2 gathers: long-scoreboard stalls 7.6 per issue with two buffers)
-    double wa[W], wb[W], wc[W];
-    uint2 w0 = fetch_rec(kb), w1 = fetch_rec(kb + 1), w2 = fetch_rec(kb + 2), w3 = fetch_rec(kb + 3),
-          w4 = fetch_rec(kb + 4), w5 = fetch_rec(kb + 5);
-    if (kb < ke) {
-      fetch_work(w0, wa);
-      fetch_work(w1, wb);
-    }
-    auto body = [&](int k, const double (&cur)[W], double (&nxt)[W]) {
-      const uint2 rec = w0;
-      fetch_work(w2, nxt);
-      w0 = w1;
-      w1 = w2;
-      w2 = w3;
-      w3 = w4;
-      w4 = w5;
-      w5 = fetch_rec(k + 6);
-      evaluate(rec, cur);
-    };
-    for (int k = kb; k < ke; k += 3) {
-      body(k, wa, wc);
-      if (k + 1 < ke) body(k + 1, wb, wa);
-      if (k + 2 < ke) body(k + 2, wc, wb);
-    }
-#else
+    // a third work buffer (the records of two facets in flight) measured 0.242 against 0.236 ms: the pass is not bound
+    // by the latency of these gathers (DESIGN.md §4, K2+K3+K4)
     double wa[W], wb[W];
     uint2 w0 = fetch_rec(kb), w1 = fetch_rec(kb + 1), w2 = fetch_rec(kb + 2), w3 = fetch_rec(kb + 3),
           w4 = fetch_rec(kb + 4);
@@ -751,7 +712,6 @@ __global__ void __launch_bounds__(kRowsBlock, KIND == 1 ? PHIFEM_SURF_MINBLOCKS 
       body(k, wa, wb);
       if (k + 1 < ke) body(k + 1, wb, wa);
     }
-#endif
   }
   acc[dpos * kRowsBlock] += diag;
   if constexpr (KIND != kSurface) {

@@ -23,18 +23,9 @@
 namespace phifem {
 namespace {
 
-#ifndef PHIFEM_TILES_MINBLOCKS
-#define PHIFEM_TILES_MINBLOCKS 2
-#endif
-#ifndef PHIFEM_TILES_MINBLOCKS_128
-#define PHIFEM_TILES_MINBLOCKS_128 4
-#endif
-#ifndef PHIFEM_PUSH_BATCH
-#define PHIFEM_PUSH_BATCH 1
-#endif
-#ifndef PHIFEM_PUSH_RACY
-#define PHIFEM_PUSH_RACY 0
-#endif
+// CTAs per SM of the tile kernels at R = 256 / 128 threads
+constexpr int kTilesMinBlocks = 2;
+constexpr int kTilesMinBlocks128 = 4;
 
 // Whole element tensor of simplex X: K[i * NV + j] at out[(i * NV + j) * stride], b[i] at out[(NV * NV + i) * stride].
 //   K_ij = |K|/((d+1)(d+2)) [ |g|^2 (1 + delta_ij) + a_i (P + p_j) + (P + p_i) a_j + G_i.G_j mu ] + 4 sigma h^2 |K| a_i a_j
@@ -130,7 +121,7 @@ __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wai
 // vertex ids of the chunk after it are being fetched -- the only global latency left on the critical path of a chunk is
 // the barrier itself.
 template <int D, int R>
-__global__ void __launch_bounds__(R, R == 128 ? PHIFEM_TILES_MINBLOCKS_128 : PHIFEM_TILES_MINBLOCKS) k_assemble_tiles_p1(
+__global__ void __launch_bounds__(R, R == 128 ? kTilesMinBlocks128 : kTilesMinBlocks) k_assemble_tiles_p1(
     const double* __restrict__ x, const double* __restrict__ phi, const double* __restrict__ f, double sigma,
     const int32_t* __restrict__ indptr, phifem_cell_tiles tl, int max_row_nnz, double* __restrict__ data,
     double* __restrict__ b) {
@@ -274,7 +265,7 @@ __global__ void __launch_bounds__(R, R == 128 ? PHIFEM_TILES_MINBLOCKS_128 : PHI
 //   bits 0-7 = its index l in the tile, 7 bits from bit 10 + 7 m = position inside row l's column list of the cell's
 //   m-th OTHER vertex (ascending cell-local order).
 template <int D, int R>
-__global__ void __launch_bounds__(R, R == 128 ? PHIFEM_TILES_MINBLOCKS_128 : PHIFEM_TILES_MINBLOCKS) k_assemble_push_p1(
+__global__ void __launch_bounds__(R, R == 128 ? kTilesMinBlocks128 : kTilesMinBlocks) k_assemble_push_p1(
     const double* __restrict__ x, const double* __restrict__ phi, const double* __restrict__ f, double sigma,
     const int32_t* __restrict__ indptr, phifem_cell_tiles tl, int max_row_nnz, double* __restrict__ data,
     double* __restrict__ b) {
@@ -350,17 +341,9 @@ __global__ void __launch_bounds__(R, R == 128 ? PHIFEM_TILES_MINBLOCKS_128 : PHI
             dst[2 + m] = acc_s + ((w >> (10 + 7 * m)) & 0x7f) * R + l;
             v[2 + m] = out[i * NV + j];
           }
-#if PHIFEM_PUSH_RACY
-          // TIMING EXPERIMENT ONLY (wrong results): plain load / add / store -- what the pass would cost if the cells
-          // running concurrently never shared a row (a vertex-disjoint colouring of each tile's cells)
-          double cur[D + 2];
-#pragma unroll
-          for (int e = 0; e < D + 2; ++e) cur[e] = *reinterpret_cast<volatile double*>(dst[e]);
-#pragma unroll
-          for (int e = 0; e < D + 2; ++e) *reinterpret_cast<volatile double*>(dst[e]) = cur[e] + v[e];
-#elif PHIFEM_PUSH_BATCH
           // the D + 2 updates of a row as ONE batch: loads, sums, compare-and-swaps issued back to back (a
-          // compiler-generated atomicAdd is a dependent LDS -> DADD -> CAS chain each); the rare loser retries alone
+          // compiler-generated atomicAdd is a dependent LDS -> DADD -> CAS chain each); the rare loser retries alone.
+          // Plain atomicAdd loops measured 2.582 against 2.846 ms at R = 256 (DESIGN.md §4, K2'').
           unsigned long long seen[D + 2], want[D + 2];
 #pragma unroll
           for (int e = 0; e < D + 2; ++e) seen[e] = *reinterpret_cast<volatile unsigned long long*>(dst[e]);
@@ -372,10 +355,6 @@ __global__ void __launch_bounds__(R, R == 128 ? PHIFEM_TILES_MINBLOCKS_128 : PHI
 #pragma unroll
           for (int e = 0; e < D + 2; ++e)
             if (want[e] != seen[e]) atomicAdd(dst[e], v[e]);
-#else
-#pragma unroll
-          for (int e = 0; e < D + 2; ++e) atomicAdd(dst[e], v[e]);
-#endif
         }
       }
     }

@@ -12,13 +12,7 @@ namespace phifem {
 namespace {
 
 constexpr int kSpmvBlock = 256;
-#ifndef PHIFEM_SPMV_LANES
-#define PHIFEM_SPMV_LANES 8
-#endif
-constexpr int kLanesPerRow = PHIFEM_SPMV_LANES;
-#ifndef PHIFEM_SPMV_BATCH
-#define PHIFEM_SPMV_BATCH 4
-#endif
+constexpr int kLanesPerRow = 8;
 
 __global__ void __launch_bounds__(kSpmvBlock) k_csr_spmv(int64_t n_rows, const int32_t* __restrict__ indptr,
                                                          const int32_t* __restrict__ indices,
@@ -104,28 +98,26 @@ __global__ void __launch_bounds__(kSpmvBlock) k_spmv_rows_dot(int64_t n_act, con
     if (i < n_act) {
       const int row = __ldg(rows + i);
       const int lo = __ldg(indptr + row), hi = __ldg(indptr + row + 1);
-#if PHIFEM_SPMV_BATCH > 1
-      // PHIFEM_SPMV_BATCH entries per lane at a time: their column ids and values are requested together, then the gathers
-      // of x, then the products -- a lane's trip through a 15-entry row is one batch instead of four dependent
-      // load -> load -> fma rounds
-      for (int k0 = lo + sub; k0 < hi; k0 += PHIFEM_SPMV_BATCH * L) {
-        int c[PHIFEM_SPMV_BATCH];
-        double a[PHIFEM_SPMV_BATCH], xv[PHIFEM_SPMV_BATCH];
+      // kBatch entries per lane at a time: their column ids and values are requested together, then the gathers of x,
+      // then the products -- a lane's trip through a 15-entry row is one batch instead of four dependent
+      // load -> load -> fma rounds (430 iterations at config E: 193.5 ms with one entry at a time, 182.2 with two,
+      // 180.3 with four; DESIGN.md §4)
+      constexpr int kBatch = 4;
+      for (int k0 = lo + sub; k0 < hi; k0 += kBatch * L) {
+        int c[kBatch];
+        double a[kBatch], xv[kBatch];
 #pragma unroll
-        for (int u = 0; u < PHIFEM_SPMV_BATCH; ++u) {
+        for (int u = 0; u < kBatch; ++u) {
           const int k = k0 + u * L;
           const bool in = k < hi;
           c[u] = in ? __ldg(cols + k) : (int)n_act;   // x[n_act] = 0 by contract (the slot of the inactive columns)
           a[u] = in ? __ldg(data + k) : 0.0;
         }
 #pragma unroll
-        for (int u = 0; u < PHIFEM_SPMV_BATCH; ++u) xv[u] = __ldg(x + c[u]);
+        for (int u = 0; u < kBatch; ++u) xv[u] = __ldg(x + c[u]);
 #pragma unroll
-        for (int u = 0; u < PHIFEM_SPMV_BATCH; ++u) acc += a[u] * xv[u];
+        for (int u = 0; u < kBatch; ++u) acc += a[u] * xv[u];
       }
-#else
-      for (int k = lo + sub; k < hi; k += L) acc += __ldg(data + k) * __ldg(x + __ldg(cols + k));
-#endif
     }
 #pragma unroll
     for (int off = L / 2; off > 0; off >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, off, L);

@@ -155,9 +155,7 @@ struct BlockCounters {
 // sequential sum (all terms share a sign => num == +-den exactly).
 // HBM-latency bound: every thread keeps kUnroll independent cells in flight (index loads first, then
 // all gathers), counters stay in registers until the end of the grid-stride loop.
-#ifndef PHIFEM_TAG_CELLS_MINBLOCKS
-#define PHIFEM_TAG_CELLS_MINBLOCKS 3
-#endif
+constexpr int kTagCellsMinBlocks = 3;
 constexpr int kUnroll = 4;
 
 // exact path for cells the sign test cannot decide; scalars in / packed (tag | zden << 8) out so
@@ -217,7 +215,7 @@ __global__ void __launch_bounds__(kBlock) k_vertex_class(const double* __restric
 }
 
 template <int CT>
-__global__ void __launch_bounds__(kBlock, PHIFEM_TAG_CELLS_MINBLOCKS) k_tag_cells_p1(phifem_mesh m, const double* __restrict__ phi,
+__global__ void __launch_bounds__(kBlock, kTagCellsMinBlocks) k_tag_cells_p1(phifem_mesh m, const double* __restrict__ phi,
                                                             const uint8_t* __restrict__ vclass,
                                                             bool exact_zero_den,
                                                             int32_t* __restrict__ tags,
@@ -335,20 +333,15 @@ __global__ void __launch_bounds__(kBlock, PHIFEM_TAG_CELLS_MINBLOCKS) k_tag_cell
 // cells, i.e. a handful of sectors of the class array); the tag bytes of a tile are collected in shared memory and leave
 // as one coalesced 32-bit word per thread AFTER the next tile's barrier, when the exact path has filled in the parked
 // cells (three 1 KB output buffers rotate so that one barrier per tile suffices).
-#ifndef PHIFEM_TAG_CELLS_STAGES
-#define PHIFEM_TAG_CELLS_STAGES 2
-#endif
-#ifndef PHIFEM_TAG_CELLS_STAGED_MINBLOCKS
-#define PHIFEM_TAG_CELLS_STAGED_MINBLOCKS 4
-#endif
-constexpr int kCellStages = PHIFEM_TAG_CELLS_STAGES;
+constexpr int kCellStages = 2;
+constexpr int kTagCellsStagedMinBlocks = 4;
 constexpr int kCellTile = kBlock * kUnroll;
 template <int CT> constexpr size_t staged_cells_smem() {
   return (size_t)kCellStages * kCellTile * CellTraits<CT>::nv * sizeof(int32_t);
 }
 
 template <int CT>
-__global__ void __launch_bounds__(kBlock, PHIFEM_TAG_CELLS_STAGED_MINBLOCKS) k_tag_cells_p1_staged(
+__global__ void __launch_bounds__(kBlock, kTagCellsStagedMinBlocks) k_tag_cells_p1_staged(
     phifem_mesh m, const double* __restrict__ phi, const uint8_t* __restrict__ vclass, bool exact_zero_den,
     int32_t* __restrict__ tags, int8_t* __restrict__ tags8, int64_t* counters) {
   using T = CellTraits<CT>;
@@ -927,17 +920,12 @@ __global__ void __launch_bounds__(kBlock) k_tag_boundary_facets_rec(phifem_mesh 
 // facet tags as one 32-bit word.  Against the per-thread LDG.128 loop of k_tag_facets (each warp instruction touching 32
 // half-used sectors, bytes in flight tied to the resident warps' loop phase) the requests for f2c leave the SM as whole
 // 8 KB copies issued three tiles ahead.
-#ifndef PHIFEM_TAG_FACETS_STAGES
-#define PHIFEM_TAG_FACETS_STAGES 4
-#endif
-#ifndef PHIFEM_TAG_FACETS_MINBLOCKS
-#define PHIFEM_TAG_FACETS_MINBLOCKS 5
-#endif
-constexpr int kFacetStages = PHIFEM_TAG_FACETS_STAGES;
+constexpr int kFacetStages = 4;
+constexpr int kTagFacetsMinBlocks = 5;
 constexpr int kFacetTile = kBlock * kUnroll;
 
 template <int CT>
-__global__ void __launch_bounds__(kBlock, PHIFEM_TAG_FACETS_MINBLOCKS) k_tag_facets_staged(
+__global__ void __launch_bounds__(kBlock, kTagFacetsMinBlocks) k_tag_facets_staged(
     phifem_mesh m, const int8_t* __restrict__ ctags, int32_t* __restrict__ ftags, int8_t* __restrict__ ftags8,
     int64_t* counters) {
   constexpr unsigned long long kTagLut = interior_facet_lut(false);
@@ -1305,13 +1293,10 @@ extern "C" int phifem_tag_facets_phase(const phifem_mesh* mesh, const phifem_lev
       int grid = persistent_grid(k_tag_facets_staged<CT>, kBlock, tiles);
       // Beside the forked mesh-boundary kernel the persistent grid gives up one CTA per SM (5 of 6): the streaming
       // kernel alone is 7 % slower that way (0.161 against 0.150 ms at config E) but the latency-bound boundary kernel
-      // then runs entirely under it: both phases 0.168 against 0.178 ms (tools/r3_run_x.sh; 4 per SM: 0.187).
+      // then runs entirely under it: both phases 0.168 against 0.178 ms (4 per SM: 0.187), measured with a grid-size
+      // override that has since been removed (it is in the history).
       int per_sm = grid / kNumSMs;
       if (beside_boundary && per_sm >= 4 && grid % kNumSMs == 0) grid -= kNumSMs;
-      if (const char* e = getenv("PHIFEM_FACETS_CTAS_PER_SM")) {  // tuning runs
-        const int64_t cap = (int64_t)kNumSMs * atoi(e);
-        if (cap > 0) grid = (int)(cap < tiles ? cap : tiles);
-      }
       k_tag_facets_staged<CT><<<grid, kBlock, 0, st>>>(*mesh, cell_tags8, facet_tags, facet_tags8, counters);
     } else {
       const int grid = persistent_grid(k_tag_facets<CT, false>, kBlock, tiles);

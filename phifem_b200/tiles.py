@@ -5,8 +5,6 @@ threads per CTA); a tile's cells = the active cells touching one of its rows, in
 a record per (row, cell) names the cell's slot in its chunk and where the cell's other vertices sit in the row's column
 list.  Sort / scatter plumbing with torch ops on the mesh's device (CPU tensors work: tests/test_tiles_symbolic.py).
 """
-import os
-
 import torch
 
 from . import _lib
@@ -16,17 +14,13 @@ MAX_ROW_NNZ = 128            # positions are 7 bits
 
 
 class CellTiles:
-    def __init__(self, mesh, active, cut, slots_cells, indptr, rows, diag_pos, rows_per_tile=ROWS_PER_TILE, push=False,
-                 interleave=None):
+    def __init__(self, mesh, active, cut, slots_cells, indptr, rows, diag_pos, rows_per_tile=ROWS_PER_TILE, push=False):
         """active [Na] int: active cells ascending; cut [Na] 0/1; slots_cells [Na, nv*nv] CSR slot of (row i, col j);
         indptr [n+1] int64; rows [L] int64 listed rows in processing order; diag_pos [L] uint8."""
         if rows_per_tile not in (128, 256):
             raise ValueError("rows_per_tile must be 128 or 256")
         dev = rows.device
         i64 = dict(dtype=torch.int64, device=dev)
-        if interleave is None:
-            interleave = os.environ.get("PHIFEM_PUSH_INTERLEAVE", "0") == "1"
-        self.interleave = bool(push and interleave)
         R = self.rows_per_tile = int(rows_per_tile)
         nv = mesh.cells.shape[1]
         n = indptr.numel() - 1
@@ -54,11 +48,6 @@ class CellTiles:
         self.n_active = na
         first = torch.cumsum(cnt, 0) - cnt
         rank = torch.arange(ukey.numel(), **i64) - first[pt]
-        if push and interleave:
-            # lanes of a warp take cells `stride` apart in the tile's list instead of neighbours (which share vertices
-            # and collide on the same accumulators): rank -> (rank % stride) * 32 + rank // stride, stride = ceil(cnt / 32)
-            stride = ((cnt + 31) // 32).clamp(min=1)[pt]
-            rank = (rank % stride) * 32 + rank // stride
         slot = chunk_ptr[pt] * R + rank
         sv = torch.full((max(nch, 1) * R, 4), -1, **i64)
         verts = cells_act[pa]
