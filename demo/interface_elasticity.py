@@ -2,6 +2,7 @@
 """The reference's interface-elasticity demo on the GPU (BASELINE.json configs[3]):
 
     python demo/interface_elasticity.py [--mesh-size 0.2] [--iterations 4] [--solver direct|bicgstab]
+                                        [--cell-type triangle|quadrilateral]
 
 mirrors `python main.py param1` of reference demo/interface-elasticity/main.py with param1.yaml: background mesh of the
 box [-1.5, 1.5]^2 (main.py:92-107), tags in box mode (:111-115), mixed space (u_in, u_out, y_in, y_out, p) (:119-129),
@@ -12,6 +13,9 @@ on the cells instead of a P3 interpolant), uniform refinement between iterations
 The tags and the assembly (matrix, right-hand side, lifting) run on the GPU; the linear solve is the step after the
 path: `direct` hands the CSR system to scipy's sparse LU on the host (the reference uses MUMPS), `bicgstab` keeps it on
 the GPU (Jacobi-BiCGStab; the least-squares penalty terms make the system ill-conditioned, so expect many iterations).
+
+--cell-type quadrilateral runs the same steps on n^2 quadrilaterals of the same box: every field of the mixed space and
+the level set Q1; the errors are integrated by 4 x 4 Gauss points on the bilinear cells.
 """
 import argparse
 import os
@@ -84,12 +88,47 @@ def errors(mesh, tags, u_in, u_out, mat):
     return (l2 / n_l2) ** 0.5, (h1 / n_h1) ** 0.5
 
 
-def main(mesh_size=0.2, iterations=4, solver="direct", pen_coef=1.0, stab_coef=1.0, quiet=False):
+def errors_quad(mesh, tags, u_in, u_out, mat):
+    """`errors` on a quadrilateral mesh: 4 x 4 Gauss points on each bilinear cell, Q1 values and physical gradients
+    J^-T grad_ref at every point."""
+    pts, wq = quadrature.square_rule(4)
+    xi, eta = pts[:, 0], pts[:, 1]
+    N = np.stack([(1 - xi) * (1 - eta), xi * (1 - eta), (1 - xi) * eta, xi * eta], axis=1)            # [q, 4]
+    dN = np.stack([np.stack([-(1 - eta), 1 - eta, -eta, eta], axis=1),
+                   np.stack([-(1 - xi), -xi, 1 - xi, xi], axis=1)], axis=2)                           # [q, 4, 2]
+    X = mesh.x.cpu().numpy()
+    cells = mesh.cells.cpu().numpy()
+    l2 = h1 = n_l2 = n_h1 = 0.0
+    for tag, uh in ((1, u_in), (3, u_out)):
+        cc = cells[tags == tag]
+        xc = X[cc]                                          # [m, 4, 2]
+        J = np.einsum("mkr,qkc->mqrc", xc, dN)              # J[r, c] = d x_r / d ref_c
+        det = J[..., 0, 0] * J[..., 1, 1] - J[..., 0, 1] * J[..., 1, 0]
+        G = np.einsum("qkc,mqcr->mqkr", dN, np.linalg.inv(J))             # physical gradients of the Q1 basis
+        xq = np.einsum("qk,mkd->mqd", N, xc).reshape(-1, 2)
+        ue, ge = exact_solution(xq, mat)
+        ue, ge = ue.reshape(len(cc), len(wq), 2), ge.reshape(len(cc), len(wq), 2)
+        uq = np.einsum("qk,mkc->mqc", N, uh[cc])
+        gh = np.einsum("mqkj,mkc->mqcj", G, uh[cc])         # d_j u_c
+        w = wq[None, :] * np.abs(det)
+        l2 += float((w[:, :, None] * (uq - ue) ** 2).sum())
+        n_l2 += float((w[:, :, None] * ue ** 2).sum())
+        h1 += float((w[:, :, None, None] * (gh - ge[:, :, None, :]) ** 2).sum())
+        n_h1 += float((w[:, :, None, None] * np.repeat(ge[:, :, None, :], 2, axis=2) ** 2).sum())
+    return (l2 / n_l2) ** 0.5, (h1 / n_h1) ** 0.5
+
+
+def main(mesh_size=0.2, iterations=4, solver="direct", pen_coef=1.0, stab_coef=1.0, quiet=False,
+         cell_type="triangle"):
+    if cell_type not in ("triangle", "quadrilateral"):
+        raise ValueError("cell_type must be 'triangle' or 'quadrilateral'")
     mat = elasticity.Material(E_in=1.0, nu_in=0.3, E_out=0.001, nu_out=0.3)            # data.py:13-22
     n = int(3.0 / mesh_size)                                                            # main.py:92-93
     results = {"dof": [], "L2 relative error": [], "H10 relative error": []}
+    make_mesh = synthetic.quadrilateral_mesh if cell_type == "quadrilateral" else synthetic.rectangle_mesh
+    error_norms = errors_quad if cell_type == "quadrilateral" else errors
     for _ in range(iterations):
-        mesh = synthetic.rectangle_mesh(n, lo=(-1.5, -1.5), hi=(1.5, 1.5))
+        mesh = make_mesh(n, lo=(-1.5, -1.5), hi=(1.5, 1.5))
         V = fem.functionspace(mesh, ("Lagrange", 1))
         phi_h = fem.Function(V, levelset(mesh.x))
         with warnings.catch_warnings():
@@ -116,7 +155,7 @@ def main(mesh_size=0.2, iterations=4, solver="direct", pen_coef=1.0, stab_coef=1
             sol, info = torch.from_numpy(s), "direct (scipy LU on %d of %d rows)" % (len(keep), M.shape[0])
         u_in, u_out, *_ = plan.split(sol)
         tags = cells_tags.values_dev.cpu().numpy()
-        l2, h1 = errors(mesh, tags, u_in.numpy(), u_out.numpy(), mat)
+        l2, h1 = error_norms(mesh, tags, u_in.numpy(), u_out.numpy(), mat)
         results["dof"].append(2 * mesh.num_vertices)
         results["L2 relative error"].append(l2)
         results["H10 relative error"].append(h1)
@@ -133,5 +172,6 @@ if __name__ == "__main__":
     ap.add_argument("--mesh-size", type=float, default=0.2)
     ap.add_argument("--iterations", type=int, default=4)
     ap.add_argument("--solver", choices=("direct", "bicgstab"), default="direct")
+    ap.add_argument("--cell-type", choices=("triangle", "quadrilateral"), default="triangle")
     a = ap.parse_args()
-    main(a.mesh_size, a.iterations, a.solver)
+    main(a.mesh_size, a.iterations, a.solver, cell_type=a.cell_type)

@@ -502,14 +502,24 @@ int phifem_assemble_neumann_ghost(const phifem_mesh* mesh, const phifem_quadratu
 
 /* ---- interface-elasticity phi-FEM operator on the mixed space (u_in, u_out, y_in, y_out, p) in
  * P1^d x P1^d x P1^(d x d) x P1^(d x d) x P1^d: demo/interface-elasticity/main.py:152-274 (`assemble_matrix(form(a), bcs)`
- * :238-240, `assemble_vector(form(L))` :271, `apply_lifting` / `bc.set` :273-275), triangles and tetrahedra, P1 or P2
- * level set.  Every field is nodal, so the mixed space has NB = 3 d + 2 d^2 dofs per vertex: global dof = NB vertex + o,
+ * :238-240, `assemble_vector(form(L))` :271, `apply_lifting` / `bc.set` :273-275), triangles, quadrilaterals and
+ * tetrahedra, P1 (Q1) or P2 (Q2) level set.  Every field is nodal, so the mixed space has NB = 3 d + 2 d^2 dofs per vertex: global dof = NB vertex + o,
  * o: u_in c -> c, u_out c -> d + c, y_in (r,s) -> 2d + r d + s, y_out (r,s) -> 2d + d^2 + r d + s, p c -> 2d + 2d^2 + c.
  * The CSR matrix is the vertex graph (`vptr` [n_vertices + 1], sorted neighbour lists: vertex pairs of every tagged cell
  * and of the macro elements of the interior facets tagged 3 / 4) with dense NB x NB blocks: entry (NB r + a, NB s + b)
  * at NB (NB vptr[r] + a deg(r) + pos) + b, pos = rank of s among r's neighbours.  Slot maps hold `pos` per vertex pair:
  * cells [n_cells, nv*nv], facets [n, (2 nv)^2] (macro order [vertices of cell +, of cell -]), entities [n, nv*nv]
- * (row = test vertex).  `f` is a P1 vector field [n_vertices, d].  ADD semantics; `data` / `b` zeroed by the caller. */
+ * (row = test vertex).  `f` is a P1 vector field [n_vertices, d].  ADD semantics; `data` / `b` zeroed by the caller.
+ *
+ * Quadrilaterals (mesh->cell_type == PHIFEM_QUADRILATERAL, gdim 2, vertices in tensor order): every field is Q1 on the
+ * bilinear cell (NB = 14, nv = 4 in the slot maps) and `f` is Q1 (vertex values).  There
+ *   - phifem_quadrature.cell_points holds REFERENCE coordinates (xi, eta) [n_cell_points, 2] on [0,1]^2, weights summing
+ *     to 1: the rule of the cut cells (phifem_b200/quadrature.py rules_for_elasticity_quad, (kphi + 2)^2 Gauss points);
+ *   - the cells tagged 1 / 3 are integrated by a fixed 2 x 2 Gauss rule, the stress jump by a fixed 2-point Gauss rule on
+ *     the edge (compile-time constants, exact on parallelograms), the one-sided terms in closed form;
+ *   - space_phi->n_dofs_per_cell must be 4 (Q1, degree 1) or 9 (Q2, degree 2, dolfinx-local order); any other value
+ *     returns PHIFEM_ERR_ARGUMENT;
+ *   - cells must be convex (either orientation); a non-convex quadrilateral is outside the method and not checked. */
 typedef struct phifem_elasticity_params {
   double lmbda_in, mu_in;    /* Lame coefficients of data.py:5-22 */
   double lmbda_out, mu_out;

@@ -21,10 +21,18 @@
 // (T_in = y_in + sigma_in(u_in), T_out, R = (y_in - y_out) grad phi, S = u_in - u_out + p phi / h, div y_in, div y_out)
 // are a small runtime bundle; the NB test offsets are unrolled at compile time, so that each contraction holds only the
 // non-zero terms of its field.  Consecutive threads write consecutive CSR entries.
+//
+// Quadrilaterals (gdim 2, vertices in tensor order): every field is Q1 on the bilinear cell (NB = 14, 4 vertices per
+// cell, the same global numbering) and the level set Q1 or Q2.  The quadrature rule's cell_points are reference
+// coordinates (xi, eta) on [0, 1]^2 and integrate the cut cells (quadrature.rules_for_elasticity_quad: (kphi + 2)^2
+// Gauss points); the uncut cells use a fixed 2 x 2 Gauss rule and the stress jump a fixed 2-point Gauss rule on the edge,
+// both compile-time constants; the one-sided terms have a closed form.  The bundle and the contractions above serve both
+// cell types: they take point values and physical gradients of a nodal basis.
 #include <utility>
 
 #include "common.cuh"
 #include "pk_common.cuh"
+#include "quad_common.cuh"
 
 namespace phifem {
 using namespace pk;
@@ -414,6 +422,291 @@ __global__ void __launch_bounds__(kBlockEl) k_elasticity_boundary(
       atomicAdd(data + block_address(vptr, vk, ou + cc, pos, oy + cc * D + s, NB), n[s] * mkj);
 }
 
+// ==== quadrilaterals: bilinear cells, every field Q1 (NB = 14 dofs per vertex, 4 vertices per cell) ==================
+// Nothing is affine, so every integral is a quadrature at reference points (xi, eta) mapped by quad::map_point.  The
+// uncut cells and the stress jump use fixed Gauss rules, exact on a parallelogram: 2 x 2 points on the cell (the
+// stiffness and the load have degree 2 per reference direction) and 2 on the edge (sigma(u) n is linear along it).
+constexpr double kGauss2Lo = 0.21132486540518711775, kGauss2Hi = 0.78867513459481288225;   // (1 -+ 1/sqrt(3)) / 2
+
+// row n of G [4][2] at a runtime index, without local memory
+__device__ __forceinline__ void pick_row(const double (&G)[quad::NV][2], int n, double (&out)[2]) {
+  out[0] = G[0][0];
+  out[1] = G[0][1];
+#pragma unroll
+  for (int q = 1; q < quad::NV; ++q)
+    if (q == n) {
+      out[0] = G[q][0];
+      out[1] = G[q][1];
+    }
+}
+
+// sigma(N e_c) n = lmbda G[c] n + mu (G n[c] + e_c (G.n)) for the gradient G of a scalar nodal function N
+__device__ __forceinline__ void stress_normal(const double (&Gn)[2], const double (&ns)[2], int c, double lm, double mu,
+                                              double (&J)[2]) {
+  const double gn = Gn[0] * ns[0] + Gn[1] * ns[1];
+  const double gc = c == 0 ? Gn[0] : Gn[1], nc = c == 0 ? ns[0] : ns[1];
+#pragma unroll
+  for (int d = 0; d < 2; ++d) J[d] = lm * gc * ns[d] + mu * (Gn[d] * nc + (d == c ? gn : 0.0));
+}
+
+// Cells tagged 1 (resp. 3): the stiffness block of u_in (resp. u_out) and its load int f.v, by the 2 x 2 Gauss rule.
+// One thread per (cell, k, j); the j == k threads write the load.
+__global__ void __launch_bounds__(kBlockEl) k_elasticity_quad_uncut(
+    phifem_mesh m, const double* __restrict__ f, const int8_t* __restrict__ ctags, const int32_t* __restrict__ vptr,
+    const int32_t* __restrict__ pos_cells, phifem_elasticity_params prm, double* __restrict__ data,
+    double* __restrict__ b) {
+  using S_ = ES<2>;
+  constexpr int NV = quad::NV, NB = S_::NB;
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= m.n_cells * (NV * NV)) return;
+  const int64_t c = t / (NV * NV);
+  const int rem = (int)(t - c * (NV * NV));
+  const int k = rem / NV, j = rem - k * NV;
+  const int tag = ctags[c];
+  if (tag != 1 && tag != 3) return;
+  const double lm = tag == 1 ? prm.lmbda_in : prm.lmbda_out, mu = tag == 1 ? prm.mu_in : prm.mu_out;
+  const int ou = tag == 1 ? S_::UI : S_::UO;
+  quad::Cell g;
+  quad::load_cell(m, c, g);
+  double K[2][2] = {{0.0, 0.0}, {0.0, 0.0}}, M[NV];   // M[l] = int N_k N_l (the j == k threads)
+#pragma unroll
+  for (int l = 0; l < NV; ++l) M[l] = 0.0;
+#pragma unroll
+  for (int q = 0; q < 4; ++q) {
+    double N[NV], G[NV][2], Jit[2][2], Gk[2], Gj[2];
+    const double w = 0.25 * quad::map_point(g, (q & 1) ? kGauss2Hi : kGauss2Lo, (q >> 1) ? kGauss2Hi : kGauss2Lo, N, G,
+                                            Jit);
+    pick_row(G, k, Gk);
+    pick_row(G, j, Gj);
+    const double gg = mu * (Gk[0] * Gj[0] + Gk[1] * Gj[1]);
+#pragma unroll
+    for (int ca = 0; ca < 2; ++ca)
+#pragma unroll
+      for (int cb = 0; cb < 2; ++cb) K[ca][cb] += w * (lm * Gk[ca] * Gj[cb] + mu * Gj[ca] * Gk[cb] + (ca == cb ? gg : 0.0));
+    const double wk = w * pick<NV>(N, k);
+#pragma unroll
+    for (int l = 0; l < NV; ++l) M[l] += wk * N[l];
+  }
+  const int vk = __ldg(m.cells + c * NV + k);
+  const int pos = __ldg(pos_cells + c * (NV * NV) + rem);
+#pragma unroll
+  for (int ca = 0; ca < 2; ++ca)
+#pragma unroll
+    for (int cb = 0; cb < 2; ++cb) atomicAdd(data + block_address(vptr, vk, ou + ca, pos, ou + cb, NB), K[ca][cb]);
+  if (j == k) {
+#pragma unroll
+    for (int ca = 0; ca < 2; ++ca) {
+      double s = 0.0;
+#pragma unroll
+      for (int l = 0; l < NV; ++l) s += __ldg(f + (int64_t)__ldg(m.cells + c * NV + l) * 2 + ca) * M[l];
+      atomicAdd(b + (int64_t)NB * vk + ou + ca, s);
+    }
+  }
+}
+
+// Cut cells (tag 2): every term of a and L by the cell rule of phifem_quadrature (reference points (xi, eta)).  One thread
+// per (cut cell, test node k, trial node j, trial offset b) = 224 per cell; the trial bundle and the contractions are the
+// simplex kernel's, at the point values and physical gradients of the Q1 basis.
+template <int KP>
+__global__ void __launch_bounds__(kBlockEl, 3) k_elasticity_quad_cells(
+    phifem_mesh m, phifem_pk_space sp, const double* __restrict__ qpt_g, const double* __restrict__ qw_g, int nq,
+    const double* __restrict__ phi, const double* __restrict__ f, const int32_t* __restrict__ cut_cells,
+    int64_t n_cut, const int32_t* __restrict__ vptr, const int32_t* __restrict__ pos_cells,
+    phifem_elasticity_params prm, double* __restrict__ data, double* __restrict__ b) {
+  using S_ = ES<2>;
+  constexpr int NV = quad::NV, NB = S_::NB, NDP = quad::QSpace<KP>::ND;
+  __shared__ double qpt[kMaxQuadPoints * 2], qw[kMaxQuadPoints];
+  for (int i = threadIdx.x; i < nq * 2; i += blockDim.x) qpt[i] = qpt_g[i];
+  for (int i = threadIdx.x; i < nq; i += blockDim.x) qw[i] = qw_g[i];
+  __syncthreads();
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_cut * (NV * NV * NB)) return;
+  const int64_t e = t / (NV * NV * NB);
+  int rem = (int)(t - e * (NV * NV * NB));
+  const int k = rem / (NV * NB);
+  rem -= k * (NV * NB);
+  const int j = rem / NB, ob = rem - j * NB;
+  const int64_t c = __ldg(cut_cells + e);
+  const int fld_b = S_::field(ob);
+  const int loc = ob - S_::base(fld_b);
+  quad::Cell g;
+  quad::load_cell(m, c, g);
+  const double h = sqrt(g.h2);
+  CellCoefs cf;
+  cf.lmbda_in = prm.lmbda_in; cf.mu_in = prm.mu_in; cf.lmbda_out = prm.lmbda_out; cf.mu_out = prm.mu_out;
+  cf.w_in = cf.w_out = 1.0;
+  cf.pen_in = prm.gamma * prm.coef_out;
+  cf.pen_out = prm.gamma * prm.coef_in;
+  cf.pen_h2 = prm.gamma / g.h2;
+  cf.stab = prm.sigma_s * g.h2;
+  double acc[NB], L[NV];   // L[l]: the load of offset ob at node k per unit nodal value of f at node l (j == k threads)
+#pragma unroll
+  for (int a = 0; a < NB; ++a) acc[a] = 0.0;
+#pragma unroll
+  for (int l = 0; l < NV; ++l) L[l] = 0.0;
+  double pc[NDP];
+  quad::load_phi<KP>(m, sp, phi, c, pc);
+  for (int q = 0; q < nq; ++q) {
+    const double xi = qpt[2 * q], eta = qpt[2 * q + 1];
+    double N[NV], G[NV][2], Jit[2][2], Gk[2], Gj[2];
+    const double w = qw[q] * quad::map_point(g, xi, eta, N, G, Jit);
+    double ph, gph[2];
+    quad::eval_phi<KP>(xi, eta, Jit, pc, ph, gph);
+    pick_row(G, k, Gk);
+    pick_row(G, j, Gj);
+    const double lk = pick<NV>(N, k), lj = pick<NV>(N, j);
+    Bundle<2> B;
+    trial_bundle<2>(ob, lj, Gj, gph, ph / h, cf, B);
+    accumulate<2>(std::make_integer_sequence<int, NB>{}, acc, w, B, fld_b, lk, Gk, gph, ph / h, cf);
+    if (j == k) {   // u: int f_loc N_k;  y (r, s0): sigma_s h^2 int f_r d_s0 N_k
+      const double wl = w * (fld_b <= 1 ? lk : (loc % 2 == 0 ? Gk[0] : Gk[1]));
+#pragma unroll
+      for (int l = 0; l < NV; ++l) L[l] += wl * N[l];
+    }
+  }
+  const int vk = __ldg(m.cells + c * NV + k);
+  const int pos = __ldg(pos_cells + c * (NV * NV) + k * NV + j);
+  const int64_t p0 = __ldg(vptr + vk), deg = __ldg(vptr + vk + 1) - p0;
+  const int64_t base = (int64_t)NB * ((int64_t)NB * p0 + pos) + ob;
+#pragma unroll
+  for (int a = 0; a < NB; ++a) {
+    if (couples(S_::field(a), fld_b)) atomicAdd(data + base + (int64_t)NB * a * deg, acc[a]);
+  }
+  if (j == k && fld_b <= 3) {
+    const int comp = fld_b <= 1 ? loc : loc / 2;
+    double s = 0.0;
+#pragma unroll
+    for (int l = 0; l < NV; ++l) s += __ldg(f + (int64_t)__ldg(m.cells + c * NV + l) * 2 + comp) * L[l];
+    atomicAdd(b + (int64_t)NB * vk + ob, fld_b <= 1 ? s : cf.stab * s);
+  }
+}
+
+// sigma_s avg(h) int_F [sigma(u) n].[sigma(v) n] over dS(3) (side 0: in) / dS(4) (side 1: out), by the 2-point Gauss
+// rule on the edge.  The edge parameter runs from the lower- to the higher-global-id vertex in both cells (as
+// k_quad_ghost_neumann), so both sides evaluate the same physical points.  One thread per (facet, trial side, node,
+// component) = 16 per facet, each summing the 16 test entries of its column.
+__global__ void __launch_bounds__(kBlockEl) k_elasticity_quad_facets(
+    phifem_mesh m, const int32_t* __restrict__ facets, int64_t n_facets, const int32_t* __restrict__ vptr,
+    const int32_t* __restrict__ pos_facets, int side, phifem_elasticity_params prm, double* __restrict__ data) {
+  using S_ = ES<2>;
+  constexpr int NV = quad::NV, NB = S_::NB, NT = 2 * NV * 2;
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_facets * NT) return;
+  const int64_t e = t / NT;
+  int rem = (int)(t - e * NT);
+  const int sb = rem / (NV * 2);
+  rem -= sb * (NV * 2);
+  const int j = rem / 2, cb = rem - j * 2;
+  const int32_t fct = __ldg(facets + e);
+  const int2 cc = __ldg(reinterpret_cast<const int2*>(m.f2c) + fct);
+  const double lm = side == 0 ? prm.lmbda_in : prm.lmbda_out, mu = side == 0 ? prm.mu_in : prm.mu_out;
+  const int ou = side == 0 ? S_::UI : S_::UO;
+  quad::Cell g[2];
+  double n[2][2], len = 0.0, r0[2][2], r1[2][2];   // per side: normal, reference end points of the parameter
+#pragma unroll
+  for (int s = 0; s < 2; ++s) {
+    const int64_t c = s == 0 ? cc.x : cc.y;
+    quad::load_cell(m, c, g[s]);
+    int o = 0;
+#pragma unroll
+    for (int k = 0; k < NV; ++k)
+      if (__ldg(m.c2f + c * NV + k) == fct) o = k;
+    int la = quad::facet_vertex(o, 0), lb = quad::facet_vertex(o, 1);
+    if (__ldg(m.cells + c * NV + la) > __ldg(m.cells + c * NV + lb)) {
+      const int tmp = la;
+      la = lb;
+      lb = tmp;
+    }
+    r0[s][0] = la & 1; r0[s][1] = la >> 1;
+    r1[s][0] = lb & 1; r1[s][1] = lb >> 1;
+    double l;
+    quad::edge_normal(g[s], o, n[s], l);
+    if (s == 0) len = l;
+  }
+  const double coef = prm.sigma_s * 0.5 * (sqrt(g[0].h2) + sqrt(g[1].h2)) * len * 0.5;   // 0.5: the Gauss weight
+  double E[2][NV][2];
+#pragma unroll
+  for (int sa = 0; sa < 2; ++sa)
+#pragma unroll
+    for (int k = 0; k < NV; ++k) E[sa][k][0] = E[sa][k][1] = 0.0;
+#pragma unroll
+  for (int q = 0; q < 2; ++q) {
+    const double tq = q == 0 ? kGauss2Lo : kGauss2Hi;
+    double G[2][NV][2];
+#pragma unroll
+    for (int s = 0; s < 2; ++s) {
+      double N[NV], Jit[2][2];
+      quad::map_point(g[s], (1.0 - tq) * r0[s][0] + tq * r1[s][0], (1.0 - tq) * r0[s][1] + tq * r1[s][1], N, G[s],
+                      Jit);
+    }
+    double Gb[2] = {G[0][0][0], G[0][0][1]}, nb[2] = {n[0][0], n[0][1]}, Jb[2];
+#pragma unroll
+    for (int s = 0; s < 2; ++s)
+#pragma unroll
+      for (int k = 0; k < NV; ++k)
+        if (s == sb && k == j) {
+          Gb[0] = G[s][k][0];
+          Gb[1] = G[s][k][1];
+          nb[0] = n[s][0];
+          nb[1] = n[s][1];
+        }
+    stress_normal(Gb, nb, cb, lm, mu, Jb);
+#pragma unroll
+    for (int sa = 0; sa < 2; ++sa)
+#pragma unroll
+      for (int k = 0; k < NV; ++k)
+#pragma unroll
+        for (int ca = 0; ca < 2; ++ca) {
+          double Ja[2];
+          stress_normal(G[sa][k], n[sa], ca, lm, mu, Ja);
+          E[sa][k][ca] += coef * (Ja[0] * Jb[0] + Ja[1] * Jb[1]);
+        }
+  }
+  const int colslot = sb * NV + j;
+#pragma unroll
+  for (int sa = 0; sa < 2; ++sa)
+#pragma unroll
+    for (int k = 0; k < NV; ++k) {
+      const int vk = __ldg(m.cells + (int64_t)(sa == 0 ? cc.x : cc.y) * NV + k);
+      const int pos = __ldg(pos_facets + (e * (2 * NV) + sa * NV + k) * (2 * NV) + colslot);
+#pragma unroll
+      for (int ca = 0; ca < 2; ++ca)
+        atomicAdd(data + block_address(vptr, vk, ou + ca, pos, ou + cb, NB), E[sa][k][ca]);
+    }
+}
+
+// int_{ds(100)} (y_in n).v_in (side 0) / int_{ds(101)} (y_out n).v_out (side 1) on quadrilaterals: Q1 restricted to the
+// straight edge is linear, so the entry (v_(k,c), y_(j,(c,s))) is n_s |F| (1 + delta_kj) / 6 for k, j the edge's two
+// vertices (as k_quad_boundary_neumann).  One thread per (entity, k, j).
+__global__ void __launch_bounds__(kBlockEl) k_elasticity_quad_boundary(
+    phifem_mesh m, const int32_t* __restrict__ entities, int64_t n_entities, const int32_t* __restrict__ vptr,
+    const int32_t* __restrict__ pos_boundary, int side, double* __restrict__ data) {
+  using S_ = ES<2>;
+  constexpr int NV = quad::NV, NB = S_::NB;
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_entities * NV * NV) return;
+  const int64_t e = t / (NV * NV);
+  const int rem = (int)(t - e * NV * NV);
+  const int k = rem / NV, j = rem - k * NV;
+  const int64_t c = __ldg(entities + 2 * e);
+  const int o = __ldg(entities + 2 * e + 1);
+  const int la = quad::facet_vertex(o, 0), lb = quad::facet_vertex(o, 1);
+  if ((k != la && k != lb) || (j != la && j != lb)) return;   // N_k or N_j vanishes on the edge
+  quad::Cell g;
+  quad::load_cell(m, c, g);
+  double n[2], len;
+  quad::edge_normal(g, o, n, len);
+  const double mkj = len * (k == j ? 2.0 : 1.0) * (1.0 / 6.0);
+  const int ou = side == 0 ? S_::UI : S_::UO, oy = side == 0 ? S_::YI : S_::YO;
+  const int vk = __ldg(m.cells + c * NV + k);
+  const int pos = __ldg(pos_boundary + e * (NV * NV) + rem);
+#pragma unroll
+  for (int cc = 0; cc < 2; ++cc)
+#pragma unroll
+    for (int s = 0; s < 2; ++s)
+      atomicAdd(data + block_address(vptr, vk, ou + cc, pos, oy + cc * 2 + s, NB), n[s] * mkj);
+}
+
 // Dirichlet conditions on an assembled CSR system, one warp per row: rows and columns of constrained dofs zeroed,
 // their diagonal 1, b <- b - A g on the free rows, b = g on the constrained ones
 // (dolfinx assemble_matrix(bcs=) + apply_lifting + bc.set: main.py:238, 271-274)
@@ -483,13 +776,16 @@ __global__ void __launch_bounds__(256) k_apply_dirichlet_list(const int32_t* __r
   }
 }
 
-int check_simplex(const phifem_mesh* m, int& D) {
+// the cell type: triangles (D = 2), tetrahedra (D = 3) and quadrilaterals (D = 2, is_quad)
+int check_mesh(const phifem_mesh* m, int& D, bool& is_quad) {
   PHIFEM_CHECK_ARG(m != nullptr && m->x && m->cells, "mesh is null");
-  if (m->cell_type != PHIFEM_TRIANGLE && m->cell_type != PHIFEM_TETRAHEDRON) {
-    set_error("the interface-elasticity operator supports triangles and tetrahedra, got cell type %d", m->cell_type);
+  if (m->cell_type != PHIFEM_TRIANGLE && m->cell_type != PHIFEM_TETRAHEDRON && m->cell_type != PHIFEM_QUADRILATERAL) {
+    set_error("the interface-elasticity operator supports triangles, quadrilaterals and tetrahedra, got cell type %d",
+              m->cell_type);
     return PHIFEM_ERR_UNSUPPORTED;
   }
-  D = m->cell_type == PHIFEM_TRIANGLE ? 2 : 3;
+  is_quad = m->cell_type == PHIFEM_QUADRILATERAL;
+  D = m->cell_type == PHIFEM_TETRAHEDRON ? 3 : 2;
   PHIFEM_CHECK_ARG(m->gdim == D, "gdim mismatch");
   return PHIFEM_OK;
 }
@@ -506,12 +802,19 @@ extern "C" int phifem_assemble_elasticity_cells(const phifem_mesh* mesh, const p
                                                 const phifem_elasticity_params* prm, double* data, double* b,
                                                 void* stream) {
   int D = 0;
-  if (int rc = check_simplex(mesh, D)) return rc;
+  bool is_quad = false;
+  if (int rc = check_mesh(mesh, D, is_quad)) return rc;
   if (mesh->n_cells == 0) return PHIFEM_OK;
   PHIFEM_CHECK_ARG(space_phi && quad && prm, "space / quadrature / parameters are null");
   if (space_phi->degree != 1 && space_phi->degree != 2) {
     set_error("level-set degree %d: degrees 1 and 2 are implemented", space_phi->degree);
     return PHIFEM_ERR_UNSUPPORTED;
+  }
+  if (is_quad) {
+    PHIFEM_CHECK_ARG(space_phi->n_dofs_per_cell == 4 || space_phi->n_dofs_per_cell == 9,
+                     "space_phi->n_dofs_per_cell must be 4 (Q1) or 9 (Q2) on quadrilaterals");
+    PHIFEM_CHECK_ARG(space_phi->degree == (space_phi->n_dofs_per_cell == 4 ? 1 : 2),
+                     "space_phi->degree does not match n_dofs_per_cell on quadrilaterals");
   }
   PHIFEM_CHECK_ARG(space_phi->dofmap || space_phi->degree == 1, "a P2 level set needs its dofmap");
   PHIFEM_CHECK_ARG(quad->cell_points && quad->cell_weights && quad->n_cell_points > 0 &&
@@ -519,11 +822,12 @@ extern "C" int phifem_assemble_elasticity_cells(const phifem_mesh* mesh, const p
   PHIFEM_CHECK_ARG(phi && f && cell_tags8 && vptr && pos_cells && data && b, "null array");
   PHIFEM_CHECK_ARG(n_cut >= 0 && (n_cut == 0 || cut_cells), "cut-cell list");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int nv = D + 1, nb = 3 * D + 2 * D * D;
+  const int nv = is_quad ? quad::NV : D + 1, nb = 3 * D + 2 * D * D;
   {
     const int64_t blocks = (mesh->n_cells * (int64_t)(nv * nv) + kBlockEl - 1) / kBlockEl;
     PHIFEM_CHECK_ARG(blocks < (1ll << 31), "too many cells for one launch");
-    if (D == 2) k_elasticity_uncut<2><<<(unsigned)blocks, kBlockEl, 0, st>>>(*mesh, f, cell_tags8, vptr, pos_cells, *prm, data, b);
+    if (is_quad) k_elasticity_quad_uncut<<<(unsigned)blocks, kBlockEl, 0, st>>>(*mesh, f, cell_tags8, vptr, pos_cells, *prm, data, b);
+    else if (D == 2) k_elasticity_uncut<2><<<(unsigned)blocks, kBlockEl, 0, st>>>(*mesh, f, cell_tags8, vptr, pos_cells, *prm, data, b);
     else k_elasticity_uncut<3><<<(unsigned)blocks, kBlockEl, 0, st>>>(*mesh, f, cell_tags8, vptr, pos_cells, *prm, data, b);
     PHIFEM_CHECK_LAUNCH();
   }
@@ -535,11 +839,18 @@ extern "C" int phifem_assemble_elasticity_cells(const phifem_mesh* mesh, const p
   k_elasticity_cells<DD, KK><<<grid, kBlockEl, 0, st>>>(*mesh, *space_phi, quad->cell_points, quad->cell_weights,     \
                                                         quad->n_cell_points, phi, f, cut_cells, n_cut, vptr, pos_cells, \
                                                         *prm, data, b)
-  if (D == 2 && space_phi->degree == 1) PHIFEM_EL_LAUNCH(2, 1);
+#define PHIFEM_EL_QUAD_LAUNCH(KK)                                                                                    \
+  k_elasticity_quad_cells<KK><<<grid, kBlockEl, 0, st>>>(*mesh, *space_phi, quad->cell_points, quad->cell_weights,     \
+                                                        quad->n_cell_points, phi, f, cut_cells, n_cut, vptr, pos_cells, \
+                                                        *prm, data, b)
+  if (is_quad && space_phi->degree == 1) PHIFEM_EL_QUAD_LAUNCH(1);
+  else if (is_quad) PHIFEM_EL_QUAD_LAUNCH(2);
+  else if (D == 2 && space_phi->degree == 1) PHIFEM_EL_LAUNCH(2, 1);
   else if (D == 2) PHIFEM_EL_LAUNCH(2, 2);
   else if (space_phi->degree == 1) PHIFEM_EL_LAUNCH(3, 1);
   else PHIFEM_EL_LAUNCH(3, 2);
 #undef PHIFEM_EL_LAUNCH
+#undef PHIFEM_EL_QUAD_LAUNCH
   PHIFEM_CHECK_LAUNCH();
   return PHIFEM_OK;
 }
@@ -548,15 +859,17 @@ extern "C" int phifem_assemble_elasticity_facets(const phifem_mesh* mesh, const 
                                                  const int32_t* vptr, const int32_t* pos_facets, int32_t side,
                                                  const phifem_elasticity_params* prm, double* data, void* stream) {
   int D = 0;
-  if (int rc = check_simplex(mesh, D)) return rc;
+  bool is_quad = false;
+  if (int rc = check_mesh(mesh, D, is_quad)) return rc;
   if (n_facets == 0) return PHIFEM_OK;
   PHIFEM_CHECK_ARG(mesh->c2f && mesh->f2c, "mesh without facet connectivity");
   PHIFEM_CHECK_ARG(facets && vptr && pos_facets && prm && data, "null array");
   PHIFEM_CHECK_ARG(side == 0 || side == 1, "side must be 0 (in) or 1 (out)");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int64_t threads = n_facets * 2 * (D + 1) * D;
+  const int64_t threads = n_facets * 2 * (is_quad ? quad::NV : D + 1) * D;
   const unsigned grid = (unsigned)((threads + kBlockEl - 1) / kBlockEl);
-  if (D == 2) k_elasticity_facets<2><<<grid, kBlockEl, 0, st>>>(*mesh, facets, n_facets, vptr, pos_facets, side, *prm, data);
+  if (is_quad) k_elasticity_quad_facets<<<grid, kBlockEl, 0, st>>>(*mesh, facets, n_facets, vptr, pos_facets, side, *prm, data);
+  else if (D == 2) k_elasticity_facets<2><<<grid, kBlockEl, 0, st>>>(*mesh, facets, n_facets, vptr, pos_facets, side, *prm, data);
   else k_elasticity_facets<3><<<grid, kBlockEl, 0, st>>>(*mesh, facets, n_facets, vptr, pos_facets, side, *prm, data);
   PHIFEM_CHECK_LAUNCH();
   return PHIFEM_OK;
@@ -567,14 +880,17 @@ extern "C" int phifem_assemble_elasticity_boundary(const phifem_mesh* mesh, cons
                                                    const int32_t* pos_boundary, int32_t side, double* data,
                                                    void* stream) {
   int D = 0;
-  if (int rc = check_simplex(mesh, D)) return rc;
+  bool is_quad = false;
+  if (int rc = check_mesh(mesh, D, is_quad)) return rc;
   if (n_entities == 0) return PHIFEM_OK;
   PHIFEM_CHECK_ARG(entities && vptr && pos_boundary && data, "null array");
   PHIFEM_CHECK_ARG(side == 0 || side == 1, "side must be 0 (in) or 1 (out)");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  const int64_t threads = n_entities * (D + 1) * (D + 1);
+  const int nv = is_quad ? quad::NV : D + 1;
+  const int64_t threads = n_entities * nv * nv;
   const unsigned grid = (unsigned)((threads + kBlockEl - 1) / kBlockEl);
-  if (D == 2) k_elasticity_boundary<2><<<grid, kBlockEl, 0, st>>>(*mesh, entities, n_entities, vptr, pos_boundary, side, data);
+  if (is_quad) k_elasticity_quad_boundary<<<grid, kBlockEl, 0, st>>>(*mesh, entities, n_entities, vptr, pos_boundary, side, data);
+  else if (D == 2) k_elasticity_boundary<2><<<grid, kBlockEl, 0, st>>>(*mesh, entities, n_entities, vptr, pos_boundary, side, data);
   else k_elasticity_boundary<3><<<grid, kBlockEl, 0, st>>>(*mesh, entities, n_entities, vptr, pos_boundary, side, data);
   PHIFEM_CHECK_LAUNCH();
   return PHIFEM_OK;

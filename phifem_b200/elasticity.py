@@ -15,6 +15,9 @@ dofmap builder).  Sparsity (dolfinx create_sparsity_pattern [dep-knowledge, SURV
 of dx((1,2)) u dx((2,3)) u dx(2) -- every tagged cell -- and all pairs among the dofs of the two cells of every interior
 facet of dS(3) u dS(4); with nodal fields that is the vertex graph with dense NB x NB blocks, which is how the kernels
 address it (one scalar slot map).  Symbolic phase = torch sort/unique on the mesh's device.
+
+On quadrilaterals every field is Q1 on the bilinear cell (NB = 14, the same numbering) with a Q1 or Q2 level set; the
+integrals follow the rules of `quadrature.rules_for_elasticity_quad`.
 """
 import ctypes
 
@@ -54,8 +57,9 @@ class ElasticityPlan:
     form = "interface-elasticity"
 
     def __init__(self, mesh, cell_tags8, facet_tags8, ents_in, ents_out, V_phi):
-        if mesh.cell_type not in ("triangle", "tetrahedron"):
-            raise NotImplementedError("the interface-elasticity operator supports triangles and tetrahedra")
+        if mesh.cell_type not in ("triangle", "tetrahedron", "quadrilateral"):
+            raise NotImplementedError("the interface-elasticity operator supports triangles, quadrilaterals and "
+                                      "tetrahedra")
         if V_phi.mesh is not mesh:
             raise ValueError("the level-set space is defined on another mesh")
         if V_phi.degree not in (1, 2):
@@ -64,7 +68,6 @@ class ElasticityPlan:
         self.mesh, self.V_phi = mesh, V_phi
         self.cell_tags8 = cell_tags8
         d = mesh.gdim
-        nv = d + 1
         self.layout, self.nb = field_layout(d)
         nb, nvx = self.nb, mesh.num_vertices
         self.n_rows = nb * nvx
@@ -129,7 +132,10 @@ class ElasticityPlan:
             indices[addr.reshape(-1)] = val.expand(-1, nb, -1).reshape(-1).to(torch.int32)
         self.indices = indices
 
-        (cl, cw), _ = quadrature.rules_for_neumann(d, V_phi.degree)   # degree 2 (kphi + 1): (lambda phi)^2
+        if mesh.cell_type == "quadrilateral":   # the cut-cell rule; the other rules are constants of the kernels
+            (cl, cw), _, _ = quadrature.rules_for_elasticity_quad(V_phi.degree)
+        else:
+            (cl, cw), _ = quadrature.rules_for_neumann(d, V_phi.degree)   # degree 2 (kphi + 1): (lambda phi)^2
         f64 = dict(dtype=torch.float64, device=dev)
         self._q = [torch.as_tensor(a, **f64).contiguous() for a in (cl, cw)]
         self.n_cell_points = len(cw)

@@ -242,3 +242,21 @@ def rules_for_strong_quad(kphi):
     direction on cells and a degree 2 kphi + 2 rule on edges are exact.  On a non-affine cell no integrand is
     polynomial: the operator is defined at these rules."""
     return square_rule(kphi + 2), simplex_rule(1, 2 * kphi + 2)
+
+
+def rules_for_elasticity_quad(kphi):
+    """Rules of the interface-elasticity forms on quadrilaterals (demo/interface-elasticity/main.py:181-269) for Q1
+    fields and a Q_kphi level set: (cut-cell rule, uncut-cell rule, edge rule).
+
+      * cut cells (tag 2), every term of a and L: (kphi + 2)^2 Gauss points, passed to the kernels in
+        `phifem_quadrature`.  On a parallelogram the worst terms, (h^-1 p phi)^2 and ((y_in - y_out) grad phi)^2, have
+        degree 2 (kphi + 1) per reference direction, so the rule is exact there;
+      * uncut cells (tags 1 and 3), the stiffness of the one material and int f.v: 2 x 2 Gauss points (degree 2 per
+        direction on a parallelogram), compile-time constants of the kernel;
+      * the stress jump sigma_s avg(h) int [sigma(u) n].[sigma(v) n] over dS(3) / dS(4): 2 Gauss points on the edge
+        (sigma(u) n is linear along the edge of a parallelogram), compile-time constants of the kernel.  Segment points
+        are (1 - t, t), t running from the edge's lower-global-id vertex to the higher one.
+
+    The one-sided terms int (y n).v over ds(100) / ds(101) are exact in closed form (Q1 restricted to a straight edge is
+    linear).  On a cell that is not a parallelogram no integrand is polynomial: the operator is defined by these rules."""
+    return square_rule(kphi + 2), square_rule(2), simplex_rule(1, 2)

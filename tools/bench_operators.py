@@ -1,14 +1,16 @@
 #!/usr/bin/env python
 """Timing of the mixed-space operators beside the headline path (not the bench.py contract: one JSON line per operator).
 
-    python tools/bench_operators.py [--ops neumann,neumann-quad,strong-quad,elasticity-2d,elasticity-3d] [--steps 10]
-                                    [--warmup 3]
+    python tools/bench_operators.py [--ops neumann,neumann-quad,strong-quad,elasticity-2d,elasticity-quad,elasticity-3d]
+                                    [--steps 10] [--warmup 3]
 
   neumann        BASELINE.json configs[1]: demo/neumann forms on a synthetic 4 M-cell triangle mesh (n = 1414), disc
   neumann-quad   the same forms on the demo's cell type: 2 M quadrilaterals on the same 2 M vertices (n = 1414), same
                  disc, Q2 level set (as the demo, levelset_degree = 2)
   strong-quad    demo/strong-dirichlet forms on the same 2 M quadrilaterals and disc: Q1 w, Q2 level set
   elasticity-2d  BASELINE.json configs[3] forms on 2 M triangles of the demo's box [-1.5, 1.5]^2 (n = 1000), unit disc
+  elasticity-quad  the same forms on 1 M quadrilaterals of the same box (n = 1000, the same 1.0 M vertices), unit disc,
+                 Q1 level set
   elasticity-3d  BASELINE.json configs[3] as stated ("3D tetra mesh"): 384 000 Kuhn tetrahedra (n = 40), sphere
 
 One step = cell tags + facet tags + zeroing + assembly (all kernels of the operator) on resident inputs, timed with CUDA
@@ -65,9 +67,10 @@ def run(op, steps, warmup):
         n = 1414
         mesh = (synthetic.rectangle_mesh if op == "neumann" else synthetic.quadrilateral_mesh)(n, device=dev)
         phi = synthetic.sphere_levelset(mesh.x, center=(0.0031, 0.0027), radius=0.6)
-    elif op == "elasticity-2d":
+    elif op in ("elasticity-2d", "elasticity-quad"):
         n = 1000
-        mesh = synthetic.rectangle_mesh(n, lo=(-1.5, -1.5), hi=(1.5, 1.5), device=dev)
+        make_mesh = synthetic.rectangle_mesh if op == "elasticity-2d" else synthetic.quadrilateral_mesh
+        mesh = make_mesh(n, lo=(-1.5, -1.5), hi=(1.5, 1.5), device=dev)
         phi = 1.0 - ((mesh.x[:, 0] - 0.0031) ** 2 + (mesh.x[:, 1] - 0.0027) ** 2)
     else:
         n = 40
