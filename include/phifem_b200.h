@@ -448,8 +448,10 @@ int phifem_csr_spmv(int64_t n_rows, const int32_t* indptr, const int32_t* indice
  *                 a trailing 0 (y, z: what the products multiply);
  *   state [8]     {rho, alpha, omega, beta, r.r, rho_new, -, -}: {1, 1, 1, 0, ...} before the first call; state[4] = |r|^2
  *                 of the current iterate after every call;
- *   partials      2 * 8 * 148 doubles; on entry its first *n_partials pairs hold partial sums of (rhat.r, r.r)
- *                 (first call: one pair); *n_partials (HOST) is updated for a continuation.
+ *   partials      at least 2 * 8 * 148 doubles (the products and the vector update write at most 8 * 148 pairs) and
+ *                 2 * *n_partials; on entry its first *n_partials pairs hold partial sums of (rhat.r, r.r) (first
+ *                 call: one pair); *n_partials (HOST) is updated for a continuation.  *n_partials below 1 or above the
+ *                 product's grid + the vector grid (each at most 8 * 148 blocks) returns PHIFEM_ERR_ARGUMENT.
  * No host synchronisation; five kernels and three one-block scalar updates per iteration, bitwise reproducible. */
 /* Set-up passes of the solve: diag[r] = a_rr (0 when the pattern has no diagonal entry) and rowmax[r] = max_c |a_rc| of
  * every row; cols[k] = cmap[indices[k]] (the column ids in the compact numbering of the active rows). */

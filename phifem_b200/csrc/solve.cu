@@ -254,7 +254,7 @@ __global__ void __launch_bounds__(256) k_remap_columns(int64_t nnz, const int32_
 extern "C" int phifem_csr_row_scan(int64_t n_rows, const int32_t* indptr, const int32_t* indices, const double* data,
                                    double* diag, double* rowmax, void* stream) {
   if (n_rows == 0) return PHIFEM_OK;
-  PHIFEM_CHECK_ARG(n_rows > 0 && indptr && diag && rowmax, "null pointer");
+  PHIFEM_CHECK_ARG(n_rows > 0 && indptr && indices && data && diag && rowmax, "null pointer");
   const int64_t threads = n_rows * 4;
   k_row_scan<<<(unsigned)((threads + 255) / 256), 256, 0, (cudaStream_t)stream>>>(n_rows, indptr, indices, data, diag,
                                                                                  rowmax);
