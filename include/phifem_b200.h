@@ -34,7 +34,8 @@ typedef enum phifem_status {
 typedef enum phifem_cell_type {
   PHIFEM_TRIANGLE = 0,
   PHIFEM_QUADRILATERAL = 1,
-  PHIFEM_TETRAHEDRON = 2
+  PHIFEM_TETRAHEDRON = 2,
+  PHIFEM_HEXAHEDRON = 3        /* vertices in tensor order; tagging and the one-sided measures only */
 } phifem_cell_type;
 
 /* Mesh arrays resident in HBM (what a dolfinx `Mesh` + its topology connectivities hold;
@@ -81,8 +82,14 @@ typedef struct phifem_levelset {
   const double* facet_table;    /* [nfpc, nq, nd] basis at the facet detection points (mode 0) */
   const double* cell_values;    /* [n_cells, npts]       (mode 1) */
   const double* facet_values;   /* [n_cells, nfpc, nq]   (mode 1) */
-  const double* coord_grad;     /* [npts, 4, 2] reference gradients of the Q1 coordinate element at
-                                   the cell detection points (quadrilaterals only) */
+  const double* coord_grad;     /* reference gradients of the coordinate element:
+                                   quadrilaterals: [npts, 4, 2] at the cell detection points (required by
+                                   phifem_tag_cells);
+                                   hexahedra: [npts + nfpc * nq, 8, 3] at the cell detection points, then at the
+                                   facet detection points of local facets 0..5 (required by phifem_tag_cells and
+                                   phifem_tag_facets*, which then also read n_cell_points); the scale of a cell point
+                                   is |det J|, that of a facet point |dx/ds x dx/dt| (faces need not be planar).
+                                   Hexahedral level sets: n_dofs_per_cell <= 27 (Q1 without dofmap: 8). */
 } phifem_levelset;
 
 /* Slots of the int64 counter block written by the tag kernels. */

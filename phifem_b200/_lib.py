@@ -11,7 +11,8 @@ import torch
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("PHIFEM_B200_LIB") or os.path.join(_HERE, "libphifem_b200.so")
 
-CELL_TYPE_ID = {"triangle": 0, "quadrilateral": 1, "tetrahedron": 2}
+CELL_TYPE_ID = {"triangle": 0, "quadrilateral": 1, "tetrahedron": 2, "hexahedron": 3}
+_SIMPLICES = ("triangle", "tetrahedron")
 N_COUNTERS = 16
 CNT_INTERIOR, CNT_CUT, CNT_EXTERIOR, CNT_UNTAGGED, CNT_ZERO_DEN, CNT_ZERO_DEN_AMBIGUOUS = 0, 1, 2, 3, 4, 5
 CNT_FACET_ZERO_DEN, CNT_FACET_CONFLICT, CNT_BOUNDARY_OWNERS = 11, 12, 13
@@ -264,9 +265,9 @@ def require_cuda(mesh):
 
 def c_mesh(mesh, with_facets=True, with_records=True):
     require_cuda(mesh)
-    lo, hi = mesh.detj_bounds() if mesh.cell_type != "quadrilateral" else (0.0, 0.0)
+    lo, hi = mesh.detj_bounds() if mesh.cell_type in _SIMPLICES else (0.0, 0.0)
     owner = scale = None
-    if with_facets and with_records and mesh.cell_type != "quadrilateral":
+    if with_facets and with_records and mesh.cell_type in _SIMPLICES:
         owner, scale = mesh.boundary_records()
     return CMesh(CELL_TYPE_ID[mesh.cell_type], mesh.gdim, mesh.num_vertices, mesh.num_cells,
                  mesh.num_facets if with_facets else 0, ptr(mesh.x), ptr(mesh.cells),

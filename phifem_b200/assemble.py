@@ -209,6 +209,13 @@ class AssemblyPlan:
         return bool(torch.equal(c8, self._sig_cells)) and bool(torch.equal(_facet_classes(f8), self._sig_facets))
 
 
+def refuse_hexahedra(mesh, what):
+    """Hexahedral meshes can be tagged (`compute_tags_measures`); no operator assembles on them yet."""
+    if mesh.cell_type == "hexahedron":
+        raise NotImplementedError("%s: no operator assembles on cell type 'hexahedron' (hexahedral meshes can be "
+                                  "tagged only)" % what)
+
+
 def _facet_classes(facet_tags8):
     """What a plan sees of a facet tag: 1 = ghost-penalty facet (tags 2 and 3 alike), 2 = Gamma_h (tag 4), 0 otherwise."""
     return ((facet_tags8 == 2) | (facet_tags8 == 3)).to(torch.int8) + 2 * (facet_tags8 == 4).to(torch.int8)
@@ -251,6 +258,7 @@ def build_plan(mesh, cells_tags, facets_tags, ds=None, method="rows", capacity=N
     cell_pass (row-gather plans): "rows" = one evaluation per (row, cell) record, "tiles" = the cell-once pass of
     csrc/assemble_tiles.cu.  geometry (row-gather plans): tabulate the cells' geometry factors once per plan (phifem_b200/rows.py; an
     option kept for the record, slower than the default on the B200)."""
+    refuse_hexahedra(mesh, "build_plan")
     c8, f8, ents = _plan_inputs(mesh, cells_tags, facets_tags, ds)
     if mesh.cell_type == "quadrilateral":
         # the quadrature kernels of csrc/assemble_quad.cu (PkAssemblyPlan); the row-gather options have no
@@ -367,6 +375,7 @@ def build_plan_weak_dirichlet(mesh, cells_tags, facets_tags, ds=None, V=None, V_
     """Symbolic phase for `a` and `L` of the weak-Dirichlet (dual) demo (reference
     demo/weak-dirichlet/flower/main.py:112-151): mixed space `V x V` (u, p) (`mixed_space`, main.py:76-82),
     level-set space `V_phi`; defaults: P1 on the mesh.  The mixed vector holds u at even, p at odd positions."""
+    refuse_hexahedra(mesh, "build_plan_weak_dirichlet")
     from . import fem
     from .assemble_pk import PkAssemblyPlan
     V = fem.functionspace(mesh, 1) if V is None else V
@@ -397,6 +406,7 @@ def build_plan_neumann(mesh, cells_tags, facets_tags, ds=None, V_phi=None, ghost
     y_c -> (d+1) s + 1 + c, p of cell k -> (d+1) Nv + k (`plan.split(x)` returns the three fields).  ghost_tag: facets
     of the gradient-jump term, dS(3) in the Neumann demo (main.py:136-139), dS(2) in the Robin demo
     (demo/robin/square/main.py:143-150)."""
+    refuse_hexahedra(mesh, "build_plan_neumann")
     from . import fem
     from .assemble_pk import PkAssemblyPlan
     V = fem.functionspace(mesh, 1)

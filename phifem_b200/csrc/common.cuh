@@ -28,7 +28,7 @@ void set_error(const char* fmt, ...);
   } while (0)
 
 // Reference-cell traits (dolfinx conventions, SURVEY.md Appendix C): simplex local facet i is opposite
-// local vertex i, its vertices listed in ascending local order; quadrilateral facets in tensor order.
+// local vertex i, its vertices listed in ascending local order; quadrilateral and hexahedron facets in tensor order.
 template <int CT> struct CellTraits;
 template <> struct CellTraits<PHIFEM_TRIANGLE> {
   static constexpr int nv = 3, nf = 3, nvf = 2, gdim = 2;
@@ -48,6 +48,15 @@ template <> struct CellTraits<PHIFEM_TETRAHEDRON> {
   static constexpr int nv = 4, nf = 4, nvf = 3, gdim = 3;
   __host__ __device__ static constexpr int fv(int f, int k) {
     constexpr int t[4][3] = {{1, 2, 3}, {0, 2, 3}, {0, 1, 3}, {0, 1, 2}};
+    return t[f][k];
+  }
+};
+// vertices in tensor order (v = i + 2 j + 4 k at (i, j, k)), faces (a, b, c, d) in tensor order: a face point (s, t)
+// sits at v_a + s (v_b - v_a) + t (v_c - v_a)
+template <> struct CellTraits<PHIFEM_HEXAHEDRON> {
+  static constexpr int nv = 8, nf = 6, nvf = 4, gdim = 3;
+  __host__ __device__ static constexpr int fv(int f, int k) {
+    constexpr int t[6][4] = {{0, 1, 2, 3}, {0, 1, 4, 5}, {0, 2, 4, 6}, {1, 3, 5, 7}, {2, 3, 6, 7}, {4, 5, 6, 7}};
     return t[f][k];
   }
 };

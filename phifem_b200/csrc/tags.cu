@@ -21,6 +21,14 @@ namespace {
 constexpr int kMaxDofs = 20;  // P3 tetrahedron
 constexpr int kBlock = 256;
 
+// Bounds of the cell-local arrays (vertices, facets, level-set dofs) per cell type.  Simplices and quadrilaterals keep
+// the sizes their kernels were tuned with; only hexahedra (8 vertices, 6 facets, 27 dofs of Q2) get larger ones.
+template <int CT> struct LocalBounds {
+  static constexpr int nv = CellTraits<CT>::nv > 4 ? CellTraits<CT>::nv : 4;
+  static constexpr int nf = CellTraits<CT>::nf > 4 ? CellTraits<CT>::nf : 4;
+  static constexpr int nd = CT == PHIFEM_HEXAHEDRON ? 27 : kMaxDofs;
+};
+
 __device__ __forceinline__ double seq_dot(const double* __restrict__ w, int wstride,
                                           const double* v, int vstride, int n) {
   // sum_k w[k] v[k], left to right, exact-zero weights skipped, unit weights not multiplied
@@ -53,8 +61,8 @@ __device__ __forceinline__ void ldg256(const double* p, double& a, double& b, do
 }
 
 template <int CT>
-__device__ __forceinline__ void load_cell(const phifem_mesh& m, int64_t c, int (&v)[4],
-                                          double (&xc)[4][3]) {
+__device__ __forceinline__ void load_cell(const phifem_mesh& m, int64_t c, int (&v)[LocalBounds<CT>::nv],
+                                          double (&xc)[LocalBounds<CT>::nv][3]) {
   using T = CellTraits<CT>;
 #pragma unroll
   for (int k = 0; k < T::nv; ++k) v[k] = __ldg(m.cells + c * T::nv + k);
@@ -114,8 +122,48 @@ __device__ __forceinline__ double facet_scale(const double (&xc)[4][3], int lf) 
   }
 }
 
+// ---- hexahedra: the trilinear map evaluated per point from the reference gradients g[8][3] of ls.coord_grad ----------
+// Jacobian column d x / d X_ax, summed like oracle/tags_hex.py
+__device__ __forceinline__ void hex_jcol(const double* g, const double (&xc)[8][3], int ax, double (&col)[3]) {
+#pragma unroll
+  for (int d = 0; d < 3; ++d) col[d] = seq_dot(g + ax, 3, &xc[0][d], 3, 8);
+}
+
+// |det J| at a point, the cofactor expansion of simplex_detj on the columns of J
+__device__ __forceinline__ double hex_detj(const double* g, const double (&xc)[8][3]) {
+  double a[3], b[3], c[3];
+  hex_jcol(g, xc, 0, a);
+  hex_jcol(g, xc, 1, b);
+  hex_jcol(g, xc, 2, c);
+  const double det = (a[0] * (b[1] * c[2] - c[1] * b[2]) - b[0] * (a[1] * c[2] - c[1] * a[2])) +
+                     c[0] * (a[1] * b[2] - b[1] * a[2]);
+  return fabs(det);
+}
+
+// |dx/ds x dx/dt| at a point of local face lf = (a, b, c, d): v_b - v_a and v_c - v_a are reference axes, so the two
+// tangents are columns of J
+__device__ __forceinline__ double hex_facet_scale(const double* g, const double (&xc)[8][3], int lf) {
+  using T = CellTraits<PHIFEM_HEXAHEDRON>;
+  int sa = 0, ta = 0;
+#pragma unroll
+  for (int f = 0; f < T::nf; ++f)
+    if (f == lf) {
+      const int db = T::fv(f, 1) - T::fv(f, 0), dc = T::fv(f, 2) - T::fv(f, 0);
+      sa = db == 1 ? 0 : (db == 2 ? 1 : 2);
+      ta = dc == 1 ? 0 : (dc == 2 ? 1 : 2);
+    }
+  double e1[3], e2[3];
+  hex_jcol(g, xc, sa, e1);
+  hex_jcol(g, xc, ta, e2);
+  const double cx = e1[1] * e2[2] - e1[2] * e2[1];
+  const double cy = e1[2] * e2[0] - e1[0] * e2[2];
+  const double cz = e1[0] * e2[1] - e1[1] * e2[0];
+  return sqrt((cx * cx + cy * cy) + cz * cz);
+}
+
+template <int NV>
 __device__ __forceinline__ void load_coeffs(const phifem_mesh& m, const phifem_levelset& ls, int nvpc,
-                                            int64_t c, const int (&v)[4], double* cd) {
+                                            int64_t c, const int (&v)[NV], double* cd) {
   const int nd = ls.n_dofs_per_cell;
   if (ls.dofmap == nullptr) {
     for (int i = 0; i < nvpc; ++i) cd[i] = __ldg(ls.coeffs + v[i]);
@@ -520,16 +568,18 @@ __global__ void __launch_bounds__(kBlock) k_tag_cells_generic(phifem_mesh m, phi
     int tag = -1;
     bool zden = false;
     if (c < m.n_cells) {
-      int v[4];
-      double xc[4][3];
+      int v[LocalBounds<CT>::nv];
+      double xc[LocalBounds<CT>::nv][3];
       load_cell<CT>(m, c, v, xc);
-      double cd[kMaxDofs];
+      double cd[LocalBounds<CT>::nd];
       if (ls.mode == 0) load_coeffs(m, ls, T::nv, c, v, cd);
       double s = 0.0;
-      if (CT != PHIFEM_QUADRILATERAL) s = simplex_detj<CT>(xc);
+      if constexpr (CT == PHIFEM_TRIANGLE || CT == PHIFEM_TETRAHEDRON) s = simplex_detj<CT>(xc);
       double num = 0.0, den = 0.0;
       for (int q = 0; q < npts; ++q) {
-        if (CT == PHIFEM_QUADRILATERAL) {
+        if constexpr (CT == PHIFEM_HEXAHEDRON) {
+          s = hex_detj(ls.coord_grad + q * 24, xc);  // [8 vertices][3]
+        } else if (CT == PHIFEM_QUADRILATERAL) {
           const double* g = ls.coord_grad + q * 8;  // [4 vertices][2]
           const double j00 = seq_dot(g + 0, 2, &xc[0][0], 3, 4);
           const double j01 = seq_dot(g + 1, 2, &xc[0][0], 3, 4);
@@ -587,13 +637,13 @@ template <int CT>
 __device__ __noinline__ bool owner_is_ds_cut(const phifem_mesh& m, const phifem_levelset& ls, int64_t c,
                                 int32_t this_facet, bool* first_of_cell, bool* zden) {
   using T = CellTraits<CT>;
-  int v[4];
-  double xc[4][3];
+  int v[LocalBounds<CT>::nv];
+  double xc[LocalBounds<CT>::nv][3];
   load_cell<CT>(m, c, v, xc);
-  double cd[kMaxDofs];
+  double cd[LocalBounds<CT>::nd];
   if (ls.mode == 0) load_coeffs(m, ls, T::nv, c, v, cd);
-  int32_t fid[4];
-  bool isb[4];
+  int32_t fid[LocalBounds<CT>::nf];
+  bool isb[LocalBounds<CT>::nf];
   int32_t smallest = INT32_MAX;
 #pragma unroll
   for (int i = 0; i < T::nf; ++i) {
@@ -616,12 +666,15 @@ __device__ __noinline__ bool owner_is_ds_cut(const phifem_mesh& m, const phifem_
       }
     if (lf < 0) break;
     last = best;
-    const double sc = facet_scale<CT>(xc, lf);
+    double sc = 0.0;  // hexahedra: per point (faces need not be planar)
+    if constexpr (CT != PHIFEM_HEXAHEDRON) sc = facet_scale<CT>(xc, lf);
     double fn = 0.0, fd = 0.0;
     for (int q = 0; q < nq; ++q) {
       const double ph = ls.mode == 0
                             ? seq_dot(ls.facet_table + ((int64_t)lf * nq + q) * nd, 1, cd, 1, nd)
                             : __ldg(ls.facet_values + (c * T::nf + lf) * nq + q);
+      if constexpr (CT == PHIFEM_HEXAHEDRON)
+        sc = hex_facet_scale(ls.coord_grad + ((int64_t)ls.n_cell_points + lf * nq + q) * 24, xc, lf);
       const double t = ph * sc;
       fn = fn + t;
       fd = fd + fabs(t);
@@ -1078,8 +1131,8 @@ __global__ void k_cell_points(phifem_mesh m, const double* __restrict__ shape, i
   using T = CellTraits<CT>;
   const int64_t c = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (c >= m.n_cells) return;
-  int v[4];
-  double xc[4][3];
+  int v[LocalBounds<CT>::nv];
+  double xc[LocalBounds<CT>::nv][3];
   load_cell<CT>(m, c, v, xc);
   for (int q = 0; q < npts; ++q)
     for (int d = 0; d < T::gdim; ++d)
@@ -1092,6 +1145,7 @@ int dispatch_cell_type(int ct, F&& fn) {
     case PHIFEM_TRIANGLE: fn(std::integral_constant<int, PHIFEM_TRIANGLE>()); return 0;
     case PHIFEM_QUADRILATERAL: fn(std::integral_constant<int, PHIFEM_QUADRILATERAL>()); return 0;
     case PHIFEM_TETRAHEDRON: fn(std::integral_constant<int, PHIFEM_TETRAHEDRON>()); return 0;
+    case PHIFEM_HEXAHEDRON: fn(std::integral_constant<int, PHIFEM_HEXAHEDRON>()); return 0;
   }
   return -1;
 }
@@ -1101,8 +1155,8 @@ int check_mesh(const phifem_mesh* m, bool need_facets) {
   PHIFEM_CHECK_ARG(m->x && m->cells, "mesh.x / mesh.cells is null");
   PHIFEM_CHECK_ARG(m->n_cells >= 0 && m->n_vertices >= 0, "negative sizes");
   PHIFEM_CHECK_ARG(!need_facets || (m->c2f && m->f2c), "mesh.c2f / mesh.f2c is null");
-  const int want = m->cell_type == PHIFEM_TETRAHEDRON ? 3 : 2;
-  if (m->cell_type < 0 || m->cell_type > 2) {
+  const int want = m->cell_type == PHIFEM_TETRAHEDRON || m->cell_type == PHIFEM_HEXAHEDRON ? 3 : 2;
+  if (m->cell_type < 0 || m->cell_type > 3) {
     set_error("unsupported cell type %d", m->cell_type);
     return PHIFEM_ERR_UNSUPPORTED;
   }
@@ -1112,10 +1166,14 @@ int check_mesh(const phifem_mesh* m, bool need_facets) {
 
 int check_levelset(const phifem_mesh* m, const phifem_levelset* ls, bool facets) {
   PHIFEM_CHECK_ARG(ls != nullptr, "levelset is null");
+  const bool hex = m->cell_type == PHIFEM_HEXAHEDRON;
   if (ls->mode == 0) {
     PHIFEM_CHECK_ARG(ls->coeffs != nullptr, "levelset.coeffs is null");
-    PHIFEM_CHECK_ARG(ls->n_dofs_per_cell >= 1 && ls->n_dofs_per_cell <= kMaxDofs,
+    PHIFEM_CHECK_ARG(ls->n_dofs_per_cell >= 1 &&
+                         ls->n_dofs_per_cell <= (hex ? LocalBounds<PHIFEM_HEXAHEDRON>::nd : kMaxDofs),
                      "levelset.n_dofs_per_cell out of range");
+    PHIFEM_CHECK_ARG(!hex || ls->dofmap != nullptr || ls->n_dofs_per_cell == 8,
+                     "levelset.dofmap is null and levelset.n_dofs_per_cell is not 8 (Q1 vertex dofs)");
     // a null cell_table selects the P1 vertex-dof kernel (checked again by the caller)
     PHIFEM_CHECK_ARG(!facets || ls->facet_table != nullptr, "levelset.facet_table is null");
   } else if (ls->mode == 1) {
@@ -1126,6 +1184,9 @@ int check_levelset(const phifem_mesh* m, const phifem_levelset* ls, bool facets)
   }
   PHIFEM_CHECK_ARG(facets || m->cell_type != PHIFEM_QUADRILATERAL || ls->coord_grad != nullptr,
                    "levelset.coord_grad is required for quadrilaterals");
+  PHIFEM_CHECK_ARG(!hex || ls->coord_grad != nullptr, "levelset.coord_grad is required for hexahedra");
+  PHIFEM_CHECK_ARG(!hex || (ls->n_cell_points >= 1 && ls->n_facet_points >= 1),
+                   "levelset.n_cell_points / levelset.n_facet_points must be positive for hexahedra");
   return PHIFEM_OK;
 }
 
@@ -1176,8 +1237,8 @@ extern "C" int phifem_tag_cells(const phifem_mesh* mesh, const phifem_levelset* 
   if (mesh->n_cells == 0) return PHIFEM_OK;
   cudaStream_t st = (cudaStream_t)stream;
   const int ct = mesh->cell_type;
-  const int nv = ct == PHIFEM_TRIANGLE ? 3 : 4;
-  const bool simplex = ct != PHIFEM_QUADRILATERAL;
+  const int nv = ct == PHIFEM_TRIANGLE ? 3 : (ct == PHIFEM_HEXAHEDRON ? 8 : 4);
+  const bool simplex = ct == PHIFEM_TRIANGLE || ct == PHIFEM_TETRAHEDRON;
   // P1 fast kernel: vertex dofs, identity table (detection degree 1 puts the points on the vertices)
   const bool p1 = simplex && ls->mode == 0 && ls->dofmap == nullptr && ls->n_dofs_per_cell == nv &&
                   ls->n_cell_points == nv && ls->cell_table == nullptr;
@@ -1306,10 +1367,15 @@ extern "C" int phifem_tag_facets_phase(const phifem_mesh* mesh, const phifem_lev
   auto launch_boundary = [&](auto c, cudaStream_t bs) {
     constexpr int CT = decltype(c)::value;
     const int g2 = (int)((mesh->n_boundary_facets + kBlock - 1) / kBlock);
-    if (mesh->boundary_owner && mesh->boundary_scale && CT != PHIFEM_QUADRILATERAL && boundary_kernel_records())
-      k_tag_boundary_facets_rec<CT><<<g2, kBlock, 0, bs>>>(*mesh, *ls, cell_tags8, facet_tags, facet_tags8, counters);
-    else
+    if constexpr (CT == PHIFEM_HEXAHEDRON) {  // no per-mesh records for hexahedra
       k_tag_boundary_facets<CT><<<g2, kBlock, 0, bs>>>(*mesh, *ls, cell_tags8, facet_tags, facet_tags8, counters);
+    } else {
+      if (mesh->boundary_owner && mesh->boundary_scale && CT != PHIFEM_QUADRILATERAL && boundary_kernel_records())
+        k_tag_boundary_facets_rec<CT><<<g2, kBlock, 0, bs>>>(*mesh, *ls, cell_tags8, facet_tags, facet_tags8,
+                                                             counters);
+      else
+        k_tag_boundary_facets<CT><<<g2, kBlock, 0, bs>>>(*mesh, *ls, cell_tags8, facet_tags, facet_tags8, counters);
+    }
   };
   dispatch_cell_type(mesh->cell_type, [&](auto c) {
     constexpr int CT = decltype(c)::value;
@@ -1352,11 +1418,16 @@ extern "C" int phifem_boundary_records(const phifem_mesh* mesh, uint32_t* bounda
   if (int rc = check_mesh(mesh, true)) return rc;
   PHIFEM_CHECK_ARG(mesh->n_boundary_facets == 0 || mesh->boundary_facets, "mesh.boundary_facets is null");
   PHIFEM_CHECK_ARG(mesh->n_boundary_facets == 0 || (boundary_owner && boundary_scale), "output pointer is null");
+  if (mesh->cell_type == PHIFEM_HEXAHEDRON) {  // 6 local facets do not fit the 2-bit fields of the meta word
+    set_error("phifem_boundary_records: no per-mesh boundary records for hexahedra");
+    return PHIFEM_ERR_UNSUPPORTED;
+  }
   if (mesh->n_boundary_facets == 0) return PHIFEM_OK;
   const int g = (int)((mesh->n_boundary_facets + kBlock - 1) / kBlock);
   dispatch_cell_type(mesh->cell_type, [&](auto c) {
-    k_boundary_records<decltype(c)::value><<<g, kBlock, 0, (cudaStream_t)stream>>>(*mesh, boundary_owner,
-                                                                                  boundary_scale);
+    constexpr int CT = decltype(c)::value;
+    if constexpr (CT != PHIFEM_HEXAHEDRON)
+      k_boundary_records<CT><<<g, kBlock, 0, (cudaStream_t)stream>>>(*mesh, boundary_owner, boundary_scale);
   });
   PHIFEM_CHECK_LAUNCH();
   return PHIFEM_OK;
@@ -1369,7 +1440,7 @@ extern "C" int phifem_entity_records(const phifem_mesh* mesh, const int8_t* cell
   if (int rc = check_mesh(mesh, true)) return rc;
   PHIFEM_CHECK_ARG(cell_tags8 && facet_tags8 && n_records && (records || capacity == 0), "null pointer");
   if (mesh->n_facets == 0) return PHIFEM_OK;
-  const int nf = mesh->cell_type == PHIFEM_TRIANGLE ? 3 : 4;
+  const int nf = mesh->cell_type == PHIFEM_TRIANGLE ? 3 : (mesh->cell_type == PHIFEM_HEXAHEDRON ? 6 : 4);
   const int grid = (int)((mesh->n_facets + kBlock - 1) / kBlock);
   k_entity_records<<<grid, kBlock, 0, (cudaStream_t)stream>>>(
       *mesh, nf, cell_tags8, facet_tags8, facet_tag, cell_mask, records, capacity,

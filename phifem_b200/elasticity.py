@@ -25,7 +25,7 @@ import numpy as np
 import torch
 
 from . import _lib, quadrature
-from .assemble import CSRMatrix, _device_vector, _plan_inputs
+from .assemble import CSRMatrix, _device_vector, _plan_inputs, refuse_hexahedra
 
 FIELDS = ("u_in", "u_out", "y_in", "y_out", "p")
 
@@ -57,6 +57,7 @@ class ElasticityPlan:
     form = "interface-elasticity"
 
     def __init__(self, mesh, cell_tags8, facet_tags8, ents_in, ents_out, V_phi):
+        refuse_hexahedra(mesh, "ElasticityPlan")
         if mesh.cell_type not in ("triangle", "tetrahedron", "quadrilateral"):
             raise NotImplementedError("the interface-elasticity operator supports triangles, quadrilaterals and "
                                       "tetrahedra")

@@ -32,18 +32,23 @@ LOCAL_EDGES = {
     "triangle": ((1, 2), (0, 2), (0, 1)),
     "quadrilateral": ((0, 1), (0, 2), (1, 3), (2, 3)),
     "tetrahedron": ((2, 3), (1, 3), (1, 2), (0, 3), (0, 2), (0, 1)),
+    "hexahedron": ((0, 1), (0, 2), (0, 4), (1, 3), (1, 5), (2, 3), (2, 6), (3, 7), (4, 5), (4, 6), (5, 7), (6, 7)),
 }
-LOCAL_FACES = {"tetrahedron": ((1, 2, 3), (0, 2, 3), (0, 1, 3), (0, 1, 2))}
+LOCAL_FACES = {"tetrahedron": ((1, 2, 3), (0, 2, 3), (0, 1, 3), (0, 1, 2)),
+               "hexahedron": ((0, 1, 2, 3), (0, 1, 4, 5), (0, 2, 4, 6), (1, 3, 5, 7), (2, 3, 6, 7), (4, 5, 6, 7))}
 REF_VERTICES = {
     "triangle": np.array([[0.0, 0.0], [1.0, 0.0], [0.0, 1.0]]),
     "quadrilateral": np.array([[0.0, 0.0], [1.0, 0.0], [0.0, 1.0], [1.0, 1.0]]),
     "tetrahedron": np.array([[0.0, 0, 0], [1.0, 0, 0], [0, 1.0, 0], [0, 0, 1.0]]),
+    "hexahedron": np.array([[i, j, k] for k in (0.0, 1.0) for j in (0.0, 1.0) for i in (0.0, 1.0)]),
 }
 
 
 def _monomial_exponents(cell_type, k):
     if cell_type == "quadrilateral":
         return [(i, j) for i in range(k + 1) for j in range(k + 1)]
+    if cell_type == "hexahedron":
+        return list(itertools.product(range(k + 1), repeat=3))
     tdim = 2 if cell_type == "triangle" else 3
     return [e for e in itertools.product(range(k + 1), repeat=tdim) if sum(e) <= k]
 
@@ -59,13 +64,16 @@ def _monomials(exps, pts):
 
 
 class LagrangeElement:
-    """Reference Lagrange element of degree 1..3 on triangle / quadrilateral / tetrahedron."""
+    """Reference Lagrange element of degree 1..3 on triangle / quadrilateral / tetrahedron, 1..2 on hexahedron
+    (Q2 nodes: vertices, edge midpoints, face centres, centre)."""
 
     def __init__(self, cell_type, degree):
         if cell_type not in REF_VERTICES:
             raise NotImplementedError(cell_type)
         if degree not in (1, 2, 3):
             raise NotImplementedError("Lagrange degree %d" % degree)
+        if cell_type == "hexahedron" and degree == 3:
+            raise NotImplementedError("Lagrange degree 3 on hexahedra")
         self.cell_type, self.degree = cell_type, degree
         rv = REF_VERTICES[cell_type]
         k = degree
@@ -77,7 +85,7 @@ class LagrangeElement:
             for j, s in enumerate(inner):
                 nodes.append((1 - s) * rv[a] + s * rv[b])
                 ents.append(("e", e, j))
-        if cell_type == "tetrahedron" and k == 3:
+        if (cell_type == "tetrahedron" and k == 3) or (cell_type == "hexahedron" and k == 2):
             for f, face in enumerate(LOCAL_FACES[cell_type]):
                 nodes.append(rv[list(face)].mean(axis=0))
                 ents.append(("f", f, 0))
@@ -88,6 +96,9 @@ class LagrangeElement:
             for j, (sy, sx) in enumerate(itertools.product(inner, inner)):
                 nodes.append(np.array([sx, sy]))
                 ents.append(("c", 0, j))
+        if cell_type == "hexahedron" and k == 2:
+            nodes.append(rv.mean(axis=0))
+            ents.append(("c", 0, 0))
         self.nodes = np.array(nodes)
         self.entities = ents
         self.exps = _monomial_exponents(cell_type, k)
@@ -166,9 +177,10 @@ class FunctionSpace:
             offset += n_edges * (k - 1)
         kinds = [ent[0] for ent in self.element.entities]
         if "f" in kinds:
+            # one dof per face, faces numbered by the lexicographic rank of their sorted vertex tuple
             faces = LOCAL_FACES[mesh.cell_type]
-            tri = np.sort(np.stack([cells[:, list(f)] for f in faces], axis=1), axis=2)
-            _, inv = _unique_rows(tri.reshape(-1, 3))
+            tup = np.sort(np.stack([cells[:, list(f)] for f in faces], axis=1), axis=2)
+            _, inv = _unique_rows(tup.reshape(-1, len(faces[0])))
             fid = inv.reshape(nc, len(faces))
             for f in range(len(faces)):
                 cols.append((offset + fid[:, f])[:, None])

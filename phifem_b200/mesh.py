@@ -9,7 +9,7 @@ duck-typed dolfinx-style accessors.
 Layout in HBM (row-major, int32 indices, fp64 coordinates):
     x      [Nv, gdim]   vertex coordinates
     cells  [Nc, nvpc]   cell -> vertex (dolfinx local order)
-    c2f    [Nc, nfpc]   cell -> facet, local facet i opposite local vertex i on simplices
+    c2f    [Nc, nfpc]   cell -> facet, local facet i opposite local vertex i on simplices, _geometry.LOCAL_FACETS order
     f2c    [Nf, 2]      facet -> cells ascending, -1 pad on the mesh boundary
     fverts [Nf, nvpf]   facet -> sorted vertex tuple
 
@@ -115,7 +115,8 @@ def morton_keys(pts, bits=21):
 
 
 class Mesh:
-    """Unstructured mesh of triangles, quadrilaterals or tetrahedra on one device."""
+    """Unstructured mesh of triangles, quadrilaterals, tetrahedra or hexahedra on one device (quadrilaterals and
+    hexahedra with their vertices in tensor order)."""
 
     def __init__(self, x, cells, cell_type, device=None):
         if cell_type not in G.CELL_TYPES:
@@ -300,11 +301,11 @@ class Mesh:
         return self._host["brec"]
 
     def detj_bounds(self):
-        """(min, max) of |det J| over the simplices of the mesh, cached.  A property of the mesh
+        """(min, max) of |det J| over the simplices of the mesh, cached ((0, 0) = unknown on other cells).  A property of the mesh
         alone: lets the P1 classifier decide uncut cells from the signs of phi without gathering
         coordinates (csrc/tags.cu, k_tag_cells_p1)."""
         if "detj" not in self._host:
-            if self.cell_type == "quadrilateral" or self.num_cells == 0:
+            if self.cell_type not in G.SIMPLICES or self.num_cells == 0:
                 self._host["detj"] = (0.0, 0.0)
             else:
                 lo, hi = float("inf"), 0.0
@@ -349,7 +350,7 @@ def build_facet_topology(cells, cell_type, num_vertices):
     if nvpf == 2:
         uniq, inv = _unique_inverse(key)
         fverts = torch.stack([uniq // nv, uniq % nv], dim=1)
-    else:
+    elif nvpf == 3:
         upair, pinv = _unique_inverse(key)          # rank of the leading pair keeps lexicographic order
         key = pinv * nv + inst[:, 2]
         del pinv
@@ -357,6 +358,19 @@ def build_facet_topology(cells, cell_type, num_vertices):
         pair = upair[uniq // nv]
         fverts = torch.stack([pair // nv, pair % nv, uniq % nv], dim=1)
         del upair, pair
+    else:
+        # hexahedron faces: one more round; the rank of the leading triple keeps the order lexicographic
+        upair, pinv = _unique_inverse(key)
+        key = pinv * nv + inst[:, 2]
+        del pinv
+        utrip, tinv = _unique_inverse(key)
+        key = tinv * nv + inst[:, 3]
+        del tinv
+        uniq, inv = _unique_inverse(key)
+        trip = utrip[uniq // nv]
+        pair = upair[trip // nv]
+        fverts = torch.stack([pair // nv, pair % nv, trip % nv, uniq % nv], dim=1)
+        del upair, utrip, trip, pair
     del inst, key
     nf = int(uniq.shape[0])
     c2f = inv.reshape(nc, nfpc).to(torch.int32)

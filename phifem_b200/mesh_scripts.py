@@ -11,8 +11,9 @@ Public API (reference :571-653):
         mesh, discrete_levelset, detection_degree, box_mode=False, single_layer_cut=False,
         overwrite_tags={})
 
-`mesh` is a `phifem_b200.mesh.Mesh`; `discrete_levelset` is a `phifem_b200.fem.Function`
-(P1..P3) or a callable of the physical coordinates `f(x)` with `x` of shape (gdim, npoints)
+`mesh` is a `phifem_b200.mesh.Mesh` of triangles, quadrilaterals, tetrahedra or hexahedra (the last two are
+extensions: the reference stops at 2D); `discrete_levelset` is a `phifem_b200.fem.Function`
+(P1..P3, Q1..Q3, Q1 / Q2 on hexahedra) or a callable of the physical coordinates `f(x)` with `x` of shape (gdim, npoints)
 (the stand-in for the reference's UFL expression of `SpatialCoordinate`).
 """
 import os
@@ -51,6 +52,12 @@ class _DeviceLevelset:
         coord_grad = None
         if ct == "quadrilateral":
             coord_grad = torch.as_tensor(G.coordinate_basis_grad(ct, pts), **f64).contiguous()
+        elif ct == "hexahedron":
+            # [npts + nfpc nq, 8, 3]: the trilinear map's gradients at the cell points, then at the facet points --
+            # the kernels take |det J| and the face scale |dx/ds x dx/dt| per point from them
+            grads = np.concatenate([G.coordinate_basis_grad(ct, pts),
+                                    G.coordinate_basis_grad(ct, fpts.reshape(-1, fpts.shape[-1]))])
+            coord_grad = torch.as_tensor(grads, **f64).contiguous()
         self.c = _lib.CLevelset()
         self.c.n_cell_points, self.c.n_facet_points = self.npts, self.nq
         self.c.coord_grad = _lib.ptr(coord_grad)
@@ -63,7 +70,7 @@ class _DeviceLevelset:
             coeffs = coeffs if torch.is_tensor(coeffs) else torch.from_numpy(np.ascontiguousarray(coeffs))
             coeffs = coeffs.to(dev, dtype=torch.float64, non_blocking=True).contiguous()
             nd = V.element.ndofs
-            simplex_p1 = (V.degree == 1 and detection_degree == 1 and ct != "quadrilateral")
+            simplex_p1 = (V.degree == 1 and detection_degree == 1 and ct in G.SIMPLICES)
             self.c.mode, self.c.n_dofs_per_cell = 0, nd
             self.c.coeffs = _lib.ptr(coeffs)
             ftab = torch.as_tensor(V.element.tabulate(fpts), **f64).contiguous()

@@ -71,6 +71,7 @@ class PartitionedProblem:
     share only: symbolic time and memory of a rank shrink with the number of ranks)."""
 
     def __init__(self, mesh, phi, f, rank, world, group=None, weights=None, single_layer_cut=False):
+        assemble.refuse_hexahedra(mesh, "PartitionedProblem")
         if mesh.cell_type not in ("triangle", "tetrahedron"):
             raise NotImplementedError("sharding supports triangles and tetrahedra")
         cell_owner, vowner = self.ownership(mesh, world, weights)
@@ -122,6 +123,7 @@ class PartitionedProblem:
                   torch.uint8)
         mine = None
         if rank == src:
+            assemble.refuse_hexahedra(mesh, "PartitionedProblem.scatter")
             if mesh.cell_type not in ("triangle", "tetrahedron"):
                 raise NotImplementedError("sharding supports triangles and tetrahedra")
             cell_owner, vowner = cls.ownership(mesh, world, weights)

@@ -3,7 +3,7 @@
 S-2D(n): n x n squares split by the "right" diagonal -> 2 n^2 triangles (what
 `dolfinx.mesh.create_rectangle` gives the reference demos,
 demo/strong-dirichlet/flower/main.py:48-49).  Q-2D(n): the same n x n squares as quadrilaterals (the cell type of
-demo/neumann/square).  S-3D(n): n^3 cubes x 6 Kuhn tetrahedra.
+demo/neumann/square).  S-3D(n): n^3 cubes x 6 Kuhn tetrahedra; H-3D(n): the same n^3 cubes as hexahedra.
 Vertices are numbered lexicographically; generated directly on the target device.
 """
 import itertools
@@ -71,6 +71,26 @@ def box_mesh(n, lo=(0.0, 0.0, 0.0), hi=(1.0, 1.0, 1.0), device=None):
         tets.append(base[:, None] + torch.tensor(offs, device=device, dtype=torch.int64)[None, :])
     cells = torch.stack(tets, dim=1).reshape(-1, 4).to(torch.int32)
     return Mesh(x, cells, "tetrahedron", device)
+
+
+def hexahedron_mesh(n, lo=(0.0, 0.0, 0.0), hi=(1.0, 1.0, 1.0), device=None):
+    """nx ny nz hexahedra (n = int or (nx, ny, nz)) in dolfinx tensor order (v0 = (x_i, y_j, z_k), v1 = +x, v2 = +y,
+    v3 = +x+y, v4..v7 the same at z_k+1); the vertices and vertex ids of `box_mesh`, cubes ordered x-major, so that
+    the two meshes can be compared cube by cube."""
+    device = torch.device(device) if device is not None else default_device()
+    nx, ny, nz = (n, n, n) if isinstance(n, int) else n
+    axes = [torch.linspace(float(a), float(b), m + 1, dtype=torch.float64, device=device)
+            for a, b, m in zip(lo, hi, (nx, ny, nz))]
+    grids = torch.meshgrid(*axes, indexing="ij")
+    x = torch.stack([g.reshape(-1) for g in grids], dim=1).contiguous()
+    I, J, K = torch.meshgrid(*[torch.arange(m, device=device, dtype=torch.int64) for m in (nx, ny, nz)],
+                             indexing="ij")
+    base = ((I * (ny + 1) + J) * (nz + 1) + K).reshape(-1)
+    sx, sy, sz = (ny + 1) * (nz + 1), nz + 1, 1
+    offs = torch.tensor([i * sx + j * sy + k * sz for k in (0, 1) for j in (0, 1) for i in (0, 1)],
+                        device=device, dtype=torch.int64)
+    cells = (base[:, None] + offs[None, :]).to(torch.int32).contiguous()
+    return Mesh(x, cells, "hexahedron", device)
 
 
 def unstructured_variant(mesh, jitter=0.2, seed=0):
