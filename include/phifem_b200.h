@@ -602,6 +602,48 @@ void phifem_pattern_destroy(phifem_pattern* pattern);
  * pool that stays cached between calls; this returns it to the driver. */
 void phifem_pattern_release_scratch(void);
 
+/* ---- symbolic phase of the quadrature-kernel operators on the device: the CSR pattern, active cells, cut-cell positions,
+ * ghost-penalty facets and the three entity -> CSR-slot maps that phifem_assemble_{cells,boundary,ghost}_pk,
+ * phifem_assemble_weak_*_pk and phifem_assemble_neumann_* take.  Every array equals, bit for bit, what
+ * phifem_b200/assemble_pk.py (PkAssemblyPlan) builds with torch sort / unique for the same inputs, on triangles,
+ * quadrilaterals and tetrahedra (hexahedra return PHIFEM_ERR_UNSUPPORTED: nothing assembles on them).
+ *   dofmap [n_cells, nd]  the PATTERN dofmap: the cell-local dofs of the space being assembled, global ids in
+ *                         [0, n_rows), 1 <= nd <= 32:
+ *                           strong Dirichlet  the trial / test space's dofmap (n_rows = its n_dofs);
+ *                           weak Dirichlet    [2 dofmap, 2 dofmap + 1] (n_rows = 2 n_dofs);
+ *                           Neumann / Robin   [(d+1) v, (d+1) v + 1 + c (node-major), (d+1) n_vertices + k]
+ *                                             (n_rows = (d+1) n_vertices + n_cells);
+ *   ghost_tag_mask        bit t set for every facet tag t (0..6) that carries the ghost penalty: (1<<2)|(1<<3) for strong
+ *                         and weak Dirichlet, 1<<3 for the Neumann demo, 1<<2 for the Robin demo; only interior facets
+ *                         (f2c[f][1] >= 0) are taken;
+ *   entities [n_entities, 2]  the (cell, local facet) pairs of ds(100) (may be empty); their cells must be tagged 1 / 2.
+ * The pattern is the sorted unique set of keys row * n_rows + col over the active cells' nd x nd pairs and the ghost macro
+ * elements' (2 nd) x (2 nd) pairs; a slot is the position of its key.  At most 2^31 - 1 keys (else PHIFEM_ERR_ARGUMENT:
+ * shard the mesh).  A dofmap entry outside [0, n_rows), or an entity whose cell is not tagged 1 / 2 or whose local facet
+ * is out of range, returns PHIFEM_ERR_ARGUMENT (checked on the device).  Sort scratch: about 32 bytes per pattern key and
+ * 8 per entity key, from the pool phifem_pattern_release_scratch trims.  The handle owns its arrays (cudaMalloc); the
+ * call synchronises the stream as phifem_pattern_create_p1 does. */
+typedef struct phifem_pk_pattern phifem_pk_pattern;
+typedef struct phifem_pk_pattern_view {
+  int64_t n_rows, nnz;            /* nnz < 2^31 */
+  int32_t nd;                     /* dofs per cell of the pattern dofmap */
+  int64_t n_active, n_cut, n_ghost, n_entities;
+  const int32_t* indptr;          /* [n_rows + 1] */
+  const int32_t* indices;         /* [nnz], sorted per row, structural zeros kept, rows without contributions empty */
+  const int32_t* active;          /* [n_active] cells tagged 1 / 2, ascending */
+  const int32_t* cut_positions;   /* [n_cut] positions in `active` of the cells tagged 2 (the Neumann entry points) */
+  const int32_t* ghost;           /* [n_ghost] interior facets whose tag is in ghost_tag_mask, ascending */
+  const int32_t* slots_cells;     /* [nd*nd, n_active]     entry-major, as phifem_assemble_cells_pk expects */
+  const int32_t* slots_ghost;     /* [n_ghost, (2 nd)^2]   macro = [dofs of f2c[f][0], dofs of f2c[f][1]] */
+  const int32_t* slots_boundary;  /* [n_entities, nd*nd] */
+} phifem_pk_pattern_view;
+
+int phifem_pk_pattern_create(const phifem_mesh* mesh, const int32_t* dofmap, int32_t nd, int64_t n_rows,
+                             const int8_t* cell_tags8, const int8_t* facet_tags8, uint32_t ghost_tag_mask,
+                             const int32_t* entities, int64_t n_entities, phifem_pk_pattern** out, void* stream);
+int phifem_pk_pattern_view_of(const phifem_pk_pattern* pattern, phifem_pk_pattern_view* out);
+void phifem_pk_pattern_destroy(phifem_pk_pattern* pattern);
+
 /* ---- the row-gather plan itself, built on the device (csrc/rows_plan.cu): CSR pattern (indptr, indices), active cells,
  * ghost facets and the two row lists of phifem_rows_plan, from the vertex -> cell adjacency (one radix sort of
  * n_active * nv keys, per-row merges) instead of one key per coupled vertex pair.  Every array equals what

@@ -88,6 +88,14 @@ class CPatternView(ctypes.Structure):
                 ("active", _vp), ("ghost", _vp), ("slots_cells", _vp), ("slots_ghost", _vp), ("slots_boundary", _vp)]
 
 
+class CPkPatternView(ctypes.Structure):
+    _fields_ = [("n_rows", ctypes.c_int64), ("nnz", ctypes.c_int64), ("nd", ctypes.c_int32),
+                ("n_active", ctypes.c_int64), ("n_cut", ctypes.c_int64), ("n_ghost", ctypes.c_int64),
+                ("n_entities", ctypes.c_int64), ("indptr", _vp), ("indices", _vp), ("active", _vp),
+                ("cut_positions", _vp), ("ghost", _vp), ("slots_cells", _vp), ("slots_ghost", _vp),
+                ("slots_boundary", _vp)]
+
+
 class CElasticityParams(ctypes.Structure):
     _fields_ = [(n, ctypes.c_double) for n in ("lmbda_in", "mu_in", "lmbda_out", "mu_out", "coef_in", "coef_out",
                                                "gamma", "sigma_s")]
@@ -167,6 +175,10 @@ _SIGNATURES = {
     "phifem_integration_entities_fill": (ctypes.c_int, [ctypes.POINTER(CMesh), _vp, _vp, ctypes.c_int32,
                                                         ctypes.c_uint32, _vp, ctypes.c_int64, _vp]),
     "phifem_pattern_destroy": (None, [_vp]),
+    "phifem_pk_pattern_create": (ctypes.c_int, [ctypes.POINTER(CMesh), _vp, ctypes.c_int32, ctypes.c_int64, _vp, _vp,
+                                                ctypes.c_uint32, _vp, ctypes.c_int64, ctypes.POINTER(_vp), _vp]),
+    "phifem_pk_pattern_view_of": (ctypes.c_int, [_vp, ctypes.POINTER(CPkPatternView)]),
+    "phifem_pk_pattern_destroy": (None, [_vp]),
     "phifem_surface_static_p1": (ctypes.c_int, [ctypes.POINTER(CMesh), ctypes.POINTER(CRowsPlan), _vp]),
     "phifem_rows_plan_create": (ctypes.c_int, [ctypes.POINTER(CMesh), _vp, _vp, _vp, ctypes.c_int64, _vp,
                                                ctypes.c_int32, ctypes.POINTER(_vp), _vp]),

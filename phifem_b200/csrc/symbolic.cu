@@ -21,6 +21,12 @@ struct phifem_pattern {
   int n_owned;
 };
 
+struct phifem_pk_pattern {
+  phifem_pk_pattern_view v;
+  void* owned[8];
+  int n_owned;
+};
+
 namespace phifem {
 // A private stream-ordered pool per device whose memory stays cached between calls (release threshold = max): the
 // default pool hands its memory back to the driver at every synchronisation, and re-allocating the ~10 GB of sort
@@ -131,6 +137,60 @@ __global__ void k_columns(const int64_t* __restrict__ uniq, int64_t nnz, int64_t
 }
 
 inline unsigned blocks_for(int64_t n) { return (unsigned)((n + kBlockSym - 1) / kBlockSym); }
+
+// ---- quadrature-kernel operators (phifem_pk_pattern_create): the same keys over a caller-given pattern dofmap
+
+struct IsMaskedGhostFacet {  // interior facets whose tag t has bit t set in `mask`
+  const int8_t* tags;
+  const int32_t* f2c;
+  uint32_t mask;
+  __device__ bool operator()(int f) const {
+    const int t = tags[f];
+    return t >= 0 && t < 7 && ((mask >> t) & 1u) && f2c[2 * (int64_t)f + 1] >= 0;
+  }
+};
+struct IsCutPosition {  // positions in `active` of the cells tagged 2
+  const int8_t* tags;
+  const int32_t* active;
+  __device__ bool operator()(int p) const { return tags[active[p]] == 2; }
+};
+
+// input checks: dofmap entries outside [0, n_rows), entities outside the active cells or their local facets
+__global__ void k_count_dofs_out_of_range(const int32_t* __restrict__ dofmap, int64_t n, int64_t n_rows,
+                                          unsigned long long* __restrict__ bad) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t < n && (dofmap[t] < 0 || dofmap[t] >= n_rows)) atomicAdd(bad, 1ull);
+}
+__global__ void k_count_bad_entities(const int32_t* __restrict__ entities, int64_t n, const int8_t* __restrict__ tags,
+                                     int64_t n_cells, int n_local_facets, unsigned long long* __restrict__ bad) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  const int32_t c = entities[2 * t], lf = entities[2 * t + 1];
+  if (c < 0 || c >= n_cells || lf < 0 || lf >= n_local_facets || (tags[c] != 1 && tags[c] != 2)) atomicAdd(bad, 1ull);
+}
+
+// keys of the active cells' dof pairs, entry-major: keys[r * n + e] = pair r = (i, j) of cell list[e], so that the slots
+// k_slots writes come out as [nd*nd, n] (the layout of phifem_assemble_cells_pk)
+__global__ void k_cell_pair_keys_entry_major(const int32_t* __restrict__ dofmap, int nd,
+                                             const int32_t* __restrict__ list, int64_t n, int64_t n_rows,
+                                             int64_t* __restrict__ keys) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n * nd * nd) return;
+  const int r = (int)(t / n);
+  const int64_t c = list[t - r * n];
+  keys[t] = (int64_t)dofmap[c * nd + r / nd] * n_rows + dofmap[c * nd + r % nd];
+}
+
+// macro dofs of an interior facet: [dofs of f2c[f][0], dofs of f2c[f][1]]
+__global__ void k_macro_dofs(const int32_t* __restrict__ f2c, const int32_t* __restrict__ dofmap, int nd,
+                             const int32_t* __restrict__ facets, int64_t n, int32_t* __restrict__ macro) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n * 2 * nd) return;
+  const int64_t e = t / (2 * nd);
+  const int k = (int)(t - e * 2 * nd);
+  const int64_t c = f2c[2 * (int64_t)facets[e] + k / nd];
+  macro[t] = dofmap[c * nd + k % nd];
+}
 
 // ordering of `_compute_integration_entities` (mesh_scripts.py:137-192): cells in first-appearance order of the
 // candidate records (key = 2 facet + column), the local facets of a cell ascending
@@ -328,6 +388,194 @@ extern "C" int phifem_pattern_create_p1(const phifem_mesh* mesh, const int8_t* c
   pat->v.indptr = indptr;
   pat->v.indices = indices;
   pat->v.active = active;
+  pat->v.ghost = ghost;
+  pat->v.slots_cells = slots_c;
+  pat->v.slots_ghost = slots_g;
+  pat->v.slots_boundary = slots_b;
+  *out = pat;
+  return PHIFEM_OK;
+}
+
+extern "C" void phifem_pk_pattern_destroy(phifem_pk_pattern* p) {
+  if (!p) return;
+  for (int i = 0; i < p->n_owned; ++i) cudaFree(p->owned[i]);
+  delete p;
+}
+
+extern "C" int phifem_pk_pattern_view_of(const phifem_pk_pattern* p, phifem_pk_pattern_view* out) {
+  PHIFEM_CHECK_ARG(p && out, "null pointer");
+  *out = p->v;
+  return PHIFEM_OK;
+}
+
+// The arrays of PkAssemblyPlan (phifem_b200/assemble_pk.py), bit for bit: pattern = sorted unique keys
+// row * n_rows + col of the active cells' nd x nd dof pairs and of the ghost macro elements' (2 nd) x (2 nd) pairs, slot =
+// position of a key in that list (the entities' keys are looked up, they add no entry).
+extern "C" int phifem_pk_pattern_create(const phifem_mesh* mesh, const int32_t* dofmap, int32_t nd, int64_t n_rows,
+                                        const int8_t* cell_tags8, const int8_t* facet_tags8, uint32_t ghost_tag_mask,
+                                        const int32_t* entities, int64_t n_entities, phifem_pk_pattern** out,
+                                        void* stream) {
+  PHIFEM_CHECK_ARG(out != nullptr, "out is null");
+  *out = nullptr;
+  PHIFEM_CHECK_ARG(mesh != nullptr && mesh->cells && mesh->c2f && mesh->f2c, "mesh / facet connectivity is null");
+  if (mesh->cell_type != PHIFEM_TRIANGLE && mesh->cell_type != PHIFEM_TETRAHEDRON &&
+      mesh->cell_type != PHIFEM_QUADRILATERAL) {
+    set_error("phifem_pk_pattern_create: the quadrature-kernel operators assemble on triangles, quadrilaterals and "
+              "tetrahedra, got cell type %d", mesh->cell_type);
+    return PHIFEM_ERR_UNSUPPORTED;
+  }
+  PHIFEM_CHECK_ARG(dofmap != nullptr, "dofmap is null");
+  PHIFEM_CHECK_ARG(cell_tags8 && facet_tags8, "tag arrays are null");
+  PHIFEM_CHECK_ARG(nd >= 1 && nd <= 32, "nd (dofs per cell) must lie in 1..32");
+  PHIFEM_CHECK_ARG(n_rows >= 1 && n_rows < (1ll << 31), "n_rows must lie in 1..2^31-1");
+  PHIFEM_CHECK_ARG(n_entities >= 0 && (n_entities == 0 || entities), "entity list");
+  PHIFEM_CHECK_ARG((ghost_tag_mask >> 7) == 0, "ghost_tag_mask sets bits outside the tag values 0..6");
+  PHIFEM_CHECK_ARG(mesh->n_cells < (1ll << 31) && mesh->n_facets < (1ll << 31), "int32 index width");
+  const int n_local_facets = mesh->cell_type == PHIFEM_TRIANGLE ? 3 : 4;
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaMemPool_t pool = scratch_pool();
+  if (!pool) {
+    set_error("phifem_pk_pattern_create: cannot create the scratch memory pool");
+    return PHIFEM_ERR_CUDA;
+  }
+  Scratch tmp(st, pool);
+  phifem_pk_pattern* pat = new phifem_pk_pattern();
+  pat->n_owned = 0;
+  auto own = [&](size_t bytes) -> void* {
+    void* q = nullptr;
+    if (cudaMalloc(&q, bytes ? bytes : 1) != cudaSuccess) return nullptr;
+    pat->owned[pat->n_owned++] = q;
+    return q;
+  };
+  auto fail = [&](const char* what) {
+    set_error("phifem_pk_pattern_create: %s: %s", what, cudaGetErrorString(cudaGetLastError()));
+    phifem_pk_pattern_destroy(pat);
+    return PHIFEM_ERR_CUDA;
+  };
+  auto refuse = [&](const char* what) {
+    set_error("phifem_pk_pattern_create: %s", what);
+    phifem_pk_pattern_destroy(pat);
+    return PHIFEM_ERR_ARGUMENT;
+  };
+
+  // 1. active cells (tags 1 / 2) and ghost-penalty facets (interior facets whose tag is in the mask), ascending; the
+  //    input checks count into the same block: {n_active, n_ghost, bad dofs, bad entities, n_cut, nnz}
+  int32_t* active_full = (int32_t*)tmp.get(sizeof(int32_t) * mesh->n_cells);
+  int32_t* ghost_full = (int32_t*)tmp.get(sizeof(int32_t) * mesh->n_facets);
+  int64_t* counts = (int64_t*)tmp.get(6 * sizeof(int64_t));
+  if (!active_full || !ghost_full || !counts) return fail("scratch allocation");
+  cudaMemsetAsync(counts, 0, 6 * sizeof(int64_t), st);
+  {
+    thrust::counting_iterator<int> it(0);
+    const IsMaskedGhostFacet is_ghost{facet_tags8, mesh->f2c, ghost_tag_mask};
+    size_t b1 = 0, b2 = 0;
+    cub::DeviceSelect::If(nullptr, b1, it, active_full, counts, (int)mesh->n_cells, IsActiveCell{cell_tags8}, st);
+    cub::DeviceSelect::If(nullptr, b2, it, ghost_full, counts + 1, (int)mesh->n_facets, is_ghost, st);
+    void* ws = tmp.get(b1 > b2 ? b1 : b2);
+    if (!ws) return fail("scratch allocation");
+    cub::DeviceSelect::If(ws, b1, it, active_full, counts, (int)mesh->n_cells, IsActiveCell{cell_tags8}, st);
+    cub::DeviceSelect::If(ws, b2, it, ghost_full, counts + 1, (int)mesh->n_facets, is_ghost, st);
+  }
+  unsigned long long* bad = (unsigned long long*)(counts + 2);
+  if (mesh->n_cells)
+    k_count_dofs_out_of_range<<<blocks_for(mesh->n_cells * nd), kBlockSym, 0, st>>>(dofmap, mesh->n_cells * nd,
+                                                                                    n_rows, bad);
+  if (n_entities)
+    k_count_bad_entities<<<blocks_for(n_entities), kBlockSym, 0, st>>>(entities, n_entities, cell_tags8, mesh->n_cells,
+                                                                       n_local_facets, bad + 1);
+  int64_t h_counts[4] = {0, 0, 0, 0};
+  if (cudaMemcpyAsync(h_counts, counts, sizeof(h_counts), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+      cudaStreamSynchronize(st) != cudaSuccess)
+    return fail("compaction");
+  if (h_counts[2]) return refuse("dofmap has entries outside [0, n_rows)");
+  if (h_counts[3])
+    return refuse("entities: an entity's cell is not tagged 1 or 2, or its local facet is out of range");
+  const int64_t na = h_counts[0], ng = h_counts[1];
+  const int64_t kc = na * nd * nd, kg = ng * 4 * nd * nd, kb = n_entities * nd * nd, nk = kc + kg;
+  if (nk >= (1ll << 31)) {
+    set_error("phifem_pk_pattern_create: %lld coupled pairs (limit 2^31): shard the mesh", (long long)nk);
+    phifem_pk_pattern_destroy(pat);
+    return PHIFEM_ERR_ARGUMENT;
+  }
+  int32_t* active = (int32_t*)own(sizeof(int32_t) * na);
+  int32_t* ghost = (int32_t*)own(sizeof(int32_t) * ng);
+  if (!active || !ghost) return fail("output allocation");
+  cudaMemcpyAsync(active, active_full, sizeof(int32_t) * na, cudaMemcpyDeviceToDevice, st);
+  cudaMemcpyAsync(ghost, ghost_full, sizeof(int32_t) * ng, cudaMemcpyDeviceToDevice, st);
+
+  // 2. cut cells: positions in `active` of the cells tagged 2 (their count comes back with nnz)
+  int32_t* cut_full = (int32_t*)tmp.get(sizeof(int32_t) * na);
+  if (!cut_full) return fail("scratch allocation");
+  if (na) {
+    thrust::counting_iterator<int> it(0);
+    const IsCutPosition is_cut{cell_tags8, active};
+    size_t b = 0;
+    cub::DeviceSelect::If(nullptr, b, it, cut_full, counts + 4, (int)na, is_cut, st);
+    void* ws = tmp.get(b);
+    if (!ws) return fail("scratch allocation");
+    cub::DeviceSelect::If(ws, b, it, cut_full, counts + 4, (int)na, is_cut, st);
+  }
+
+  // 3. keys: active cells (entry-major), ghost macro elements, one-sided entities (looked up only)
+  int64_t* keys = (int64_t*)tmp.get(sizeof(int64_t) * (nk + kb));
+  int32_t* macro = (int32_t*)tmp.get(sizeof(int32_t) * ng * 2 * nd);
+  if (!keys || !macro) return fail("scratch allocation");
+  if (kc) k_cell_pair_keys_entry_major<<<blocks_for(kc), kBlockSym, 0, st>>>(dofmap, nd, active, na, n_rows, keys);
+  if (ng) {
+    k_macro_dofs<<<blocks_for(ng * 2 * nd), kBlockSym, 0, st>>>(mesh->f2c, dofmap, nd, ghost, ng, macro);
+    k_pair_keys<<<blocks_for(kg), kBlockSym, 0, st>>>(macro, ng, 2 * nd, n_rows, keys + kc);
+  }
+  if (kb) k_cell_pair_keys<<<blocks_for(kb), kBlockSym, 0, st>>>(dofmap, nd, entities, 2, n_entities, n_rows, keys + nk);
+
+  // 4. pattern = sorted unique keys of the cells and macro elements
+  int64_t* sorted = (int64_t*)tmp.get(sizeof(int64_t) * nk);
+  int64_t* uniq = (int64_t*)tmp.get(sizeof(int64_t) * nk);
+  if (!sorted || !uniq) return fail("scratch allocation");
+  if (nk) {
+    int end_bit = 1;
+    while (end_bit < 63 && (1ll << end_bit) < n_rows * n_rows) ++end_bit;
+    size_t b1 = 0, b2 = 0;
+    cub::DeviceRadixSort::SortKeys(nullptr, b1, keys, sorted, (int)nk, 0, end_bit, st);
+    cub::DeviceSelect::Unique(nullptr, b2, sorted, uniq, counts + 5, (int)nk, st);
+    void* ws = tmp.get(b1 > b2 ? b1 : b2);
+    if (!ws) return fail("scratch allocation");
+    cub::DeviceRadixSort::SortKeys(ws, b1, keys, sorted, (int)nk, 0, end_bit, st);
+    cub::DeviceSelect::Unique(ws, b2, sorted, uniq, counts + 5, (int)nk, st);
+  }
+  int64_t h_sizes[2] = {0, 0};  // n_cut, nnz
+  if (cudaMemcpyAsync(h_sizes, counts + 4, sizeof(h_sizes), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+      cudaStreamSynchronize(st) != cudaSuccess)
+    return fail("sort / unique");
+  const int64_t n_cut = h_sizes[0], nnz = h_sizes[1];
+
+  // 5. CSR arrays and slot maps
+  int32_t* cut = (int32_t*)own(sizeof(int32_t) * n_cut);
+  int32_t* indptr = (int32_t*)own(sizeof(int32_t) * (n_rows + 1));
+  int32_t* indices = (int32_t*)own(sizeof(int32_t) * nnz);
+  // three allocations: the kernels read their slot rows with vector loads (cudaMalloc alignment)
+  int32_t* slots_c = (int32_t*)own(sizeof(int32_t) * kc);
+  int32_t* slots_g = (int32_t*)own(sizeof(int32_t) * kg);
+  int32_t* slots_b = (int32_t*)own(sizeof(int32_t) * kb);
+  if (!cut || !indptr || !indices || !slots_c || !slots_g || !slots_b) return fail("output allocation");
+  cudaMemcpyAsync(cut, cut_full, sizeof(int32_t) * n_cut, cudaMemcpyDeviceToDevice, st);
+  k_row_pointers<<<blocks_for(n_rows + 1), kBlockSym, 0, st>>>(uniq, nnz, n_rows, indptr);
+  if (nnz) k_columns<<<blocks_for(nnz), kBlockSym, 0, st>>>(uniq, nnz, n_rows, indices);
+  if (kc) k_slots<<<blocks_for(kc), kBlockSym, 0, st>>>(uniq, nnz, keys, kc, slots_c);
+  if (kg) k_slots<<<blocks_for(kg), kBlockSym, 0, st>>>(uniq, nnz, keys + kc, kg, slots_g);
+  if (kb) k_slots<<<blocks_for(kb), kBlockSym, 0, st>>>(uniq, nnz, keys + nk, kb, slots_b);
+  if (cudaStreamSynchronize(st) != cudaSuccess || cudaGetLastError() != cudaSuccess) return fail("pattern kernels");
+
+  pat->v.n_rows = n_rows;
+  pat->v.nnz = nnz;
+  pat->v.nd = nd;
+  pat->v.n_active = na;
+  pat->v.n_cut = n_cut;
+  pat->v.n_ghost = ng;
+  pat->v.n_entities = n_entities;
+  pat->v.indptr = indptr;
+  pat->v.indices = indices;
+  pat->v.active = active;
+  pat->v.cut_positions = cut;
   pat->v.ghost = ghost;
   pat->v.slots_cells = slots_c;
   pat->v.slots_ghost = slots_g;

@@ -5,6 +5,9 @@ the per-entity kernels.
 
     pat = symbolic.DevicePattern(mesh, cells_tags, facets_tags, ds_bdy(100))
     A, b = pat.assemble(phi, f, stab_coef=1.0)
+
+`DevicePkPattern` does the same for the quadrature-kernel operators (strong / weak Dirichlet, Neumann, Robin;
+phifem_pk_pattern_create): the arrays of `assemble_pk.PkAssemblyPlan` for a caller-given pattern dofmap.
 """
 import ctypes
 
@@ -81,3 +84,63 @@ class DevicePattern:
         A = CSRMatrix(self.indptr, self.indices, data, (self.n_rows, self.n_rows))
         A._pattern = self          # indptr / indices are views of arrays this object owns
         return A, b
+
+
+class DevicePkPattern:
+    """The symbolic phase of the quadrature-kernel operators through the C ABI (phifem_pk_pattern_create): the arrays of
+    `assemble_pk.PkAssemblyPlan` under the same names and shapes, built on the device and owned by the library.
+
+        plan = assemble.build_plan_weak_dirichlet(mesh, cells_tags, facets_tags, ds(100))
+        pat = symbolic.DevicePkPattern(mesh, cells_tags, facets_tags, ds(100), plan.pattern_dofmap, plan.n_rows)
+
+    `pattern_dofmap` [n_cells, nd]: the cell-local dofs of the space being assembled; `ghost_tags`: the facet tags that
+    carry the ghost penalty, (2, 3) for strong and weak Dirichlet, (3,) for the Neumann demo, (2,) for the Robin demo."""
+
+    def __init__(self, mesh, cells_tags, facets_tags, ds, pattern_dofmap, n_rows, ghost_tags=(2, 3)):
+        _lib.require_cuda(mesh)
+        c8, f8, ents = _plan_inputs(mesh, cells_tags, facets_tags, ds)
+        self.mesh, self.cell_tags8 = mesh, c8
+        self.entities = ents.reshape(-1, 2).to(torch.int32).contiguous()
+        dm = pattern_dofmap.to(device=mesh.device, dtype=torch.int32).contiguous()
+        nd = int(dm.shape[1])
+        mask = 0
+        for t in ghost_tags:
+            if not 0 <= int(t) <= 6:
+                raise ValueError("ghost tag %r outside the tag values 0..6" % (t,))
+            mask |= 1 << int(t)
+        lib = _lib.load()
+        self._handle = _PkPatternHandle()
+        _lib.check(lib.phifem_pk_pattern_create(_lib.c_mesh(mesh), _lib.ptr(dm), nd, int(n_rows), _lib.ptr(c8),
+                                                _lib.ptr(f8), mask,
+                                                _lib.ptr(self.entities) if self.entities.numel() else None,
+                                                self.entities.shape[0], ctypes.byref(self._handle.h), _lib.stream()))
+        v = _lib.CPkPatternView()
+        _lib.check(lib.phifem_pk_pattern_view_of(self._handle.h, ctypes.byref(v)))
+        dev, i32 = mesh.device, torch.int32
+
+        def view(p, *shape):           # each tensor keeps the handle alive: the arrays outlive this object if need be
+            return _lib.device_view(p, shape, i32, dev, owner=self._handle)
+        self.n_rows, self.nnz = int(v.n_rows), int(v.nnz)
+        self.indptr = view(v.indptr, v.n_rows + 1)
+        self.indices = view(v.indices, v.nnz)
+        self.active = view(v.active, v.n_active)
+        self.cut_positions = view(v.cut_positions, v.n_cut)
+        self.ghost = view(v.ghost, v.n_ghost)
+        self.slots_cells = view(v.slots_cells, nd * nd, v.n_active)
+        self.slots_ghost = view(v.slots_ghost, v.n_ghost, 4 * nd * nd)
+        self.slots_boundary = view(v.slots_boundary, v.n_entities, nd * nd)
+
+
+class _PkPatternHandle:
+    """Owner of a phifem_pk_pattern: destroyed with the last tensor that views its arrays."""
+
+    def __init__(self):
+        self.h = ctypes.c_void_p()
+
+    def __del__(self):
+        if self.h and _lib is not None:       # (module globals are gone at interpreter shutdown)
+            try:
+                _lib.load().phifem_pk_pattern_destroy(self.h)
+            except Exception:
+                pass
+            self.h = None
