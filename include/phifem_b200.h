@@ -644,6 +644,51 @@ int phifem_pk_pattern_create(const phifem_mesh* mesh, const int32_t* dofmap, int
 int phifem_pk_pattern_view_of(const phifem_pk_pattern* pattern, phifem_pk_pattern_view* out);
 void phifem_pk_pattern_destroy(phifem_pk_pattern* pattern);
 
+/* ---- symbolic phase of the interface-elasticity operator on the device: the vertex graph, the blocked CSR pattern, the
+ * cut cells, the interface facets and the five position maps that phifem_assemble_elasticity_{cells,facets,boundary},
+ * phifem_apply_dirichlet and phifem_apply_dirichlet_symmetric take.  Every array equals, bit for bit, what
+ * phifem_b200/elasticity.py (ElasticityPlan) builds with torch sort / unique for the same inputs, on triangles,
+ * quadrilaterals and tetrahedra (hexahedra and unknown cell types return PHIFEM_ERR_UNSUPPORTED).
+ *   entities_in [n_in, 2], entities_out [n_out, 2]  the (cell, local facet) pairs of ds(100) and ds(101) (either may be
+ *                         empty); their cells must be tagged 1, 2 or 3.
+ * vptr is the vertex graph: the sorted unique keys row * n_vertices + col over the vertex pairs of every cell tagged 1..3
+ * and of the macro element [vertices of f2c[f][0], vertices of f2c[f][1]] of every interior facet tagged 3 or 4.  The
+ * blocked matrix has NB = 3 d + 2 d^2 dofs per vertex (14 in 2D, 27 in 3D): row NB r + a starts at NB (NB vptr[r] +
+ * a deg(r)) and its entry NB pos + b holds column NB s + b, s = the neighbour of rank pos.  A position is the rank of the
+ * column vertex among the row vertex's neighbours (slot - vptr[row]).  At most 2^31 - 1 blocked entries, NB^2 n_pairs
+ * (else PHIFEM_ERR_ARGUMENT before the blocked arrays are allocated: shard the mesh).
+ * An entity whose cell is not tagged 1..3 or whose local facet is out of range returns PHIFEM_ERR_ARGUMENT (checked on
+ * the device).  This is the one difference from ElasticityPlan, which clamps such a pair's lookup and stores a
+ * meaningless position.  Sort scratch: about 32 bytes per vertex-pair key and 8 per entity key, from the pool
+ * phifem_pattern_release_scratch trims.  The handle owns its arrays (cudaMalloc); the call synchronises the stream as
+ * phifem_pattern_create_p1 does. */
+typedef struct phifem_elasticity_pattern phifem_elasticity_pattern;
+typedef struct phifem_elasticity_pattern_view {
+  int64_t n_vertices;                /* Nv */
+  int32_t nb;                        /* NB: 14 (triangles, quadrilaterals) or 27 (tetrahedra) */
+  int64_t n_rows;                    /* NB Nv */
+  int64_t nnz;                       /* NB^2 n_pairs < 2^31 */
+  int64_t n_pairs;                   /* vptr[Nv]: entries of the vertex graph */
+  int64_t n_cells, n_cut, n_facets_in, n_facets_out, n_entities_in, n_entities_out;
+  const int32_t* vptr;               /* [Nv + 1] */
+  const int32_t* indptr;             /* [n_rows + 1] */
+  const int32_t* indices;            /* [nnz], sorted per row */
+  const int32_t* cut_cells;          /* [n_cut] cells tagged 2, ascending */
+  const int32_t* facets_in;          /* [n_facets_in]  interior facets tagged 3, ascending */
+  const int32_t* facets_out;         /* [n_facets_out] interior facets tagged 4, ascending */
+  const int32_t* pos_cells;          /* [n_cells, nv*nv] cell-major, over all cells; 0 for a cell not tagged 1..3 */
+  const int32_t* pos_facets_in;      /* [n_facets_in, (2 nv)^2]  macro order [vertices of cell +, of cell -] */
+  const int32_t* pos_facets_out;     /* [n_facets_out, (2 nv)^2] */
+  const int32_t* pos_entities_in;    /* [n_entities_in, nv*nv]  row = test vertex */
+  const int32_t* pos_entities_out;   /* [n_entities_out, nv*nv] */
+} phifem_elasticity_pattern_view;
+
+int phifem_elasticity_pattern_create(const phifem_mesh* mesh, const int8_t* cell_tags8, const int8_t* facet_tags8,
+                                     const int32_t* entities_in, int64_t n_in, const int32_t* entities_out,
+                                     int64_t n_out, phifem_elasticity_pattern** out, void* stream);
+int phifem_elasticity_pattern_view_of(const phifem_elasticity_pattern* pattern, phifem_elasticity_pattern_view* out);
+void phifem_elasticity_pattern_destroy(phifem_elasticity_pattern* pattern);
+
 /* ---- the row-gather plan itself, built on the device (csrc/rows_plan.cu): CSR pattern (indptr, indices), active cells,
  * ghost facets and the two row lists of phifem_rows_plan, from the vertex -> cell adjacency (one radix sort of
  * n_active * nv keys, per-row merges) instead of one key per coupled vertex pair.  Every array equals what

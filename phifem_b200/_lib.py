@@ -96,6 +96,15 @@ class CPkPatternView(ctypes.Structure):
                 ("slots_boundary", _vp)]
 
 
+class CElasticityPatternView(ctypes.Structure):
+    _fields_ = [("n_vertices", ctypes.c_int64), ("nb", ctypes.c_int32), ("n_rows", ctypes.c_int64),
+                ("nnz", ctypes.c_int64), ("n_pairs", ctypes.c_int64), ("n_cells", ctypes.c_int64),
+                ("n_cut", ctypes.c_int64), ("n_facets_in", ctypes.c_int64), ("n_facets_out", ctypes.c_int64),
+                ("n_entities_in", ctypes.c_int64), ("n_entities_out", ctypes.c_int64)] + \
+        [(n, _vp) for n in ("vptr", "indptr", "indices", "cut_cells", "facets_in", "facets_out", "pos_cells",
+                            "pos_facets_in", "pos_facets_out", "pos_entities_in", "pos_entities_out")]
+
+
 class CElasticityParams(ctypes.Structure):
     _fields_ = [(n, ctypes.c_double) for n in ("lmbda_in", "mu_in", "lmbda_out", "mu_out", "coef_in", "coef_out",
                                                "gamma", "sigma_s")]
@@ -179,6 +188,10 @@ _SIGNATURES = {
                                                 ctypes.c_uint32, _vp, ctypes.c_int64, ctypes.POINTER(_vp), _vp]),
     "phifem_pk_pattern_view_of": (ctypes.c_int, [_vp, ctypes.POINTER(CPkPatternView)]),
     "phifem_pk_pattern_destroy": (None, [_vp]),
+    "phifem_elasticity_pattern_create": (ctypes.c_int, [ctypes.POINTER(CMesh), _vp, _vp, _vp, ctypes.c_int64, _vp,
+                                                        ctypes.c_int64, ctypes.POINTER(_vp), _vp]),
+    "phifem_elasticity_pattern_view_of": (ctypes.c_int, [_vp, ctypes.POINTER(CElasticityPatternView)]),
+    "phifem_elasticity_pattern_destroy": (None, [_vp]),
     "phifem_surface_static_p1": (ctypes.c_int, [ctypes.POINTER(CMesh), ctypes.POINTER(CRowsPlan), _vp]),
     "phifem_rows_plan_create": (ctypes.c_int, [ctypes.POINTER(CMesh), _vp, _vp, _vp, ctypes.c_int64, _vp,
                                                ctypes.c_int32, ctypes.POINTER(_vp), _vp]),

@@ -8,7 +8,9 @@
 //
 // Device algorithm: stream compaction of the active cells and ghost facets (cub::DeviceSelect), one 64-bit key
 // row * n_vertices + col per coupled vertex pair, radix sort + unique (cub) = the pattern, binary searches for the row
-// pointers and the slot maps.
+// pointers and the slot maps.  The same steps serve the quadrature-kernel operators (phifem_pk_pattern_create, over a
+// caller-given dofmap) and the interface-elasticity operator (phifem_elasticity_pattern_create: the vertex graph, then
+// its expansion into dense NB x NB blocks).
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_select.cuh>
 #include <thrust/iterator/counting_iterator.h>
@@ -24,6 +26,12 @@ struct phifem_pattern {
 struct phifem_pk_pattern {
   phifem_pk_pattern_view v;
   void* owned[8];
+  int n_owned;
+};
+
+struct phifem_elasticity_pattern {
+  phifem_elasticity_pattern_view v;
+  void* owned[12];
   int n_owned;
 };
 
@@ -212,6 +220,81 @@ __global__ void k_entity_unpack(const int64_t* __restrict__ sval, int64_t n, int
   if (t >= n) return;
   out[2 * t] = (int32_t)(sval[t] >> 3);
   out[2 * t + 1] = (int32_t)(sval[t] & 7);
+}
+
+// ---- interface elasticity (phifem_elasticity_pattern_create): the vertex graph, expanded into dense NB x NB blocks
+
+struct IsMaskedCell {  // cells whose tag t has bit t set in `mask`
+  const int8_t* tags;
+  uint32_t mask;
+  __device__ bool operator()(int c) const {
+    const int t = tags[c];
+    return t >= 0 && t < 7 && ((mask >> t) & 1u);
+  }
+};
+
+// input check of the one-sided entities: cell outside the mesh or not tagged in `cell_mask`, local facet out of range
+__global__ void k_count_entities_outside(const int32_t* __restrict__ entities, int64_t n,
+                                         const int8_t* __restrict__ tags, int64_t n_cells, int n_local_facets,
+                                         uint32_t cell_mask, unsigned long long* __restrict__ bad) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n) return;
+  const int32_t c = entities[2 * t], lf = entities[2 * t + 1];
+  if (c < 0 || c >= n_cells || lf < 0 || lf >= n_local_facets) atomicAdd(bad, 1ull);
+  else if (tags[c] < 0 || tags[c] > 6 || !((cell_mask >> tags[c]) & 1u)) atomicAdd(bad, 1ull);
+}
+
+// position of a vertex pair = its slot minus the row's first slot = rank of the column among the row's neighbours;
+// keys[e * w + i] -> pos[scatter[e] * w + i] (scatter null: pos[e * w + i])
+__global__ void k_positions(const int64_t* __restrict__ uniq, int64_t nnz, const int32_t* __restrict__ vptr,
+                            int64_t n_vertices, const int64_t* __restrict__ keys, int64_t n, int w,
+                            const int32_t* __restrict__ scatter, int32_t* __restrict__ pos) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n * w) return;
+  const int64_t key = keys[t];
+  const int32_t p = (int32_t)(lower_bound(uniq, nnz, key) - vptr[key / n_vertices]);
+  if (scatter) {
+    const int64_t e = t / w;
+    pos[(int64_t)scatter[e] * w + (t - e * w)] = p;
+  } else {
+    pos[t] = p;
+  }
+}
+
+// blocked row NB r + a starts at NB (NB vptr[r] + a deg(r)); the last entry (r = n_vertices, a = 0) is NB^2 vptr[Nv]
+__global__ void k_blocked_row_pointers(const int32_t* __restrict__ vptr, int64_t n_vertices, int nb,
+                                       int32_t* __restrict__ indptr) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t > nb * n_vertices) return;
+  const int64_t r = t / nb, a = t - r * nb;
+  const int64_t deg = r < n_vertices ? vptr[r + 1] - vptr[r] : 0;
+  indptr[t] = (int32_t)(nb * (nb * (int64_t)vptr[r] + a * deg));
+}
+
+// column indices of the blocked matrix: the NB rows of vertex r are NB copies of the same run of L = NB deg(r) words,
+// word j = NB vcol[vptr[r] + j / NB] + j % NB, and they are contiguous from NB^2 vptr[r] on.  One warp per vertex walks
+// that block of NB L words with consecutive lanes on consecutive words (the stores coalesce); j = w mod L is carried
+// from one step to the next.  Bound by its stores: 4 NB^2 bytes per vertex pair, every address 64-bit.
+template <int NB>
+__global__ void k_expand_blocks(const int32_t* __restrict__ vptr, const int32_t* __restrict__ vcols,
+                                int64_t n_vertices, int32_t* __restrict__ indices) {
+  const int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (r >= n_vertices) return;
+  const int lane = threadIdx.x & 31;
+  const int64_t beg = vptr[r];
+  const int L = NB * (int)(vptr[r + 1] - beg);
+  if (L == 0) return;
+  const int32_t* __restrict__ cols = vcols + beg;
+  int32_t* __restrict__ out = indices + NB * NB * beg;
+  const int64_t total = (int64_t)NB * L;
+  int j = lane;
+  while (j >= L) j -= L;
+  for (int64_t w = lane; w < total; w += 32) {
+    const int p = j / NB;
+    out[w] = NB * cols[p] + (j - p * NB);
+    j += 32;
+    while (j >= L) j -= L;
+  }
 }
 
 struct Scratch {  // device allocations freed on scope exit (stream-ordered)
@@ -580,6 +663,238 @@ extern "C" int phifem_pk_pattern_create(const phifem_mesh* mesh, const int32_t* 
   pat->v.slots_cells = slots_c;
   pat->v.slots_ghost = slots_g;
   pat->v.slots_boundary = slots_b;
+  *out = pat;
+  return PHIFEM_OK;
+}
+
+extern "C" void phifem_elasticity_pattern_destroy(phifem_elasticity_pattern* p) {
+  if (!p) return;
+  for (int i = 0; i < p->n_owned; ++i) cudaFree(p->owned[i]);
+  delete p;
+}
+
+extern "C" int phifem_elasticity_pattern_view_of(const phifem_elasticity_pattern* p,
+                                                 phifem_elasticity_pattern_view* out) {
+  PHIFEM_CHECK_ARG(p && out, "null pointer");
+  *out = p->v;
+  return PHIFEM_OK;
+}
+
+// The arrays of ElasticityPlan (phifem_b200/elasticity.py), bit for bit: vertex graph = sorted unique keys
+// row * Nv + col of the vertex pairs of every cell tagged 1..3 and of the macro elements of the interior facets tagged
+// 3 / 4, blocked CSR = that graph with dense NB x NB blocks, positions = ranks of the column vertices in their rows.
+extern "C" int phifem_elasticity_pattern_create(const phifem_mesh* mesh, const int8_t* cell_tags8,
+                                                const int8_t* facet_tags8, const int32_t* entities_in, int64_t n_in,
+                                                const int32_t* entities_out, int64_t n_out,
+                                                phifem_elasticity_pattern** out, void* stream) {
+  PHIFEM_CHECK_ARG(out != nullptr, "out is null");
+  *out = nullptr;
+  PHIFEM_CHECK_ARG(mesh != nullptr && mesh->cells && mesh->c2f && mesh->f2c, "mesh / facet connectivity is null");
+  if (mesh->cell_type != PHIFEM_TRIANGLE && mesh->cell_type != PHIFEM_TETRAHEDRON &&
+      mesh->cell_type != PHIFEM_QUADRILATERAL) {
+    set_error("phifem_elasticity_pattern_create: the interface-elasticity operator assembles on triangles, "
+              "quadrilaterals and tetrahedra, got cell type %d", mesh->cell_type);
+    return PHIFEM_ERR_UNSUPPORTED;
+  }
+  PHIFEM_CHECK_ARG(cell_tags8 && facet_tags8, "tag arrays are null");
+  PHIFEM_CHECK_ARG(n_in >= 0 && (n_in == 0 || entities_in), "entities_in list");
+  PHIFEM_CHECK_ARG(n_out >= 0 && (n_out == 0 || entities_out), "entities_out list");
+  const int d = mesh->cell_type == PHIFEM_TETRAHEDRON ? 3 : 2;
+  const int nv = mesh->cell_type == PHIFEM_TRIANGLE ? 3 : 4, n_local_facets = nv, nm = 2 * nv;
+  const int nb = 3 * d + 2 * d * d;
+  const int64_t n_vertices = mesh->n_vertices;
+  PHIFEM_CHECK_ARG(mesh->n_cells < (1ll << 31) && mesh->n_facets < (1ll << 31) && n_vertices >= 0 &&
+                       nb * n_vertices < (1ll << 31),
+                   "int32 index width");
+  cudaStream_t st = (cudaStream_t)stream;
+  cudaMemPool_t pool = scratch_pool();
+  if (!pool) {
+    set_error("phifem_elasticity_pattern_create: cannot create the scratch memory pool");
+    return PHIFEM_ERR_CUDA;
+  }
+  Scratch tmp(st, pool);
+  phifem_elasticity_pattern* pat = new phifem_elasticity_pattern();
+  pat->n_owned = 0;
+  auto own = [&](size_t bytes) -> void* {
+    void* q = nullptr;
+    if (cudaMalloc(&q, bytes ? bytes : 1) != cudaSuccess) return nullptr;
+    pat->owned[pat->n_owned++] = q;
+    return q;
+  };
+  auto fail = [&](const char* what) {
+    set_error("phifem_elasticity_pattern_create: %s: %s", what, cudaGetErrorString(cudaGetLastError()));
+    phifem_elasticity_pattern_destroy(pat);
+    return PHIFEM_ERR_CUDA;
+  };
+  auto refuse = [&](const char* what) {
+    set_error("phifem_elasticity_pattern_create: %s", what);
+    phifem_elasticity_pattern_destroy(pat);
+    return PHIFEM_ERR_ARGUMENT;
+  };
+
+  // 1. tagged cells (1..3), cut cells (2), interior facets tagged 3 and 4, ascending; the entity check counts into the
+  //    same block: {n_tagged, n_cut, n_facets_in, n_facets_out, bad entities, n_pairs}
+  const int64_t n_cells = mesh->n_cells;
+  int32_t* tagged_full = (int32_t*)tmp.get(sizeof(int32_t) * n_cells);
+  int32_t* cut_full = (int32_t*)tmp.get(sizeof(int32_t) * n_cells);
+  int32_t* fin_full = (int32_t*)tmp.get(sizeof(int32_t) * mesh->n_facets);
+  int32_t* fout_full = (int32_t*)tmp.get(sizeof(int32_t) * mesh->n_facets);
+  int64_t* counts = (int64_t*)tmp.get(6 * sizeof(int64_t));
+  if (!tagged_full || !cut_full || !fin_full || !fout_full || !counts) return fail("scratch allocation");
+  cudaMemsetAsync(counts, 0, 6 * sizeof(int64_t), st);
+  {
+    thrust::counting_iterator<int> it(0);
+    const IsMaskedCell is_tagged{cell_tags8, (1u << 1) | (1u << 2) | (1u << 3)}, is_cut{cell_tags8, 1u << 2};
+    const IsMaskedGhostFacet is_in{facet_tags8, mesh->f2c, 1u << 3}, is_out{facet_tags8, mesh->f2c, 1u << 4};
+    size_t b1 = 0, b2 = 0;
+    cub::DeviceSelect::If(nullptr, b1, it, tagged_full, counts, (int)n_cells, is_tagged, st);
+    cub::DeviceSelect::If(nullptr, b2, it, fin_full, counts + 2, (int)mesh->n_facets, is_in, st);
+    void* ws = tmp.get(b1 > b2 ? b1 : b2);
+    if (!ws) return fail("scratch allocation");
+    cub::DeviceSelect::If(ws, b1, it, tagged_full, counts, (int)n_cells, is_tagged, st);
+    cub::DeviceSelect::If(ws, b1, it, cut_full, counts + 1, (int)n_cells, is_cut, st);
+    cub::DeviceSelect::If(ws, b2, it, fin_full, counts + 2, (int)mesh->n_facets, is_in, st);
+    cub::DeviceSelect::If(ws, b2, it, fout_full, counts + 3, (int)mesh->n_facets, is_out, st);
+  }
+  unsigned long long* bad = (unsigned long long*)(counts + 4);
+  const uint32_t tagged_mask = (1u << 1) | (1u << 2) | (1u << 3);
+  if (n_in)
+    k_count_entities_outside<<<blocks_for(n_in), kBlockSym, 0, st>>>(entities_in, n_in, cell_tags8, n_cells,
+                                                                     n_local_facets, tagged_mask, bad);
+  if (n_out)
+    k_count_entities_outside<<<blocks_for(n_out), kBlockSym, 0, st>>>(entities_out, n_out, cell_tags8, n_cells,
+                                                                      n_local_facets, tagged_mask, bad);
+  int64_t h_counts[5] = {0, 0, 0, 0, 0};
+  if (cudaMemcpyAsync(h_counts, counts, sizeof(h_counts), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+      cudaStreamSynchronize(st) != cudaSuccess)
+    return fail("compaction");
+  if (h_counts[4])
+    return refuse("entities: an entity's cell is not tagged 1, 2 or 3, or its local facet is out of range");
+  const int64_t nt = h_counts[0], n_cut = h_counts[1], nfi = h_counts[2], nfo = h_counts[3];
+  const int64_t kc = nt * nv * nv, kfi = nfi * nm * nm, kfo = nfo * nm * nm, nk = kc + kfi + kfo;
+  const int64_t kei = n_in * nv * nv, keo = n_out * nv * nv;
+  if (nk >= (1ll << 31)) {
+    set_error("phifem_elasticity_pattern_create: %lld coupled vertex pairs (limit 2^31): shard the mesh", (long long)nk);
+    phifem_elasticity_pattern_destroy(pat);
+    return PHIFEM_ERR_ARGUMENT;
+  }
+  int32_t* cut = (int32_t*)own(sizeof(int32_t) * n_cut);
+  int32_t* fin = (int32_t*)own(sizeof(int32_t) * nfi);
+  int32_t* fout = (int32_t*)own(sizeof(int32_t) * nfo);
+  if (!cut || !fin || !fout) return fail("output allocation");
+  cudaMemcpyAsync(cut, cut_full, sizeof(int32_t) * n_cut, cudaMemcpyDeviceToDevice, st);
+  cudaMemcpyAsync(fin, fin_full, sizeof(int32_t) * nfi, cudaMemcpyDeviceToDevice, st);
+  cudaMemcpyAsync(fout, fout_full, sizeof(int32_t) * nfo, cudaMemcpyDeviceToDevice, st);
+
+  // 2. keys: tagged cells, the macro elements [vertices of f2c[f][0], of f2c[f][1]] of both facet lists, both entity
+  //    lists (looked up only: their cells are tagged, so they add no pair)
+  int64_t* keys = (int64_t*)tmp.get(sizeof(int64_t) * (nk + kei + keo));
+  int32_t* macro = (int32_t*)tmp.get(sizeof(int32_t) * (nfi + nfo) * nm);
+  if (!keys || !macro) return fail("scratch allocation");
+  if (kc) k_cell_pair_keys<<<blocks_for(kc), kBlockSym, 0, st>>>(mesh->cells, nv, tagged_full, 1, nt, n_vertices, keys);
+  if (nfi) {
+    k_macro_dofs<<<blocks_for(nfi * nm), kBlockSym, 0, st>>>(mesh->f2c, mesh->cells, nv, fin, nfi, macro);
+    k_pair_keys<<<blocks_for(kfi), kBlockSym, 0, st>>>(macro, nfi, nm, n_vertices, keys + kc);
+  }
+  if (nfo) {
+    k_macro_dofs<<<blocks_for(nfo * nm), kBlockSym, 0, st>>>(mesh->f2c, mesh->cells, nv, fout, nfo, macro + nfi * nm);
+    k_pair_keys<<<blocks_for(kfo), kBlockSym, 0, st>>>(macro + nfi * nm, nfo, nm, n_vertices, keys + kc + kfi);
+  }
+  if (kei)
+    k_cell_pair_keys<<<blocks_for(kei), kBlockSym, 0, st>>>(mesh->cells, nv, entities_in, 2, n_in, n_vertices,
+                                                           keys + nk);
+  if (keo)
+    k_cell_pair_keys<<<blocks_for(keo), kBlockSym, 0, st>>>(mesh->cells, nv, entities_out, 2, n_out, n_vertices,
+                                                           keys + nk + kei);
+
+  // 3. vertex graph = sorted unique keys of the cells and macro elements
+  int64_t* sorted = (int64_t*)tmp.get(sizeof(int64_t) * nk);
+  int64_t* uniq = (int64_t*)tmp.get(sizeof(int64_t) * nk);
+  if (!sorted || !uniq) return fail("scratch allocation");
+  if (nk) {
+    int end_bit = 1;
+    while (end_bit < 63 && (1ll << end_bit) < n_vertices * n_vertices) ++end_bit;
+    size_t b1 = 0, b2 = 0;
+    cub::DeviceRadixSort::SortKeys(nullptr, b1, keys, sorted, (int)nk, 0, end_bit, st);
+    cub::DeviceSelect::Unique(nullptr, b2, sorted, uniq, counts + 5, (int)nk, st);
+    void* ws = tmp.get(b1 > b2 ? b1 : b2);
+    if (!ws) return fail("scratch allocation");
+    cub::DeviceRadixSort::SortKeys(ws, b1, keys, sorted, (int)nk, 0, end_bit, st);
+    cub::DeviceSelect::Unique(ws, b2, sorted, uniq, counts + 5, (int)nk, st);
+  }
+  int64_t n_pairs = 0;
+  if (cudaMemcpyAsync(&n_pairs, counts + 5, sizeof(n_pairs), cudaMemcpyDeviceToHost, st) != cudaSuccess ||
+      cudaStreamSynchronize(st) != cudaSuccess)
+    return fail("sort / unique");
+  const int64_t nnz = (int64_t)nb * nb * n_pairs;
+  if (nnz >= (1ll << 31)) {
+    set_error("phifem_elasticity_pattern_create: %lld blocked entries (%d^2 x %lld vertex pairs; limit 2^31 - 1): "
+              "shard the mesh", (long long)nnz, nb, (long long)n_pairs);
+    phifem_elasticity_pattern_destroy(pat);
+    return PHIFEM_ERR_ARGUMENT;
+  }
+
+  // 4. vertex row pointers, positions, blocked CSR
+  const int64_t n_rows = nb * n_vertices;
+  int32_t* vptr = (int32_t*)own(sizeof(int32_t) * (n_vertices + 1));
+  int32_t* indptr = (int32_t*)own(sizeof(int32_t) * (n_rows + 1));
+  int32_t* indices = (int32_t*)own(sizeof(int32_t) * nnz);
+  int32_t* pos_c = (int32_t*)own(sizeof(int32_t) * n_cells * nv * nv);
+  int32_t* pos_fi = (int32_t*)own(sizeof(int32_t) * kfi);
+  int32_t* pos_fo = (int32_t*)own(sizeof(int32_t) * kfo);
+  int32_t* pos_ei = (int32_t*)own(sizeof(int32_t) * kei);
+  int32_t* pos_eo = (int32_t*)own(sizeof(int32_t) * keo);
+  int32_t* vcols = (int32_t*)tmp.get(sizeof(int32_t) * n_pairs);
+  if (!vptr || !indptr || !indices || !pos_c || !pos_fi || !pos_fo || !pos_ei || !pos_eo) return fail("output allocation");
+  if (!vcols) return fail("scratch allocation");
+  k_row_pointers<<<blocks_for(n_vertices + 1), kBlockSym, 0, st>>>(uniq, n_pairs, n_vertices, vptr);
+  if (n_pairs) k_columns<<<blocks_for(n_pairs), kBlockSym, 0, st>>>(uniq, n_pairs, n_vertices, vcols);
+  cudaMemsetAsync(pos_c, 0, sizeof(int32_t) * n_cells * nv * nv, st);  // cells not tagged 1..3 keep 0
+  if (kc)
+    k_positions<<<blocks_for(kc), kBlockSym, 0, st>>>(uniq, n_pairs, vptr, n_vertices, keys, nt, nv * nv, tagged_full,
+                                                      pos_c);
+  if (kfi)
+    k_positions<<<blocks_for(kfi), kBlockSym, 0, st>>>(uniq, n_pairs, vptr, n_vertices, keys + kc, nfi, nm * nm,
+                                                       nullptr, pos_fi);
+  if (kfo)
+    k_positions<<<blocks_for(kfo), kBlockSym, 0, st>>>(uniq, n_pairs, vptr, n_vertices, keys + kc + kfi, nfo, nm * nm,
+                                                       nullptr, pos_fo);
+  if (kei)
+    k_positions<<<blocks_for(kei), kBlockSym, 0, st>>>(uniq, n_pairs, vptr, n_vertices, keys + nk, n_in, nv * nv,
+                                                       nullptr, pos_ei);
+  if (keo)
+    k_positions<<<blocks_for(keo), kBlockSym, 0, st>>>(uniq, n_pairs, vptr, n_vertices, keys + nk + kei, n_out,
+                                                       nv * nv, nullptr, pos_eo);
+  k_blocked_row_pointers<<<blocks_for(n_rows + 1), kBlockSym, 0, st>>>(vptr, n_vertices, nb, indptr);
+  if (nnz) {
+    const unsigned grid = (unsigned)((n_vertices + kBlockSym / 32 - 1) / (kBlockSym / 32));  // one warp per vertex
+    if (nb == 14) k_expand_blocks<14><<<grid, kBlockSym, 0, st>>>(vptr, vcols, n_vertices, indices);
+    else k_expand_blocks<27><<<grid, kBlockSym, 0, st>>>(vptr, vcols, n_vertices, indices);
+  }
+  if (cudaStreamSynchronize(st) != cudaSuccess || cudaGetLastError() != cudaSuccess) return fail("pattern kernels");
+
+  pat->v.n_vertices = n_vertices;
+  pat->v.nb = nb;
+  pat->v.n_rows = n_rows;
+  pat->v.nnz = nnz;
+  pat->v.n_pairs = n_pairs;
+  pat->v.n_cells = n_cells;
+  pat->v.n_cut = n_cut;
+  pat->v.n_facets_in = nfi;
+  pat->v.n_facets_out = nfo;
+  pat->v.n_entities_in = n_in;
+  pat->v.n_entities_out = n_out;
+  pat->v.vptr = vptr;
+  pat->v.indptr = indptr;
+  pat->v.indices = indices;
+  pat->v.cut_cells = cut;
+  pat->v.facets_in = fin;
+  pat->v.facets_out = fout;
+  pat->v.pos_cells = pos_c;
+  pat->v.pos_facets_in = pos_fi;
+  pat->v.pos_facets_out = pos_fo;
+  pat->v.pos_entities_in = pos_ei;
+  pat->v.pos_entities_out = pos_eo;
   *out = pat;
   return PHIFEM_OK;
 }

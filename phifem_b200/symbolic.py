@@ -8,6 +8,8 @@ the per-entity kernels.
 
 `DevicePkPattern` does the same for the quadrature-kernel operators (strong / weak Dirichlet, Neumann, Robin;
 phifem_pk_pattern_create): the arrays of `assemble_pk.PkAssemblyPlan` for a caller-given pattern dofmap.
+`DeviceElasticityPattern` does it for the interface-elasticity operator (phifem_elasticity_pattern_create): the arrays
+of `elasticity.ElasticityPlan`.
 """
 import ctypes
 
@@ -109,7 +111,7 @@ class DevicePkPattern:
                 raise ValueError("ghost tag %r outside the tag values 0..6" % (t,))
             mask |= 1 << int(t)
         lib = _lib.load()
-        self._handle = _PkPatternHandle()
+        self._handle = _PatternHandle("phifem_pk_pattern_destroy")
         _lib.check(lib.phifem_pk_pattern_create(_lib.c_mesh(mesh), _lib.ptr(dm), nd, int(n_rows), _lib.ptr(c8),
                                                 _lib.ptr(f8), mask,
                                                 _lib.ptr(self.entities) if self.entities.numel() else None,
@@ -131,16 +133,62 @@ class DevicePkPattern:
         self.slots_boundary = view(v.slots_boundary, v.n_entities, nd * nd)
 
 
-class _PkPatternHandle:
-    """Owner of a phifem_pk_pattern: destroyed with the last tensor that views its arrays."""
+class DeviceElasticityPattern:
+    """The symbolic phase of the interface-elasticity operator through the C ABI (phifem_elasticity_pattern_create): the
+    arrays of `elasticity.ElasticityPlan` under the same names and shapes, built on the device and owned by the library.
 
-    def __init__(self):
+        pat = symbolic.DeviceElasticityPattern(mesh, cells_tags, facets_tags, d_bdry)
+
+    `d_bdry`: the measure of compute_tags_measures(box_mode=True), whose ids 100 and 101 are used, or a pair of entity
+    arrays (ds100, ds101), as for `elasticity.build_plan_interface_elasticity`."""
+
+    def __init__(self, mesh, cells_tags, facets_tags, d_bdry):
+        from .mesh import Measure
+        _lib.require_cuda(mesh)
+        d100, d101 = (d_bdry(100), d_bdry(101)) if isinstance(d_bdry, Measure) else d_bdry
+        c8, f8, e_in = _plan_inputs(mesh, cells_tags, facets_tags, d100)
+        _, _, e_out = _plan_inputs(mesh, cells_tags, facets_tags, d101)
+        self.mesh, self.cell_tags8 = mesh, c8
+        self.entities_in = e_in.reshape(-1, 2).to(torch.int32).contiguous()
+        self.entities_out = e_out.reshape(-1, 2).to(torch.int32).contiguous()
+        lib = _lib.load()
+        self._handle = _PatternHandle("phifem_elasticity_pattern_destroy")
+        ents = [(_lib.ptr(e) if e.numel() else None, e.shape[0]) for e in (self.entities_in, self.entities_out)]
+        _lib.check(lib.phifem_elasticity_pattern_create(_lib.c_mesh(mesh), _lib.ptr(c8), _lib.ptr(f8), *ents[0],
+                                                        *ents[1], ctypes.byref(self._handle.h), _lib.stream()))
+        v = _lib.CElasticityPatternView()
+        _lib.check(lib.phifem_elasticity_pattern_view_of(self._handle.h, ctypes.byref(v)))
+        dev, i32 = mesh.device, torch.int32
+        nv = mesh.cells.shape[1]
+
+        def view(p, *shape):           # each tensor keeps the handle alive: the arrays outlive this object if need be
+            return _lib.device_view(p, shape, i32, dev, owner=self._handle)
+        self.nb, self.n_rows, self.nnz = int(v.nb), int(v.n_rows), int(v.nnz)
+        self.vptr = view(v.vptr, v.n_vertices + 1)
+        self.indptr = view(v.indptr, v.n_rows + 1)
+        self.indices = view(v.indices, v.nnz)
+        self.cut_cells = view(v.cut_cells, v.n_cut)
+        self.facets_in = view(v.facets_in, v.n_facets_in)
+        self.facets_out = view(v.facets_out, v.n_facets_out)
+        self.pos_cells = view(v.pos_cells, v.n_cells, nv * nv)
+        self.pos_facets_in = view(v.pos_facets_in, v.n_facets_in, 4 * nv * nv)
+        self.pos_facets_out = view(v.pos_facets_out, v.n_facets_out, 4 * nv * nv)
+        self.pos_entities_in = view(v.pos_entities_in, v.n_entities_in, nv * nv)
+        self.pos_entities_out = view(v.pos_entities_out, v.n_entities_out, nv * nv)
+
+
+class _PatternHandle:
+    """Owner of a library pattern handle, released by `destroy`: destroyed with the last tensor that views its
+    arrays."""
+
+    def __init__(self, destroy):
         self.h = ctypes.c_void_p()
+        self.destroy = destroy
 
     def __del__(self):
         if self.h and _lib is not None:       # (module globals are gone at interpreter shutdown)
             try:
-                _lib.load().phifem_pk_pattern_destroy(self.h)
+                getattr(_lib.load(), self.destroy)(self.h)
             except Exception:
                 pass
             self.h = None
